@@ -9,13 +9,13 @@ trackers on as in the reference).  For N > 1 launch with torchrun (one rank per 
 batch; the only collective of the path is one NCCL all-reduce of the episode statistics).
 
 Prints ONE JSON line (rank 0).
-  value      whole-job env-steps/s with inputs resident in HBM.  The K steps are captured once as a CUDA graph of the K step
-             launches; the graph is replayed M times back to back (M chosen so that the region lasts >= ~100 ms per rank),
-             every replay bracketed by its own CUDA-event pair on the launch stream, barrier + synchronize around the region.
-             Per rank the MEDIAN replay is taken; the job's figure is the MAX over ranks of those medians (a 0.5 ms region
-             with a plain max-reduce is one scheduling hiccup away from -26 %: round-1 SCALE at N = 8).  Every rank's
-             median / min / max is in `per_rank`.  The L2 is kept cold by data size: R independent replicas of the batch
-             are stepped round robin so that >= 256 MiB of state is touched between two visits of a replica.
+  value      whole-job env-steps/s with inputs resident in HBM.  The timed region is exactly K = --steps steps of every env:
+             the K steps of all replicas are captured once as a CUDA graph (NoMove + scripted gaze: one d2d_rollout call
+             per replica; otherwise K step launches per replica) and the graph is replayed once between a CUDA-event pair on
+             the launch stream, barrier + synchronize around it.  The job's figure is the MAX over ranks; every rank's
+             figure is in `per_rank`.  A short K gives a short, noisier region.  The L2 is kept cold by data size: R
+             independent replicas of the batch are stepped in turn so that >= 256 MiB of state is touched between two visits
+             of a replica.  The e2e legs and `per_step_events` also run K steps each.
   e2e        the same metric through d2d_step_host with pinned HOST buffers, host<->device traffic inside the timed region:
              headline = zero-copy mirror transport (d2d_bind_host_mirror), `e2e.full_copy` = plain copies of the whole
              observation every step.
@@ -25,6 +25,13 @@ Prints ONE JSON line (rank 0).
              roofline and per-rank figures.
   shard_invariant (N > 1)  every rank also steps a 64-env slice of its neighbour's shard; the state hashes agree.
   cpu_baseline   the oracle port of the reference path (oracle/drone2d_oracle.c) on the host cores, bounded sample.
+
+--dump-outputs DIR writes what the headline path returned to its caller at the last of its K timed steps, for every env
+of every replica (observation, done, reward, the `info` arrays; the fused Oxford call also the next actions), as
+DIR/<name>.npy, float32 or float64, under 64 MiB: above that a fixed seeded sample of envs, whose indices are in
+DIR/env_index.npy.  Before that step every env has run exactly W warm-up, the burn-in and the K timed steps from seeded
+worlds and actions, so with the same arguments two builds can be compared output for output.  With several ranks the
+files hold rank 0's shard.
 """
 import argparse
 import hashlib
@@ -105,6 +112,48 @@ def public_config(cfg, n_gpus):
     return {"workload": cfg["name"], "envs_per_gpu": cfg["envs"], "agents_per_env": n_agents_of(cfg),
             "rays_per_env_step": n_rays_of(cfg), "planner": cfg["params"]["planner"], "gaze": cfg["gaze"],
             "trackers": True, "auto_reset": True, "l2": L2_NOTE, "parallelism": "env-sharded x%d" % n_gpus}
+
+
+DUMP_BYTES = 60 << 20                           # array data; with the .npy headers the files stay under 64 MiB
+
+
+def caller_outputs(envs, next_actions=None):
+    """What a caller of the step receives from every replica in `envs` (observation, reward, done, info; the fused Oxford
+    call also the next actions, one tensor per replica) as host arrays: float64, int32 and int64 buffers as float64, the
+    8-bit and float32 ones as float32 (both exact).  Rows are envs, replica r's env i at row r * B + i; when the rows are
+    above DUMP_BYTES a fixed seeded sample of them is kept, named by `env_index`."""
+    import torch
+
+    def named(e, nxt):
+        obs, info = e._obs(), e.info
+        out = [("local_map", obs["local_map"]), ("yaw_angle", obs["yaw_angle"]), ("reward", e.reward), ("done", e.buffer("done"))]
+        out += sorted(info.items())
+        if nxt is not None:
+            out.append(("next_actions", nxt))
+        return out
+    wide = (torch.float64, torch.int32, torch.int64)
+    B = envs[0].num_envs
+    per_env = 8 + sum((8 if t.dtype in wide else 4) * (t.numel() // B) for _, t in named(envs[0], None if next_actions is None
+                                                                                          else next_actions[0]))
+    total = B * len(envs)
+    n = min(total, DUMP_BYTES // per_env)
+    rows = np.arange(total) if n == total else np.sort(np.random.RandomState(0).choice(total, n, replace=False))
+    parts = {}
+    for r, e in enumerate(envs):
+        local = rows[(rows >= r * B) & (rows < (r + 1) * B)] - r * B
+        idx = torch.as_tensor(local, device=e.device)
+        for name, t in named(e, None if next_actions is None else next_actions[r]):
+            t = t.index_select(0, idx)
+            parts.setdefault(name, []).append(t.to(torch.float64 if t.dtype in wide else torch.float32).cpu().numpy())
+    out = {"env_index": rows.astype(np.float64)}
+    out.update({name: np.concatenate(p) for name, p in parts.items()})
+    return out
+
+
+def write_dump(directory, arrays):
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def _gen_chunk(args):
@@ -355,8 +404,9 @@ def measure(ctx, cfg, worlds, t_world, unique, headline):
     actions = table[torch.randint(0, 6, (K + W, B), device=dev, generator=gen)].contiguous()
     burn = args.burn_in if headline else min(args.burn_in, 300)
 
-    for t in range(max(W, R)):                      # eager warm-up: every replica steps at least once
-        do_step(actions[t % (K + W)], envs[t % R])
+    for e in envs:                                  # eager warm-up: W steps of every replica
+        for t in range(W):
+            do_step(actions[t], e)
     # burn-in (untimed): episodes last up to 800 steps, so the mix of fresh / explored / tracking envs -- and with it the
     # cost of a step -- only becomes stationary after about a thousand steps (SURVEY 8d: 1000 steps with auto-reset)
     for t in range(burn):
@@ -364,52 +414,49 @@ def measure(ctx, cfg, worlds, t_world, unique, headline):
             do_step(actions[t % (K + W)], e)
     ctx.barrier()
     side = torch.cuda.Stream(device=dev)
-    graph = torch.cuda.CUDAGraph()
-    l0 = sum(e.launch_count() for e in envs)
-    with torch.cuda.stream(side):
-        with torch.cuda.graph(graph, stream=side):
-            for t in range(K):
-                do_step(actions[W + t], envs[t % R])
-    launches = sum(e.launch_count() for e in envs) - l0          # kernel nodes of the graph == launches per K steps
-    ctx.barrier()
-    # untimed replays: graph upload, K more warm-up steps, and an estimate of the replay time to size M
-    graph.replay()
-    torch.cuda.synchronize()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record(); graph.replay(); e1.record()
-    torch.cuda.synchronize()
-    est_ms = max(1e-3, float(e0.elapsed_time(e1)))
-    M = int(min(4000, max(7, -(-args.region_ms // est_ms))))
-    if world > 1:                                   # same M on every rank
-        M = int(ctx.gather_rows([float(M)])[:, 0].max())
     sampler = None
     if headline:
         sampler = ClockSampler(ctx.local_rank if "CUDA_VISIBLE_DEVICES" not in os.environ else
                                int(os.environ["CUDA_VISIBLE_DEVICES"].split(",")[ctx.local_rank]))
         sampler.start()
-    evs = [torch.cuda.Event(enable_timing=True) for _ in range(M + 1)]
-    ctx.barrier()
-    if sampler is not None:
         sampler.mark = len(sampler.rows)
-    wall0 = time.perf_counter()
-    evs[0].record()
-    for m in range(M):
-        graph.replay()
-        evs[m + 1].record()
-    ctx.barrier()
-    wall = time.perf_counter() - wall0
-    rep_ms = np.array([evs[m].elapsed_time(evs[m + 1]) for m in range(M)], dtype=np.float64)
-    med_ms, min_ms, max_ms = float(np.median(rep_ms)), float(rep_ms.min()), float(rep_ms.max())
+
+    def timed_replay(g):
+        """One replay of `g` between a CUDA-event pair, barrier + synchronize around it; returns (ms, wall s)."""
+        q0, q1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        ctx.barrier()
+        w0 = time.perf_counter()
+        q0.record(); g.replay(); q1.record()
+        ctx.barrier()
+        return float(q0.elapsed_time(q1)), time.perf_counter() - w0
+
+    # ---- K steps of every env as K launches per replica (one d2d_step per step), replicas interleaved step by step;
+    #      captured as one CUDA graph, replayed once: the timed region holds exactly these K steps of every env
+    rollout_ok = pk["planner"] == "NoMove" and not use_ox and pk.get("motion_profile", "CVM") != "RVO" and args.envs_per_block <= 0
+    graph = torch.cuda.CUDAGraph()
+    l0 = sum(e.launch_count() for e in envs)
+    with torch.cuda.stream(side):
+        with torch.cuda.graph(graph, stream=side):
+            for t in range(K):
+                for e in envs:
+                    do_step(actions[W + t], e)
+    launches = (sum(e.launch_count() for e in envs) - l0) // R     # kernel nodes of the graph per replica
+    dump = None
+    if rollout_ok:
+        ms_graph, wall = None, None               # timed after the headline below (a second K steps of every env)
+    else:
+        ms_graph, wall = timed_replay(graph)
+        if headline and args.dump_outputs and rank == 0:
+            dump = caller_outputs(envs, [ox_next.get(e) for e in envs] if fused_ox else None)
 
     # ---- the same K steps as ONE launch per replica (d2d_rollout): every warp walks its env through the K steps with the
     #      env's working set resident on chip -- the device-resident form of a scripted-gaze run (experiment.py:65-70).
-    #      Replicas are visited round robin exactly as above; the launches are captured once and replayed for >= region-ms.
+    #      The R calls are captured as one CUDA graph after a W-step warm-up call per replica and replayed once.
     rollout = None
-    if pk["planner"] == "NoMove" and not use_ox and pk.get("motion_profile", "CVM") != "RVO" and args.envs_per_block <= 0:
+    if rollout_ok:
+        for e in envs:
+            e.rollout(actions[:W].contiguous())
         act_k = actions[W:W + K].contiguous()
-        for e in envs:                               # warm-up launch per replica (also a K-step continuation of the burn-in)
-            e.rollout(act_k)
-        torch.cuda.synchronize()
         rgraph = torch.cuda.CUDAGraph()
         r0 = sum(e.launch_count() for e in envs)
         with torch.cuda.stream(side):
@@ -417,32 +464,20 @@ def measure(ctx, cfg, worlds, t_world, unique, headline):
                 for e in envs:
                     e.rollout(act_k)
         r_launches = sum(e.launch_count() for e in envs) - r0
-        rgraph.replay()
-        torch.cuda.synchronize()
-        q0, q1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        q0.record(); rgraph.replay(); q1.record()
-        torch.cuda.synchronize()
-        Mr = int(min(4000, max(7, -(-args.region_ms // max(1e-3, float(q0.elapsed_time(q1)))))))
-        if world > 1:
-            Mr = int(ctx.gather_rows([float(Mr)])[:, 0].max())
-        revs = [torch.cuda.Event(enable_timing=True) for _ in range(Mr + 1)]
-        ctx.barrier()
-        revs[0].record()
-        for m in range(Mr):
-            rgraph.replay()
-            revs[m + 1].record()
-        ctx.barrier()
-        r_ms = np.array([revs[m].elapsed_time(revs[m + 1]) for m in range(Mr)], dtype=np.float64) / (K * R)
-        rollout = {"med": float(np.median(r_ms)), "min": float(r_ms.min()), "max": float(r_ms.max()), "replays": Mr,
-                   "launches": int(r_launches), "region_ms": float(r_ms.sum() * K * R),
+        r_ms, wall = timed_replay(rgraph)
+        rollout = {"ms": r_ms / (K * R), "launches": int(r_launches), "region_ms": r_ms,
                    "resident": int(r_launches) == R}     # above two waves of warps d2d_rollout issues K per-step launches
         del rgraph
+        if headline and args.dump_outputs and rank == 0:
+            dump = caller_outputs(envs)
+        ms_graph, _ = timed_replay(graph)
+    ms_launch = ms_graph / (K * R)
 
     per_step = None
     if headline:
         # secondary: the same step timed one launch at a time (CUDA events around every step, 256 MiB L2 flush in between,
         # untimed): includes ~3-4 us of event / launch gap per step; kept for the per-step distribution
-        Kp = min(K, 100)
+        Kp = K
         flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device=dev)
         pe0 = [torch.cuda.Event(enable_timing=True) for _ in range(Kp)]
         pe1 = [torch.cuda.Event(enable_timing=True) for _ in range(Kp)]
@@ -466,7 +501,7 @@ def measure(ctx, cfg, worlds, t_world, unique, headline):
     done_host = torch.empty((B,), dtype=torch.uint8).pin_memory()
     a_rows = [a_host[t] for t in range(K + W)]       # views of the pinned action buffer, one per step
     stage = env.buffer("actions_staging")
-    Ke = int(min(2000, max(K, -(-(0.5 * args.region_ms) // (est_ms / K + 0.02)))))
+    Ke = K
 
     def e2e_step_host(t):
         if use_ox:      # the policy runs on the device: its actions never leave the GPU, the observation still does
@@ -553,15 +588,14 @@ def measure(ctx, cfg, worlds, t_world, unique, headline):
             torch.cuda.synchronize()
         clocks = sampler.stop()
 
-    # ---- over ranks: max of the per-rank medians; every rank's figures are reported
-    rows = ctx.gather_rows([med_ms / K, min_ms / K, max_ms / K, e2e_s * 1e3 / Ke, e2e_copy_s * 1e3 / Ke,
+    # ---- over ranks: the max; every rank's figures are reported
+    rows = ctx.gather_rows([ms_launch, 0.0, 0.0, e2e_s * 1e3 / Ke, e2e_copy_s * 1e3 / Ke,
                             (e2e_mirror_s if e2e_mirror_s is not None else e2e_copy_s) * 1e3 / Ke,
                             (e2e_bound_s if e2e_bound_s is not None else e2e_copy_s) * 1e3 / Ke,
-                            rollout["med"] if rollout else 0.0, rollout["min"] if rollout else 0.0,
-                            rollout["max"] if rollout else 0.0])
+                            rollout["ms"] if rollout else ms_launch])
     ms_launch_per_step = float(rows[:, 0].max())     # K single-step launches
     # headline: the K steps through the fastest device-resident entry point that executes exactly these K steps
-    ms_step = float(rows[:, 7].max()) if rollout else ms_launch_per_step
+    ms_step = float(rows[:, 7].max())
     e2e_ms, e2e_copy_ms, e2e_mirror_ms = float(rows[:, 3].max()), float(rows[:, 4].max()), float(rows[:, 5].max())
     e2e_bound_ms = float(rows[:, 6].max())
     # the one collective of the path: all-reduce of the episode statistics
@@ -592,22 +626,22 @@ def measure(ctx, cfg, worlds, t_world, unique, headline):
     res = {
         "value": value, "unit": "env-steps/s", "ms_per_step": ms_step, "rays_per_sec": value * n_rays,
         "config": public_config(cfg, world),
-        "method": {"timing": (("K = %d steps of every env as ONE d2d_rollout call per replica (%s; R = %d calls captured as a CUDA "
-                              "graph, replayed M = %d times back to back); " % (
+        "method": {"timing": (("K = %d steps of every env as ONE d2d_rollout call per replica (%s; R = %d calls captured as one "
+                              "CUDA graph); " % (
                                   K, "one resident launch" if rollout["resident"] else "K per-step launches: batch above two waves",
-                                  R, rollout["replays"])) if rollout else
-                              ("K = %d steps captured as one CUDA graph (K step launches), replayed M = %d times back to back, " % (K, M))) +
-                             "one CUDA-event pair per replay on the launch stream, barrier + synchronize around the region; "
-                             "per rank the median replay, over ranks the max of the medians",
-                   "graph_replays": rollout["replays"] if rollout else M,
-                   "timed_region_ms_this_rank": rollout["region_ms"] if rollout else float(rep_ms.sum()), "wall_s_timed_region": wall,
+                                  R)) if rollout else
+                              ("K = %d steps of every env as K step launches per replica, replicas interleaved step by step, "
+                               "captured as one CUDA graph; " % K)) +
+                             "the graph replayed once between a CUDA-event pair on the launch stream, barrier + synchronize "
+                             "around it; ms per step = region / (K x R); over ranks the max",
+                   "timed_steps_per_env": K, "graph_replays": 1,
+                   "timed_region_ms_this_rank": rollout["region_ms"] if rollout else ms_launch * K * R, "wall_s_timed_region": wall,
                    "replicas": R, "state_touched_between_visits_mb": round(R * touched / 1e6, 1),
                    "l2": "no rotation (--no-flush): state stays L2-resident" if args.no_flush else L2_NOTE,
                    "burn_in_steps_per_replica": burn, "unique_worlds_per_gpu": int(unique), "world_gen_s": round(t_world, 2),
                    "envs_per_block": int(env.cfg.envs_per_block)},
-        "per_rank": [{"rank": r, "ms_per_step_median": float(rows[r, 7 if rollout else 0]),
-                      "ms_per_step_min": float(rows[r, 8 if rollout else 1]), "ms_per_step_max": float(rows[r, 9 if rollout else 2]),
-                      "single_step_launch_ms_median": float(rows[r, 0]), "e2e_ms_per_step": float(rows[r, 3])} for r in range(world)],
+        "per_rank": [{"rank": r, "ms_per_step": float(rows[r, 7]), "single_step_launch_ms": float(rows[r, 0]),
+                      "e2e_ms_per_step": float(rows[r, 3])} for r in range(world)],
         "e2e": {"value": e2e, "unit": "env-steps/s", "h2d_bytes_per_step": 0 if use_ox else B * 8,
                 "d2h_bytes_per_step": B * (1089 + 4 + 1) if mirror_bytes is None else int(round(B * 5 + mirror_bytes)),
                 "steps": Ke,
@@ -643,14 +677,16 @@ def measure(ctx, cfg, worlds, t_world, unique, headline):
     if rollout:
         res["single_step_launches"] = {
             "value": world * B / (ms_launch_per_step * 1e-3), "ms_per_step": ms_launch_per_step, "gpu_launches": int(launches),
-            "what": "the same K steps as K d2d_step launches (one fused kernel per step, captured as one CUDA graph, M = %d replays): "
-                    "the per-step entry point a device-side policy calls; round-1 / early round-2 headline" % M,
+            "what": "K more steps of every env as K d2d_step launches per replica (one fused kernel per step, captured as one "
+                    "CUDA graph, replayed once): the per-step entry point a device-side policy calls",
             "roofline_frac": algorithmic_bytes(N) * B / (ms_launch_per_step * 1e-3) / 1e9 / peak}
-        res["gpu_launches_note"] = "launches per K steps of ONE replica of the batch (the timed region visits R replicas round robin)"
+        res["gpu_launches_note"] = "launches per K steps of ONE replica of the batch (the timed region steps all R replicas)"
     if per_step is not None:
         res["per_step_events"] = per_step
     if clocks is not None:
         res["clocks"] = clocks
+    if dump is not None:
+        res["dump"] = dump
     del graph
     for e in envs:
         e.close()
@@ -702,7 +738,6 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-workloads", action="store_true", help="headline workload only (skip the `workloads` list)")
     ap.add_argument("--burn-in", type=int, default=1000, help="untimed steps per replica before the timed region")
-    ap.add_argument("--region-ms", type=float, default=100.0, help="minimum length of the timed region per rank")
     ap.add_argument("--no-flush", action="store_true", help="do not rotate replicas (state stays in L2; reported)")
     ap.add_argument("--strip-width", type=int, default=10, help="ray strip width: rays = ceil(500 / strip_width) (config 5 sweep: 10/5/2)")
     ap.add_argument("--view-range", type=int, default=0, help="drone_view_range in degrees (config 5 sweep: 90/180/360)")
@@ -712,7 +747,13 @@ def main():
     ap.add_argument("--e2e-full-copy", action="store_true", help="e2e leg with plain D2H copies instead of the zero-copy mirror")
     ap.add_argument("--gaze", default=None, choices=["scripted", "Oxford"],
                     help="scripted: random actions from the Oxford action set; Oxford: d2d_plan_oxford every step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline path's outputs after its last timed step as DIR/<name>.npy (see the module doc)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.warmup < 3:
         args.warmup = 3
     cfg = make_cfg(args.config, planner=args.planner, gaze=args.gaze, view_range=args.view_range,
@@ -742,7 +783,7 @@ def main():
 
     import torch.distributed as dist
     ctx = Ctx(args)
-    line = None
+    line = dump = None
     workloads = []
     for i, (c, worlds, t_world, unique) in enumerate(gen):
         t0 = time.perf_counter()
@@ -751,6 +792,7 @@ def main():
                                                             time.perf_counter() - t0))
         gen[i] = None                                # release the host arrays of this workload
         if i == 0:
+            dump = res.pop("dump", None)
             line = res
         else:
             workloads.append(res)
@@ -778,6 +820,9 @@ def main():
             v, dt = cpu_port_run(pk, n_envs, steps_c, cores, oxford=use_ox)
             out["cpu_baseline"] = {"value": v, "unit": "env-steps/s", "cores": cores, "kind": "port",
                                    "sample": "%d envs x %d steps of the same workload, auto-reset on (%.1f s)" % (n_envs, steps_c, dt)}
+        if dump is not None:
+            write_dump(args.dump_outputs, dump)
+            log("outputs of the headline path (%d envs) written to %s" % (len(dump["env_index"]), args.dump_outputs))
         emit(out)
     if world > 1:
         dist.destroy_process_group()
