@@ -56,7 +56,7 @@ class D2DBufferInfo(C.Structure):
 
 EXPORTS = ["d2d_version", "d2d_last_error", "d2d_create", "d2d_destroy", "d2d_set_world", "d2d_set_rng", "d2d_set_rvo", "d2d_set_jerk_tables", "d2d_reset", "d2d_request_reset", "d2d_step", "d2d_rollout",
            "d2d_step_host", "d2d_bind_host_mirror", "d2d_bind_host_io", "d2d_step_bound", "d2d_step_pipelined", "d2d_plan_oxford", "d2d_step_plan_oxford", "d2d_step_bound_plan_oxford", "d2d_plan_gaze", "d2d_set_drone_pose", "d2d_get_buffer", "d2d_stats",
-           "d2d_launch_count"]
+           "d2d_launch_count", "d2d_clone_envs", "d2d_state_layout", "d2d_save_state", "d2d_load_state"]
 
 _lib = None
 
@@ -103,6 +103,10 @@ def load():
     L.d2d_stats.argtypes = [vp, vp, C.c_int32, vp]
     L.d2d_launch_count.argtypes = [vp]
     L.d2d_launch_count.restype = C.c_int64
+    L.d2d_clone_envs.argtypes = [vp, vp, vp, C.c_int32, vp]
+    L.d2d_state_layout.argtypes = [vp, C.POINTER(C.c_int64), C.POINTER(C.c_uint64)]
+    L.d2d_save_state.argtypes = [vp, vp, C.c_int32, vp, vp]
+    L.d2d_load_state.argtypes = [vp, vp, C.c_int32, vp, C.c_uint64, vp]
     for name in EXPORTS:
         if name not in ("d2d_version", "d2d_last_error", "d2d_launch_count"):
             getattr(L, name).restype = C.c_int

@@ -14,13 +14,29 @@
 #include "d2d_step.cuh"
 #include "d2d_plan.cuh"
 #include "d2d_rvo.cuh"
+#include "d2d_clone.cuh"
 
 // ------------------------------------------------------------------------------------------ handle
+// Per-env state tag of an arena buffer: env e's row of `row_bytes` bytes starts at offset + e * row_stride, in each of
+// `planes` planes that lie plane_stride bytes apart.  d2d_clone_envs / d2d_save_state / d2d_load_state copy exactly the
+// tagged rows.  planes == 0 (NOT_ENV_STATE): global tables, the statistics, caller data and scratch a step consumes within
+// itself.  add_buf takes the tag as a required argument, so every buffer added later must say which it is.
+struct EnvRows {
+    int64_t row_bytes, row_stride;
+    int planes;
+    int64_t plane_stride;
+};
+static const EnvRows NOT_ENV_STATE = {0, 0, 0, 0};
+static EnvRows env_rows(int64_t row_bytes, int planes = 1, int64_t plane_stride = 0) {
+    return EnvRows{row_bytes, row_bytes, planes, plane_stride};
+}
+
 struct BufDesc {
     std::string name;
     size_t offset, nbytes;
     int dtype, ndim;
     int64_t shape[4], strides[4];
+    EnvRows rows = NOT_ENV_STATE;
 };
 
 struct d2d_handle {
@@ -41,6 +57,12 @@ struct d2d_handle {
     size_t smem_step = 0, smem_post = 0;
     int plan_threads = 64;
     OxProgram *ox_prog = nullptr;
+    CloneTable state_tab;                 // per-env state rows (EnvRows tags) and their packed layout
+    uint64_t state_fingerprint = 0;
+    int *clone_idx = nullptr;             // device copy of the index arrays of the last clone / save / load
+    size_t clone_idx_bytes = 0;
+    std::vector<int32_t> clone_stage;     // host staging of those arrays
+    cudaEvent_t clone_ev = nullptr;       // recorded behind the last kernel that read clone_idx
     double *ox_export = nullptr;          // lazily allocated [B][2500] view of last_time_observed
     // zero-copy observation mirror (d2d_bind_host_mirror): host addresses as bound; *_stale: the host copy must be
     // refreshed by a full device->host copy at the next d2d_step_host (after bind / eager reset)
@@ -117,9 +139,10 @@ static size_t dtype_size(int dt) {
 
 // registers a buffer of `count` rows x inner dims; returns offset
 static size_t add_buf(d2d_handle *h, size_t &cursor, const char *name, int dtype, int ndim,
-                      std::initializer_list<int64_t> shape, std::initializer_list<int64_t> strides, size_t alloc_elems) {
+                      std::initializer_list<int64_t> shape, std::initializer_list<int64_t> strides, size_t alloc_elems,
+                      EnvRows rows) {
     BufDesc b;
-    b.name = name; b.dtype = dtype; b.ndim = ndim;
+    b.name = name; b.dtype = dtype; b.ndim = ndim; b.rows = rows;
     for (int i = 0; i < 4; i++) { b.shape[i] = i < ndim ? shape.begin()[i] : 1; b.strides[i] = i < ndim ? strides.begin()[i] : 1; }
     cursor = (cursor + 255) / 256 * 256;
     b.offset = cursor;
@@ -241,6 +264,47 @@ static void build_ox_program(OxProgram *p, int n) {
     p->lev_off[maxlev] = w;
 }
 
+// ------------------------------------------------------------------------------------------ per-env state layout
+// Bump when the packed state format changes in a way the config does not show (it is part of the fingerprint).
+#define D2D_STATE_LAYOUT_VERSION 1
+
+static uint64_t fnv1a(uint64_t x, const void *p, size_t n) {
+    const unsigned char *c = (const unsigned char *)p;
+    for (size_t i = 0; i < n; i++) { x ^= c[i]; x *= 1099511628211ull; }
+    return x;
+}
+
+// The field table of d2d_clone_kernel from the EnvRows tags (one field per plane; packed rows 16-B aligned, the whole
+// packed state a multiple of 128 B) and the fingerprint of the layout: the config without num_envs / device /
+// envs_per_block (which change neither the rows nor their meaning), the layout version, and every field's name and shape.
+static bool build_state_layout(d2d_handle *h) {
+    CloneTable &T = h->state_tab;
+    memset(&T, 0, sizeof(T));
+    d2d_config c = h->cfg;
+    c.num_envs = 0; c.device = 0; c.envs_per_block = 0;
+    const uint32_t version = D2D_STATE_LAYOUT_VERSION;
+    uint64_t fp = fnv1a(14695981039346656037ull, &version, sizeof(version));
+    fp = fnv1a(fp, &c, sizeof(c));
+    uint64_t pack = 0;
+    for (const BufDesc &b : h->bufs)
+        for (int p = 0; p < b.rows.planes; p++) {
+            if (T.n == D2D_CLONE_MAX_FIELDS) return false;
+            CloneField &f = T.f[T.n++];
+            f.off = b.offset + (uint64_t)p * b.rows.plane_stride;
+            f.stride = (uint64_t)b.rows.row_stride;
+            f.bytes = (unsigned int)b.rows.row_bytes;
+            f.pack = (unsigned int)pack;
+            pack = (pack + f.bytes + 15) / 16 * 16;
+            fp = fnv1a(fp, b.name.c_str(), b.name.size() + 1);
+            fp = fnv1a(fp, &p, sizeof(p));
+            fp = fnv1a(fp, &f.bytes, sizeof(f.bytes));
+            fp = fnv1a(fp, &f.pack, sizeof(f.pack));
+        }
+    T.pack_bytes = (unsigned int)((pack + 127) / 128 * 128);
+    h->state_fingerprint = fnv1a(fp, &T.pack_bytes, sizeof(T.pack_bytes));
+    return true;
+}
+
 // ------------------------------------------------------------------------------------------ create / destroy
 extern "C" int d2d_create(const d2d_config *cfg, d2d_handle **out) {
     if (!cfg || !out) { g_create_err = "null argument"; return D2D_ERR_INVALID; }
@@ -297,26 +361,37 @@ extern "C" int d2d_create(const d2d_config *cfg, d2d_handle **out) {
     memset(&P, 0, sizeof(P));
     const int64_t sB = Bpad;
 #define SHP(...) {__VA_ARGS__}
-    size_t o_apos = add_buf(h, cur, "agent_pos", D2D_F64, 3, SHP(B, N, 2), SHP(NP * 2, 2, 1), (size_t)sB * NP * 2);
-    size_t o_apref = add_buf(h, cur, "agent_pref", D2D_F64, 3, SHP(B, N, 2), SHP(NP * 2, 2, 1), (size_t)sB * NP * 2);
-    size_t o_apos0 = add_buf(h, cur, "agent_pos0", D2D_F64, 3, SHP(B, N, 2), SHP(NP * 2, 2, 1), (size_t)sB * NP * 2);
-    size_t o_apref0 = add_buf(h, cur, "agent_pref0", D2D_F64, 3, SHP(B, N, 2), SHP(NP * 2, 2, 1), (size_t)sB * NP * 2);
+    size_t o_apos = add_buf(h, cur, "agent_pos", D2D_F64, 3, SHP(B, N, 2), SHP(NP * 2, 2, 1), (size_t)sB * NP * 2,
+                            env_rows(NP * 16));
+    size_t o_apref = add_buf(h, cur, "agent_pref", D2D_F64, 3, SHP(B, N, 2), SHP(NP * 2, 2, 1), (size_t)sB * NP * 2,
+                            env_rows(NP * 16));
+    size_t o_apos0 = add_buf(h, cur, "agent_pos0", D2D_F64, 3, SHP(B, N, 2), SHP(NP * 2, 2, 1), (size_t)sB * NP * 2,
+                            env_rows(NP * 16));
+    size_t o_apref0 = add_buf(h, cur, "agent_pref0", D2D_F64, 3, SHP(B, N, 2), SHP(NP * 2, 2, 1), (size_t)sB * NP * 2,
+                            env_rows(NP * 16));
     const bool rvo = cfg->motion_profile == D2D_MOTION_RVO;
     const size_t vel_elems = rvo ? (size_t)sB * NP * 2 : 2;
-    size_t o_avel = add_buf(h, cur, "agent_vel", D2D_F64, 3, SHP(B, N, 2), SHP(NP * 2, 2, 1), vel_elems);
-    size_t o_avel0 = add_buf(h, cur, "agent_vel0", D2D_F64, 3, SHP(B, N, 2), SHP(NP * 2, 2, 1), vel_elems);
-    size_t o_aveln = add_buf(h, cur, "agent_vel_next", D2D_F64, 3, SHP(B, N, 2), SHP(NP * 2, 2, 1), vel_elems);
+    size_t o_avel = add_buf(h, cur, "agent_vel", D2D_F64, 3, SHP(B, N, 2), SHP(NP * 2, 2, 1), vel_elems,
+                            rvo ? env_rows(NP * 16) : NOT_ENV_STATE);
+    size_t o_avel0 = add_buf(h, cur, "agent_vel0", D2D_F64, 3, SHP(B, N, 2), SHP(NP * 2, 2, 1), vel_elems,
+                            rvo ? env_rows(NP * 16) : NOT_ENV_STATE);
+    size_t o_aveln = add_buf(h, cur, "agent_vel_next", D2D_F64, 3, SHP(B, N, 2), SHP(NP * 2, 2, 1), vel_elems, NOT_ENV_STATE);
     size_t o_robs = add_buf(h, cur, "rvo_obstacles", D2D_F64, 3, SHP(B, D2D_RVO_MAX_OBS, 3), SHP(D2D_RVO_MAX_OBS * 3, 3, 1),
-                            rvo ? (size_t)sB * D2D_RVO_MAX_OBS * 3 : 4);
-    size_t o_rnobs = add_buf(h, cur, "rvo_num_obstacles", D2D_I32, 1, SHP(B), SHP(1), sB);
-    size_t o_arad = add_buf(h, cur, "agent_radius", D2D_F64, 2, SHP(B, N), SHP(NP, 1), (size_t)sB * NP);
-    size_t o_trad0 = add_buf(h, cur, "tracker_radius0", D2D_F64, 2, SHP(B, N), SHP(NP, 1), (size_t)sB * NP);
-    size_t o_gt = add_buf(h, cur, "gt_rows", D2D_I64, 2, SHP(B, D2D_GRID), SHP(D2D_GRID, 1), (size_t)sB * D2D_GRID);
+                            rvo ? (size_t)sB * D2D_RVO_MAX_OBS * 3 : 4,
+                            rvo ? env_rows(D2D_RVO_MAX_OBS * 3 * 8) : NOT_ENV_STATE);
+    size_t o_rnobs = add_buf(h, cur, "rvo_num_obstacles", D2D_I32, 1, SHP(B), SHP(1), sB,
+                            rvo ? env_rows(4) : NOT_ENV_STATE);
+    size_t o_arad = add_buf(h, cur, "agent_radius", D2D_F64, 2, SHP(B, N), SHP(NP, 1), (size_t)sB * NP,
+                            env_rows(NP * 8));
+    size_t o_trad0 = add_buf(h, cur, "tracker_radius0", D2D_F64, 2, SHP(B, N), SHP(NP, 1), (size_t)sB * NP,
+                            env_rows(NP * 8));
+    size_t o_gt = add_buf(h, cur, "gt_rows", D2D_I64, 2, SHP(B, D2D_GRID), SHP(D2D_GRID, 1), (size_t)sB * D2D_GRID,
+                            env_rows(D2D_GT_ROW_BYTES));
     size_t o_bel = add_buf(h, cur, "belief", D2D_U8, 3, SHP(B, D2D_GRID, D2D_GRID), SHP(D2D_BELIEF_STRIDE, D2D_GRID, 1),
-                           (size_t)sB * D2D_BELIEF_STRIDE);
+                           (size_t)sB * D2D_BELIEF_STRIDE, env_rows(D2D_BELIEF_STRIDE));
     // per-env scalar state: one 128-byte EnvRec per env; its fields are exposed as strided [B] views
     size_t o_rec = add_buf(h, cur, "env_records", D2D_U8, 2, SHP(B, (int64_t)sizeof(EnvRec)), SHP((int64_t)sizeof(EnvRec), 1),
-                           (size_t)sB * sizeof(EnvRec));
+                           (size_t)sB * sizeof(EnvRec), env_rows(sizeof(EnvRec)));
     {
         const size_t rb = (size_t)sB * sizeof(EnvRec);
         const int64_t s8 = sizeof(EnvRec) / 8, s4 = sizeof(EnvRec) / 4, s1 = sizeof(EnvRec);
@@ -335,56 +410,75 @@ extern "C" int d2d_create(const d2d_config *cfg, d2d_handle **out) {
 #undef RECF
         add_view(h, "drone_pose0", D2D_F64, 2, SHP(3, B), SHP(1, s8), o_rec + offsetof(EnvRec, p0x), rb - offsetof(EnvRec, p0x));
     }
-    size_t o_col = add_buf(h, cur, "collision_flag", D2D_U8, 1, SHP(B), SHP(1), sB);
-    size_t o_dead = add_buf(h, cur, "dead_lock_flag", D2D_U8, 1, SHP(B), SHP(1), sB);
-    size_t o_frz = add_buf(h, cur, "freezing_flag", D2D_U8, 1, SHP(B), SHP(1), sB);
-    size_t o_done = add_buf(h, cur, "done", D2D_U8, 1, SHP(B), SHP(1), sB);
+    size_t o_col = add_buf(h, cur, "collision_flag", D2D_U8, 1, SHP(B), SHP(1), sB, env_rows(1));
+    size_t o_dead = add_buf(h, cur, "dead_lock_flag", D2D_U8, 1, SHP(B), SHP(1), sB, env_rows(1));
+    size_t o_frz = add_buf(h, cur, "freezing_flag", D2D_U8, 1, SHP(B), SHP(1), sB, env_rows(1));
+    size_t o_done = add_buf(h, cur, "done", D2D_U8, 1, SHP(B), SHP(1), sB, env_rows(1));
     size_t o_lm = add_buf(h, cur, "local_map", D2D_U8, 4, SHP(B, 1, D2D_LOCAL, D2D_LOCAL),
-                          SHP(D2D_LOCAL_CELLS, D2D_LOCAL_CELLS, D2D_LOCAL, 1), (size_t)sB * D2D_LOCAL_CELLS);
-    size_t o_yawo = add_buf(h, cur, "yaw_angle", D2D_F32, 2, SHP(B, 1), SHP(1, 1), sB);
-    size_t o_rew = add_buf(h, cur, "reward", D2D_F32, 1, SHP(B), SHP(1), sB);
-    size_t o_hit = add_buf(h, cur, "hit", D2D_I8, 2, SHP(B, N), SHP(NP, 1), (size_t)sB * NP);
-    size_t o_tact = add_buf(h, cur, "tracker_active", D2D_U8, 2, SHP(B, N), SHP(NP, 1), (size_t)sB * NP);
-    size_t o_tmu = add_buf(h, cur, "tracker_mu", D2D_F64, 3, SHP(B, N, 4), SHP(NP * 4, 4, 1), (size_t)sB * NP * 4);
-    size_t o_tsg = add_buf(h, cur, "tracker_sigma", D2D_F64, 4, SHP(B, N, 4, 4), SHP(NP * 16, 16, 4, 1), (size_t)sB * NP * 16);
-    size_t o_trad = add_buf(h, cur, "tracker_radius", D2D_F64, 2, SHP(B, N), SHP(NP, 1), (size_t)sB * NP);
-    size_t o_tts = add_buf(h, cur, "tracker_ts", D2D_I32, 2, SHP(B, N), SHP(NP, 1), (size_t)sB * NP);
+                          SHP(D2D_LOCAL_CELLS, D2D_LOCAL_CELLS, D2D_LOCAL, 1), (size_t)sB * D2D_LOCAL_CELLS, env_rows(D2D_LOCAL_CELLS));
+    size_t o_yawo = add_buf(h, cur, "yaw_angle", D2D_F32, 2, SHP(B, 1), SHP(1, 1), sB, env_rows(4));
+    size_t o_rew = add_buf(h, cur, "reward", D2D_F32, 1, SHP(B), SHP(1), sB, NOT_ENV_STATE);
+    size_t o_hit = add_buf(h, cur, "hit", D2D_I8, 2, SHP(B, N), SHP(NP, 1), (size_t)sB * NP, env_rows(NP));
+    size_t o_tact = add_buf(h, cur, "tracker_active", D2D_U8, 2, SHP(B, N), SHP(NP, 1), (size_t)sB * NP, env_rows(NP));
+    size_t o_tmu = add_buf(h, cur, "tracker_mu", D2D_F64, 3, SHP(B, N, 4), SHP(NP * 4, 4, 1), (size_t)sB * NP * 4,
+                            env_rows(NP * 32));
+    size_t o_tsg = add_buf(h, cur, "tracker_sigma", D2D_F64, 4, SHP(B, N, 4, 4), SHP(NP * 16, 16, 4, 1), (size_t)sB * NP * 16,
+                            env_rows(NP * 128));
+    size_t o_trad = add_buf(h, cur, "tracker_radius", D2D_F64, 2, SHP(B, N), SHP(NP, 1), (size_t)sB * NP,
+                            env_rows(NP * 8));
+    size_t o_tts = add_buf(h, cur, "tracker_ts", D2D_I32, 2, SHP(B, N), SHP(NP, 1), (size_t)sB * NP,
+                            env_rows(NP * 4));
     size_t o_coef = add_buf(h, cur, "traj_coeff", D2D_F64, 3, SHP(B, D2D_MAX_SEGMENTS, 6), SHP(D2D_MAX_SEGMENTS * 6, 6, 1),
-                            cfg->planner == D2D_PLANNER_PRIMITIVE ? (size_t)sB * D2D_MAX_SEGMENTS * 6 : 16);
-    size_t o_need = add_buf(h, cur, "need_plan", D2D_U8, 1, SHP(B), SHP(1), sB);
-    size_t o_pok = add_buf(h, cur, "plan_ok", D2D_U8, 1, SHP(B), SHP(1), sB);
-    size_t o_rep = add_buf(h, cur, "replan", D2D_U8, 1, SHP(B), SHP(1), sB);
-    size_t o_tac = add_buf(h, cur, "tmp_active_count", D2D_I32, 1, SHP(B), SHP(1), sB);
-    size_t o_tat = add_buf(h, cur, "tmp_active_ts", D2D_I32, 1, SHP(B), SHP(1), sB);
+                            cfg->planner == D2D_PLANNER_PRIMITIVE ? (size_t)sB * D2D_MAX_SEGMENTS * 6 : 16,
+                            cfg->planner == D2D_PLANNER_PRIMITIVE ? env_rows(D2D_MAX_SEGMENTS * 6 * 8) : NOT_ENV_STATE);
+    size_t o_need = add_buf(h, cur, "need_plan", D2D_U8, 1, SHP(B), SHP(1), sB, env_rows(1));
+    size_t o_pok = add_buf(h, cur, "plan_ok", D2D_U8, 1, SHP(B), SHP(1), sB, env_rows(1));
+    size_t o_rep = add_buf(h, cur, "replan", D2D_U8, 1, SHP(B), SHP(1), sB, env_rows(1));
+    size_t o_tac = add_buf(h, cur, "tmp_active_count", D2D_I32, 1, SHP(B), SHP(1), sB, NOT_ENV_STATE);
+    size_t o_tat = add_buf(h, cur, "tmp_active_ts", D2D_I32, 1, SHP(B), SHP(1), sB, NOT_ENV_STATE);
     const bool noisy = cfg->var_cam != 0.0;
-    size_t o_rk = add_buf(h, cur, "rng_key", D2D_I32, 2, SHP(B, 624), SHP(624, 1), noisy ? (size_t)sB * 624 : 16);
-    size_t o_rk0 = add_buf(h, cur, "rng_key0", D2D_I32, 2, SHP(B, 624), SHP(624, 1), noisy ? (size_t)sB * 624 : 16);
-    size_t o_rp = add_buf(h, cur, "rng_pos", D2D_I32, 2, SHP(4, B), SHP(B, 1), (size_t)4 * sB);      // pos, pos0, has, has0
-    size_t o_rg = add_buf(h, cur, "rng_gauss", D2D_F64, 2, SHP(2, B), SHP(B, 1), (size_t)2 * sB);     // gauss, gauss0
-    size_t o_oxp = add_buf(h, cur, "oxford_program", D2D_U8, 1, SHP((int64_t)sizeof(OxProgram)), SHP(1), sizeof(OxProgram));
+    size_t o_rk = add_buf(h, cur, "rng_key", D2D_I32, 2, SHP(B, 624), SHP(624, 1), noisy ? (size_t)sB * 624 : 16,
+                            noisy ? env_rows(624 * 4) : NOT_ENV_STATE);
+    size_t o_rk0 = add_buf(h, cur, "rng_key0", D2D_I32, 2, SHP(B, 624), SHP(624, 1), noisy ? (size_t)sB * 624 : 16,
+                            noisy ? env_rows(624 * 4) : NOT_ENV_STATE);
+    size_t o_rp = add_buf(h, cur, "rng_pos", D2D_I32, 2, SHP(4, B), SHP(B, 1), (size_t)4 * sB,      // pos, pos0, has, has0
+                          env_rows(4, 4, sB * 4));
+    size_t o_rg = add_buf(h, cur, "rng_gauss", D2D_F64, 2, SHP(2, B), SHP(B, 1), (size_t)2 * sB,     // gauss, gauss0
+                          env_rows(8, 2, sB * 8));
+    size_t o_oxp = add_buf(h, cur, "oxford_program", D2D_U8, 1, SHP((int64_t)sizeof(OxProgram)), SHP(1), sizeof(OxProgram),
+                            NOT_ENV_STATE);
     size_t o_oxs = add_buf(h, cur, "oxford_seen_call", D2D_I32, 1, SHP(1), SHP(1),
-                           (cfg->oxford & D2D_POLICY_OXFORD) ? (size_t)sB * D2D_OX_SEEN_STRIDE / 2 : 4);   // uint16 [B][2560]
-    size_t o_oxc = add_buf(h, cur, "oxford_calls", D2D_I32, 1, SHP(B), SHP(1), sB);
-    size_t o_oxt = add_buf(h, cur, "oxford_tables", D2D_F64, 2, SHP(2, D2D_OX_TAB), SHP(D2D_OX_TAB, 1), 2 * D2D_OX_TAB);
+                           (cfg->oxford & D2D_POLICY_OXFORD) ? (size_t)sB * D2D_OX_SEEN_STRIDE / 2 : 4,   // uint16 [B][2560]
+                           (cfg->oxford & D2D_POLICY_OXFORD) ? env_rows(D2D_OX_SEEN_STRIDE * 2) : NOT_ENV_STATE);
+    size_t o_oxc = add_buf(h, cur, "oxford_calls", D2D_I32, 1, SHP(B), SHP(1), sB, env_rows(4));
+    size_t o_oxt = add_buf(h, cur, "oxford_tables", D2D_F64, 2, SHP(2, D2D_OX_TAB), SHP(D2D_OX_TAB, 1), 2 * D2D_OX_TAB,
+                            NOT_ENV_STATE);
     const bool owl = (cfg->oxford & D2D_POLICY_OWL) != 0;
-    size_t o_owlU = add_buf(h, cur, "owl_U", D2D_F64, 2, SHP(B, D2D_OWL_BINS), SHP(D2D_OWL_BINS, 1), owl ? (size_t)sB * D2D_OWL_BINS : 2);
-    size_t o_owlq = add_buf(h, cur, "owl_queue_len", D2D_I32, 1, SHP(B), SHP(1), sB);
-    size_t o_owlu = add_buf(h, cur, "owl_queue_value", D2D_F64, 1, SHP(B), SHP(1), sB);
-    size_t o_dacc = add_buf(h, cur, "drone_acc", D2D_F64, 2, SHP(B, 2), SHP(2, 1), (size_t)sB * 2);
+    size_t o_owlU = add_buf(h, cur, "owl_U", D2D_F64, 2, SHP(B, D2D_OWL_BINS), SHP(D2D_OWL_BINS, 1), owl ? (size_t)sB * D2D_OWL_BINS : 2,
+                            owl ? env_rows(D2D_OWL_BINS * 8) : NOT_ENV_STATE);
+    size_t o_owlq = add_buf(h, cur, "owl_queue_len", D2D_I32, 1, SHP(B), SHP(1), sB, env_rows(4));
+    size_t o_owlu = add_buf(h, cur, "owl_queue_value", D2D_F64, 1, SHP(B), SHP(1), sB, env_rows(8));
+    size_t o_dacc = add_buf(h, cur, "drone_acc", D2D_F64, 2, SHP(B, 2), SHP(2, 1), (size_t)sB * 2, env_rows(16));
     size_t o_jerk = add_buf(h, cur, "jerk_tables", D2D_U8, 1, SHP((int64_t)sizeof(d2d_jerk_tables)), SHP(1),
-                            cfg->planner == D2D_PLANNER_JERK ? sizeof(d2d_jerk_tables) : 16);
-    size_t o_stats = add_buf(h, cur, "stats", D2D_I64, 1, SHP(D2D_NUM_STATS), SHP(1), D2D_NUM_STATS);
-    size_t o_tab = add_buf(h, cur, "tables", D2D_U8, 1, SHP((int64_t)sizeof(DevTables)), SHP(1), sizeof(DevTables));
-    size_t o_stage = add_buf(h, cur, "actions_staging", D2D_F64, 1, SHP(B), SHP(1), sB + 8);   // + the stamp slot of the resident gated kernel
+                            cfg->planner == D2D_PLANNER_JERK ? sizeof(d2d_jerk_tables) : 16, NOT_ENV_STATE);
+    size_t o_stats = add_buf(h, cur, "stats", D2D_I64, 1, SHP(D2D_NUM_STATS), SHP(1), D2D_NUM_STATS, NOT_ENV_STATE);
+    size_t o_tab = add_buf(h, cur, "tables", D2D_U8, 1, SHP((int64_t)sizeof(DevTables)), SHP(1), sizeof(DevTables),
+                            NOT_ENV_STATE);
+    // caller data (+ the stamp slot of the resident gated kernel): not env state
+    size_t o_stage = add_buf(h, cur, "actions_staging", D2D_F64, 1, SHP(B), SHP(1), sB + 8, NOT_ENV_STATE);
     size_t o_plan_ws = 0;
     size_t plan_ws_bytes = 0;
     if (cfg->planner == D2D_PLANNER_PRIMITIVE) {
         plan_ws_bytes = d2d_plan_workspace_bytes(cfg->n_u) * (size_t)D2D_PLAN_SLOTS;
-        o_plan_ws = add_buf(h, cur, "plan_workspace", D2D_U8, 1, SHP((int64_t)plan_ws_bytes), SHP(1), plan_ws_bytes);
+        o_plan_ws = add_buf(h, cur, "plan_workspace", D2D_U8, 1, SHP((int64_t)plan_ws_bytes), SHP(1), plan_ws_bytes,
+                            NOT_ENV_STATE);
     }
-    size_t o_plan_list = add_buf(h, cur, "plan_list", D2D_I32, 1, SHP(B + 8), SHP(1), sB + 8);
-    size_t o_plan_over = add_buf(h, cur, "plan_overflow", D2D_I32, 1, SHP(B + 8), SHP(1), sB + 8);
+    size_t o_plan_list = add_buf(h, cur, "plan_list", D2D_I32, 1, SHP(B + 8), SHP(1), sB + 8, NOT_ENV_STATE);
+    size_t o_plan_over = add_buf(h, cur, "plan_overflow", D2D_I32, 1, SHP(B + 8), SHP(1), sB + 8, NOT_ENV_STATE);
 #undef SHP
+    if (!build_state_layout(h)) {
+        g_create_err = "per-env state: more than " + std::to_string(D2D_CLONE_MAX_FIELDS) + " rows"; delete h; return D2D_ERR_INVALID;
+    }
     h->arena_bytes = (cur + 255) / 256 * 256;
     ce = cudaMalloc((void **)&h->arena, h->arena_bytes);
     if (ce != cudaSuccess) {
@@ -532,6 +626,8 @@ extern "C" int d2d_destroy(d2d_handle *h) {
     for (int i = 0; i < 3; i++) if (h->pipe_ev[i]) cudaEventDestroy(h->pipe_ev[i]);
     if (h->arena) cudaFree(h->arena);
     if (h->ox_export) cudaFree(h->ox_export);
+    if (h->clone_idx) cudaFree(h->clone_idx);
+    if (h->clone_ev) cudaEventDestroy(h->clone_ev);
     delete h;
     return D2D_OK;
 }
@@ -1228,6 +1324,124 @@ extern "C" int d2d_stats(d2d_handle *h, int64_t *out_host, int32_t reset, void *
     CUDA_TRY(h, cudaMemcpyAsync(out_host, h->P.stats, D2D_NUM_STATS * 8, cudaMemcpyDeviceToHost, st));
     if (reset) CUDA_TRY(h, cudaMemsetAsync(h->P.stats, 0, D2D_NUM_STATS * 8, st));
     CUDA_TRY(h, cudaStreamSynchronize(st));
+    return D2D_OK;
+}
+
+// ------------------------------------------------------------------------------------------ per-env state: clone / save / load
+extern "C" int d2d_state_layout(const d2d_handle *h, int64_t *bytes_per_env, uint64_t *fingerprint) {
+    if (!h) return D2D_ERR_INVALID;
+    if (bytes_per_env) *bytes_per_env = h->state_tab.pack_bytes;
+    if (fingerprint) *fingerprint = h->state_fingerprint;
+    return D2D_OK;
+}
+
+// Host index arrays: every entry in [0, num_envs); `written` (dst of a clone, envs of a load) without repeats, and no env
+// both read and written.  Checked before anything is enqueued.
+static int check_env_indices(d2d_handle *h, const char *what, const int32_t *read, const int32_t *written, int32_t count) {
+    std::vector<uint8_t> w(written ? (size_t)h->B : 0, 0);
+    for (int32_t i = 0; written && i < count; i++) {
+        const int32_t e = written[i];
+        if (e < 0 || e >= h->B) { h->err = std::string(what) + ": env index " + std::to_string(e) + " out of range"; return D2D_ERR_INVALID; }
+        if (w[e]) { h->err = std::string(what) + ": env " + std::to_string(e) + " is written twice"; return D2D_ERR_INVALID; }
+        w[e] = 1;
+    }
+    for (int32_t i = 0; read && i < count; i++) {
+        const int32_t e = read[i];
+        if (e < 0 || e >= h->B) { h->err = std::string(what) + ": env index " + std::to_string(e) + " out of range"; return D2D_ERR_INVALID; }
+        if (written && w[e]) { h->err = std::string(what) + ": env " + std::to_string(e) + " is both a source and a destination"; return D2D_ERR_INVALID; }
+    }
+    return D2D_OK;
+}
+
+// A packed state buffer must be device memory of the handle's device, 16-B aligned.
+static int check_state_ptr(d2d_handle *h, const char *what, const void *p) {
+    if (!p) { h->err = std::string(what) + ": null state buffer"; return D2D_ERR_INVALID; }
+    if (((uintptr_t)p & 15) != 0) { h->err = std::string(what) + ": the state buffer must be 16-byte aligned"; return D2D_ERR_INVALID; }
+    cudaPointerAttributes at;
+    if (cudaPointerGetAttributes(&at, p) != cudaSuccess || at.type != cudaMemoryTypeDevice || at.device != h->cfg.device) {
+        cudaGetLastError();
+        h->err = std::string(what) + ": the state buffer is not device memory of device " + std::to_string(h->cfg.device);
+        return D2D_ERR_INVALID;
+    }
+    return D2D_OK;
+}
+
+// One launch of d2d_clone_kernel over `count` copies.  The index arrays go to a per-handle device buffer with one copy on
+// `stream`; an event recorded behind each kernel that reads the buffer makes the next call's stream wait before it
+// overwrites the buffer, so consecutive calls on different streams never race on it.
+static int launch_clone(d2d_handle *h, int mode, const int32_t *src_host, const int32_t *dst_host, int32_t count,
+                        unsigned char *packed, cudaStream_t st) {
+    const int nidx = (src_host ? 1 : 0) + (dst_host ? 1 : 0);
+    const size_t need = (size_t)nidx * count * 4;
+    if (!h->clone_ev) CUDA_TRY(h, cudaEventCreateWithFlags(&h->clone_ev, cudaEventDisableTiming));
+    if (need > h->clone_idx_bytes) {
+        CUDA_TRY(h, cudaEventSynchronize(h->clone_ev));          // the old buffer may still be read by an earlier kernel
+        if (h->clone_idx) CUDA_TRY(h, cudaFree(h->clone_idx));
+        h->clone_idx = nullptr; h->clone_idx_bytes = 0;
+        CUDA_TRY(h, cudaMalloc((void **)&h->clone_idx, need));
+        h->clone_idx_bytes = need;
+    }
+    int *idx = h->clone_idx;
+    if (need) {
+        h->clone_stage.resize((size_t)nidx * count);
+        if (src_host) memcpy(h->clone_stage.data(), src_host, (size_t)count * 4);
+        if (dst_host) memcpy(h->clone_stage.data() + (src_host ? (size_t)count : 0), dst_host, (size_t)count * 4);
+        CUDA_TRY(h, cudaStreamWaitEvent(st, h->clone_ev, 0));
+        CUDA_TRY(h, cudaMemcpyAsync(idx, h->clone_stage.data(), need, cudaMemcpyHostToDevice, st));
+    }
+    const int *src = src_host ? idx : nullptr, *dst = dst_host ? idx + (src_host ? count : 0) : nullptr;
+    d2d_clone_kernel<<<count, D2D_CLONE_THREADS, 0, st>>>(h->state_tab, mode, h->arena, packed, src, dst);
+    h->launches++;
+    CUDA_TRY(h, cudaGetLastError());
+    CUDA_TRY(h, cudaEventRecord(h->clone_ev, st));
+    return D2D_OK;
+}
+
+extern "C" int d2d_clone_envs(d2d_handle *h, const int32_t *src_host, const int32_t *dst_host, int32_t count, void *stream) {
+    if (!h) return D2D_ERR_INVALID;
+    D2D_NO_PIPE(h);
+    if (!h->world_set) { h->err = "d2d_clone_envs before d2d_set_world"; return D2D_ERR_STATE; }
+    if (count < 0 || (count > 0 && (!src_host || !dst_host))) { h->err = "d2d_clone_envs: bad count or null index array"; return D2D_ERR_INVALID; }
+    int rc = check_env_indices(h, "d2d_clone_envs", src_host, dst_host, count);
+    if (rc != D2D_OK || count == 0) return rc;
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    rc = launch_clone(h, D2D_CLONE_ARENA, src_host, dst_host, count, nullptr, (cudaStream_t)stream);
+    if (rc != D2D_OK) return rc;
+    h->mir_stale = true;          // the clone rewrites the device observation only
+    return D2D_OK;
+}
+
+extern "C" int d2d_save_state(d2d_handle *h, const int32_t *envs_host, int32_t count, void *state_dev, void *stream) {
+    if (!h) return D2D_ERR_INVALID;
+    D2D_NO_PIPE(h);
+    if (!h->world_set) { h->err = "d2d_save_state before d2d_set_world"; return D2D_ERR_STATE; }
+    if (count < 0 || (!envs_host && count > h->B)) { h->err = "d2d_save_state: bad count"; return D2D_ERR_INVALID; }
+    int rc = check_env_indices(h, "d2d_save_state", envs_host, nullptr, count);
+    if (rc != D2D_OK || count == 0) return rc;
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    if ((rc = check_state_ptr(h, "d2d_save_state", state_dev)) != D2D_OK) return rc;
+    return launch_clone(h, D2D_CLONE_SAVE, envs_host, nullptr, count, (unsigned char *)state_dev, (cudaStream_t)stream);
+}
+
+extern "C" int d2d_load_state(d2d_handle *h, const int32_t *envs_host, int32_t count, const void *state_dev,
+                              uint64_t fingerprint, void *stream) {
+    if (!h) return D2D_ERR_INVALID;
+    D2D_NO_PIPE(h);
+    if (!h->world_set) { h->err = "d2d_load_state before d2d_set_world"; return D2D_ERR_STATE; }
+    if (count < 0 || (!envs_host && count > h->B)) { h->err = "d2d_load_state: bad count"; return D2D_ERR_INVALID; }
+    if (fingerprint != h->state_fingerprint) {
+        h->err = "d2d_load_state: the state was saved from a handle with another layout (fingerprint mismatch)";
+        return D2D_ERR_INVALID;
+    }
+    int rc = check_env_indices(h, "d2d_load_state", nullptr, envs_host, count);
+    if (rc != D2D_OK || count == 0) return rc;
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    if ((rc = check_state_ptr(h, "d2d_load_state", state_dev)) != D2D_OK) return rc;
+    std::vector<int32_t> all;
+    if (!envs_host) { all.resize(count); for (int32_t i = 0; i < count; i++) all[i] = i; envs_host = all.data(); }
+    rc = launch_clone(h, D2D_CLONE_LOAD, nullptr, envs_host, count, (unsigned char *)state_dev, (cudaStream_t)stream);
+    if (rc != D2D_OK) return rc;
+    h->mir_stale = true;
     return D2D_OK;
 }
 

@@ -270,6 +270,15 @@ class Drone2DEnv2(object):
         state = {"local_map": lm, "swep_map": lm.copy(), "yaw_angle": obs["yaw_angle"][0].cpu().numpy()}
         return state, 0, bool(done[0].item()), self.info
 
+    # ---- state snapshots (ALE cloneState / restoreState, MuJoCo get_state / set_state)
+    def get_state(self):
+        """A snapshot of the whole env -- live state and reset snapshot -- as returned by Drone2DVecEnv.save_state."""
+        return self._vec.save_state([0])
+
+    def set_state(self, s):
+        """Restores a snapshot of `get_state` (of this env or of one with the same params); later steps repeat bit for bit."""
+        self._vec.load_state(s, [0])
+
     def render(self, mode="human"):
         raise NotImplementedError("rendering (pygame) is out of scope of the B200 path; see DESIGN.md §7")
 

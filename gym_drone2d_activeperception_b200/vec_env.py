@@ -371,6 +371,76 @@ class Drone2DVecEnv(object):
         self._check(self._lib.d2d_set_drone_pose(self._h, pose.ctypes.data_as(C.c_void_p), self._stream()),
                     "d2d_set_drone_pose")
 
+    # ------------------------------------------------------------------ per-env state (clone / save / load)
+    @staticmethod
+    def _env_indices(x):
+        """int sequence, numpy array or CPU tensor -> contiguous int32 numpy array (range checks are the library's)."""
+        if torch.is_tensor(x):
+            if x.device.type != "cpu":
+                raise ValueError("env indices must be a host sequence, numpy array or CPU tensor")
+            x = x.numpy()
+        a = np.asarray(x).reshape(-1)
+        if a.size and a.dtype.kind not in "iu":
+            raise ValueError("env indices must be integers, got %s" % a.dtype)
+        a = a.astype(np.int64)
+        if a.size and (a.min() < -2 ** 31 or a.max() >= 2 ** 31):
+            raise _native.Drone2DNativeError("env index out of range")
+        return np.ascontiguousarray(a, dtype=np.int32)
+
+    def state_layout(self):
+        """(bytes per env of a packed state row, 64-bit layout fingerprint) -- d2d_state_layout."""
+        nbytes, fp = C.c_int64(), C.c_uint64()
+        self._check(self._lib.d2d_state_layout(self._h, C.byref(nbytes), C.byref(fp)), "d2d_state_layout")
+        return int(nbytes.value), int(fp.value)
+
+    def clone_envs(self, src, dst):
+        """Env dst[i] becomes an exact copy of env src[i], live state and reset snapshot (d2d_clone_envs, one kernel):
+        with the same actions every later step, reset and policy call of dst[i] is bit-identical to src[i]'s.  src may
+        repeat an env (fork it into several copies); dst must not, and no env may be in both.  The clone's reset target came
+        with it, so `seeds[dst] = seeds[src]`.  Actions kept in "actions_staging" are caller data and are not copied: re-plan
+        after a clone when stepping with `step_bound_plan_oxford`."""
+        s, d = self._env_indices(src), self._env_indices(dst)
+        if s.size != d.size:
+            raise ValueError("clone_envs: %d sources for %d destinations" % (s.size, d.size))
+        self._check(self._lib.d2d_clone_envs(self._h, s.ctypes.data_as(C.c_void_p), d.ctypes.data_as(C.c_void_p), int(s.size),
+                                             self._stream()), "d2d_clone_envs")
+        self.seeds[d] = self.seeds[s]
+
+    def save_state(self, envs=None):
+        """Packs the state of `envs` (default: all) into a uint8 CUDA tensor [count, bytes_per_env] (d2d_save_state).
+        Returns {"fingerprint": int, "state": tensor, "seeds": int64 array}; the state tensor may be moved (`.cpu()`,
+        `torch.save`, `.to("cuda:k")`) and is loaded with `load_state` into any env with the same fingerprint."""
+        nbytes, fp = self.state_layout()
+        idx = None if envs is None else self._env_indices(envs)
+        count = self.num_envs if idx is None else int(idx.size)
+        state = torch.zeros((count, nbytes), dtype=torch.uint8, device=self.device)
+        self._check(self._lib.d2d_save_state(self._h, None if idx is None else idx.ctypes.data_as(C.c_void_p), count,
+                                             C.c_void_p(state.data_ptr()), self._stream()), "d2d_save_state")
+        seeds = self.seeds.copy() if idx is None else self.seeds[idx]
+        return {"fingerprint": fp, "state": state, "seeds": np.asarray(seeds, dtype=np.int64)}
+
+    def load_state(self, saved, envs=None):
+        """Writes row i of `saved["state"]` into env envs[i] (default: envs 0..count-1) -- d2d_load_state.  The state must
+        be a uint8 tensor [count, bytes_per_env] on this env's device; the library rejects a state of another layout
+        (fingerprint).  Seeds travel with the state."""
+        nbytes, _ = self.state_layout()
+        state = saved["state"]
+        if not torch.is_tensor(state) or state.dtype != torch.uint8 or state.dim() != 2 or state.shape[1] != nbytes:
+            raise ValueError("load_state: expected a uint8 tensor [count, %d]" % nbytes)
+        if state.device.type != "cuda" or state.device.index != self._dev_index:
+            raise ValueError("load_state: the state is on %s, this env is on cuda:%d (move it with .to())"
+                             % (state.device, self._dev_index))
+        state = state.contiguous()
+        count = int(state.shape[0])
+        idx = None if envs is None else self._env_indices(envs)
+        if idx is not None and idx.size != count:
+            raise ValueError("load_state: %d rows for %d envs" % (count, idx.size))
+        self._check(self._lib.d2d_load_state(self._h, None if idx is None else idx.ctypes.data_as(C.c_void_p), count,
+                                             C.c_void_p(state.data_ptr()), C.c_uint64(int(saved["fingerprint"])),
+                                             self._stream()), "d2d_load_state")
+        if saved.get("seeds") is not None:
+            self.seeds[np.arange(count) if idx is None else idx] = np.asarray(saved["seeds"], dtype=np.int64)
+
     def plan_oxford(self, out=None):
         """Oxford.plan for every env (yaw_planner.py:81-127): returns float64 CUDA tensor [B] of actions."""
         if out is None:

@@ -292,6 +292,39 @@ int d2d_get_buffer(d2d_handle *h, const char *name, d2d_buffer_info *out);
  * counters to out_host (synchronises the stream).  The multi-GPU host all-reduces this vector (NCCL). */
 int d2d_stats(d2d_handle *h, int64_t *out_host, int32_t reset, void *stream);
 
+/* Per-env state copies, the counterpart of ALE cloneState / restoreState and MuJoCo get_state / set_state: branch an env
+ * into copies, checkpoint and replay it, move it to another handle or GPU.  The state of an env is every per-env arena row:
+ * the live state AND its reset snapshot (agents and their *0 rows, RVO velocities and obstacles, radii, ground truth,
+ * belief, the 128-byte env record verbatim -- pending_reset included --, the step outputs and flags, trackers, trajectory,
+ * planner verdicts, the np.random stream with its reset copy, Oxford / Owl policy state, drone acceleration).  Not part of
+ * it: global tables, the statistics, the constant reward, scratch a step consumes within itself, and "actions_staging",
+ * which holds caller data -- a caller that keeps the next actions there (d2d_step_bound_plan_oxford) must re-plan
+ * (d2d_plan_oxford) after a clone or load.
+ * d2d_clone_envs, d2d_save_state and d2d_load_state return D2D_ERR_STATE before d2d_set_world and while a pipelined step
+ * is in flight, and check every argument before anything is enqueued (a rejected call changes nothing).  Each is ONE kernel
+ * launch on `stream`.  Clone and load mark the host observation mirror stale, so the next host step refreshes it with one
+ * full copy (as after d2d_reset). */
+
+/* Env dst[i] becomes an exact copy of env src[i] (i < count): live state AND reset snapshot, so every later step,
+ * auto/lazy reset and policy call of dst[i] is bit-identical to what src[i] would do with the same actions.
+ * src_host / dst_host: HOST int32 arrays, validated before anything is enqueued (0 <= index < num_envs, dst entries
+ * distinct, no index in both arrays; src entries may repeat: one env forks into several).  Statistics are not touched.
+ * count = 0 does nothing.  One kernel launch. */
+int d2d_clone_envs(d2d_handle *h, const int32_t *src_host, const int32_t *dst_host, int32_t count, void *stream);
+
+/* Size of one env's packed state (a multiple of 128 B) and a 64-bit fingerprint of everything that decides the layout
+ * or its meaning: d2d_config without num_envs / device / envs_per_block, plus a layout version.  Any handle, any time. */
+int d2d_state_layout(const d2d_handle *h, int64_t *bytes_per_env, uint64_t *fingerprint);
+
+/* Packs envs[i] into row i of a DEVICE buffer [count][bytes_per_env] (envs_host NULL: envs 0..count-1; entries may
+ * repeat), and back: d2d_load_state writes row i into env envs[i] (entries distinct).  state_dev: device memory of the
+ * handle's device, 16-byte aligned (else D2D_ERR_INVALID).  The packed rows can be moved anywhere (host, file, another
+ * GPU) and loaded into any handle whose fingerprint matches; a different fingerprint is D2D_ERR_INVALID.  Padding bytes
+ * between the fields of a packed row are left as they were. */
+int d2d_save_state(d2d_handle *h, const int32_t *envs_host, int32_t count, void *state_dev, void *stream);
+int d2d_load_state(d2d_handle *h, const int32_t *envs_host, int32_t count, const void *state_dev,
+                   uint64_t fingerprint, void *stream);
+
 /* Number of kernel launches issued by this handle so far (bench.py's gpu_launches). */
 int64_t d2d_launch_count(const d2d_handle *h);
 
