@@ -49,6 +49,20 @@ class D2DJerkTables(C.Structure):
     ]
 
 
+WORLD_MAX_RANDOM, WORLD_MAX_PILLARS, WORLD_GROUPS = 256, 64, 100
+WORLD_EAGER, WORLD_LAZY = 1, 2
+
+
+class D2DWorldSource(C.Structure):
+    _fields_ = [
+        ("struct_size", C.c_int32), ("agent_number", C.c_int32), ("pillar_number", C.c_int32), ("pad_", C.c_int32),
+        ("agent_radius", C.c_double), ("agent_max_speed", C.c_double), ("drone_radius", C.c_double),
+        ("init_x", C.c_double), ("init_y", C.c_double), ("map_w", C.c_double), ("map_h", C.c_double),
+        ("headings", (C.c_double * 2) * WORLD_MAX_RANDOM),
+        ("static_map", (C.c_uint8 * 50) * 50),
+    ]
+
+
 class D2DBufferInfo(C.Structure):
     _fields_ = [("dev_ptr", C.c_void_p), ("nbytes", C.c_int64), ("dtype", C.c_int32), ("ndim", C.c_int32),
                 ("shape", C.c_int64 * 4), ("strides", C.c_int64 * 4)]
@@ -56,7 +70,8 @@ class D2DBufferInfo(C.Structure):
 
 EXPORTS = ["d2d_version", "d2d_last_error", "d2d_create", "d2d_destroy", "d2d_set_world", "d2d_set_rng", "d2d_set_rvo", "d2d_set_jerk_tables", "d2d_reset", "d2d_request_reset", "d2d_step", "d2d_rollout",
            "d2d_step_host", "d2d_bind_host_mirror", "d2d_bind_host_io", "d2d_step_bound", "d2d_step_pipelined", "d2d_plan_oxford", "d2d_step_plan_oxford", "d2d_step_bound_plan_oxford", "d2d_plan_gaze", "d2d_set_drone_pose", "d2d_get_buffer", "d2d_stats",
-           "d2d_launch_count", "d2d_clone_envs", "d2d_state_layout", "d2d_save_state", "d2d_load_state"]
+           "d2d_launch_count", "d2d_clone_envs", "d2d_state_layout", "d2d_save_state", "d2d_load_state",
+           "d2d_set_world_source", "d2d_generate_worlds"]
 
 _lib = None
 
@@ -107,6 +122,8 @@ def load():
     L.d2d_state_layout.argtypes = [vp, C.POINTER(C.c_int64), C.POINTER(C.c_uint64)]
     L.d2d_save_state.argtypes = [vp, vp, C.c_int32, vp, vp]
     L.d2d_load_state.argtypes = [vp, vp, C.c_int32, vp, C.c_uint64, vp]
+    L.d2d_set_world_source.argtypes = [vp, C.POINTER(D2DWorldSource)]
+    L.d2d_generate_worlds.argtypes = [vp, vp, vp, C.c_int32, C.c_int32, vp]
     for name in EXPORTS:
         if name not in ("d2d_version", "d2d_last_error", "d2d_launch_count"):
             getattr(L, name).restype = C.c_int

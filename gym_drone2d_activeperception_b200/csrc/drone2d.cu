@@ -15,6 +15,7 @@
 #include "d2d_plan.cuh"
 #include "d2d_rvo.cuh"
 #include "d2d_clone.cuh"
+#include "d2d_worldgen.cuh"
 
 // ------------------------------------------------------------------------------------------ handle
 // Per-env state tag of an arena buffer: env e's row of `row_bytes` bytes starts at offset + e * row_stride, in each of
@@ -64,6 +65,14 @@ struct d2d_handle {
     std::vector<int32_t> clone_stage;     // host staging of those arrays
     cudaEvent_t clone_ev = nullptr;       // recorded behind the last kernel that read clone_idx
     double *ox_export = nullptr;          // lazily allocated [B][2500] view of last_time_observed
+    // world generation (d2d_set_world_source / d2d_generate_worlds)
+    WgTables *wg_tab = nullptr;           // device copy of the seed-independent tables
+    int32_t *wg_idx = nullptr;            // device: [count] envs, [count] seeds (u32), [num_envs] eager reset mask
+    size_t wg_idx_bytes = 0;
+    std::vector<int32_t> wg_stage;        // host staging of those arrays
+    cudaEvent_t wg_ev = nullptr;          // recorded behind the last kernel that read wg_idx
+    volatile unsigned long long *wg_fault = nullptr;   // pinned, mapped: (1 << 63 | env << 32 | seed) of a world given up
+    unsigned long long *wg_fault_dev = nullptr;        // device-visible address of wg_fault
     // zero-copy observation mirror (d2d_bind_host_mirror): host addresses as bound; *_stale: the host copy must be
     // refreshed by a full device->host copy at the next d2d_step_host (after bind / eager reset)
     uint8_t *mir_lm = nullptr; float *mir_yaw = nullptr; uint8_t *mir_done = nullptr;
@@ -628,6 +637,10 @@ extern "C" int d2d_destroy(d2d_handle *h) {
     if (h->ox_export) cudaFree(h->ox_export);
     if (h->clone_idx) cudaFree(h->clone_idx);
     if (h->clone_ev) cudaEventDestroy(h->clone_ev);
+    if (h->wg_tab) cudaFree(h->wg_tab);
+    if (h->wg_idx) cudaFree(h->wg_idx);
+    if (h->wg_ev) cudaEventDestroy(h->wg_ev);
+    if (h->wg_fault) cudaFreeHost((void *)h->wg_fault);
     delete h;
     return D2D_OK;
 }
@@ -1442,6 +1455,95 @@ extern "C" int d2d_load_state(d2d_handle *h, const int32_t *envs_host, int32_t c
     rc = launch_clone(h, D2D_CLONE_LOAD, nullptr, envs_host, count, (unsigned char *)state_dev, (cudaStream_t)stream);
     if (rc != D2D_OK) return rc;
     h->mir_stale = true;
+    return D2D_OK;
+}
+
+// ------------------------------------------------------------------------------------------ world generation
+extern "C" int d2d_set_world_source(d2d_handle *h, const d2d_world_source *src) {
+    if (!h) return D2D_ERR_INVALID;
+    if (!src) { h->err = "d2d_set_world_source: null source"; return D2D_ERR_INVALID; }
+    D2D_NO_PIPE(h);
+    std::vector<unsigned char> tmp(sizeof(WgTables));
+    WgTables *T = (WgTables *)tmp.data();
+    const char *bad = wg_build_tables(T, src, h->cfg.targets, h->cfg.n_targets, h->cfg.map_scale, h->N, h->P.motion_rvo,
+                                      h->cfg.var_cam != 0.0 ? 1 : 0);
+    if (bad) { h->err = std::string("d2d_set_world_source: ") + bad; return D2D_ERR_INVALID; }
+    if (src->map_w != h->cfg.map_w || src->map_h != h->cfg.map_h || src->drone_radius != h->cfg.drone_radius ||
+        src->agent_radius != h->cfg.agent_radius) {
+        h->err = "d2d_set_world_source: map size, drone_radius or agent_radius differ from the config"; return D2D_ERR_INVALID;
+    }
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    if (!h->wg_tab) CUDA_TRY(h, cudaMalloc((void **)&h->wg_tab, sizeof(WgTables)));
+    if (!h->wg_fault) {
+        CUDA_TRY(h, cudaHostAlloc((void **)&h->wg_fault, sizeof(unsigned long long), cudaHostAllocMapped));
+        *h->wg_fault = 0ull;
+        CUDA_TRY(h, cudaHostGetDevicePointer((void **)&h->wg_fault_dev, (void *)h->wg_fault, 0));
+    }
+    if (h->wg_ev) CUDA_TRY(h, cudaEventSynchronize(h->wg_ev));     // no generation kernel may still read the old tables
+    CUDA_TRY(h, cudaMemcpy(h->wg_tab, T, sizeof(WgTables), cudaMemcpyHostToDevice));
+    return D2D_OK;
+}
+
+extern "C" int d2d_generate_worlds(d2d_handle *h, const int32_t *envs_host, const int64_t *seeds_host, int32_t count,
+                                   int32_t flags, void *stream) {
+    if (!h) return D2D_ERR_INVALID;
+    D2D_NO_PIPE(h);
+    if (!h->wg_tab) { h->err = "d2d_generate_worlds before d2d_set_world_source"; return D2D_ERR_STATE; }
+    const unsigned long long fault = *h->wg_fault;
+    if (fault) {
+        *h->wg_fault = 0ull;
+        h->err = "d2d_generate_worlds: the world of seed " + std::to_string((unsigned)(fault & 0xffffffffull)) + " (env " +
+                 std::to_string((int)((fault >> 32) & 0x7fffffffull)) + ") could not be built: more than " +
+                 std::to_string(D2D_WORLD_MAX_REJECTS) + " rejected draws in a row; that env's world is undefined";
+        return D2D_ERR_STATE;
+    }
+    if (flags != D2D_WORLD_EAGER && flags != D2D_WORLD_LAZY) {
+        h->err = "d2d_generate_worlds: flags must be D2D_WORLD_EAGER or D2D_WORLD_LAZY"; return D2D_ERR_INVALID;
+    }
+    if (count < 0 || (count > 0 && (!envs_host || !seeds_host))) { h->err = "d2d_generate_worlds: bad count or null array"; return D2D_ERR_INVALID; }
+    int rc = check_env_indices(h, "d2d_generate_worlds", nullptr, envs_host, count);
+    if (rc != D2D_OK) return rc;
+    for (int32_t i = 0; i < count; i++)
+        if (seeds_host[i] < 0 || seeds_host[i] > 0xffffffffll) {
+            h->err = "d2d_generate_worlds: seed " + std::to_string((long long)seeds_host[i]) + " outside [0, 2**32)";
+            return D2D_ERR_INVALID;
+        }
+    if (count == 0) return D2D_OK;
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const bool eager = flags == D2D_WORLD_EAGER;
+    // envs, seeds and (eager) the reset mask in one staged copy; the event keeps the next call from overwriting the device
+    // buffer while a kernel still reads it (as launch_clone does)
+    const size_t words = 2 * (size_t)count + (eager ? ((size_t)h->B + 3) / 4 : 0);
+    if (!h->wg_ev) CUDA_TRY(h, cudaEventCreateWithFlags(&h->wg_ev, cudaEventDisableTiming));
+    if (words * 4 > h->wg_idx_bytes) {
+        CUDA_TRY(h, cudaEventSynchronize(h->wg_ev));
+        if (h->wg_idx) CUDA_TRY(h, cudaFree(h->wg_idx));
+        h->wg_idx = nullptr; h->wg_idx_bytes = 0;
+        CUDA_TRY(h, cudaMalloc((void **)&h->wg_idx, words * 4));
+        h->wg_idx_bytes = words * 4;
+    }
+    h->wg_stage.assign(words, 0);
+    memcpy(h->wg_stage.data(), envs_host, (size_t)count * 4);
+    for (int32_t i = 0; i < count; i++) h->wg_stage[(size_t)count + i] = (int32_t)(uint32_t)seeds_host[i];
+    uint8_t *mask = (uint8_t *)(h->wg_stage.data() + 2 * (size_t)count);
+    if (eager) for (int32_t i = 0; i < count; i++) mask[envs_host[i]] = 1;
+    CUDA_TRY(h, cudaStreamWaitEvent(st, h->wg_ev, 0));
+    CUDA_TRY(h, cudaMemcpyAsync(h->wg_idx, h->wg_stage.data(), words * 4, cudaMemcpyHostToDevice, st));
+    d2d_worldgen_kernel<<<(count + D2D_WG_WARPS - 1) / D2D_WG_WARPS, D2D_WG_WARPS * 32, 0, st>>>(
+        h->P, h->wg_tab, h->wg_idx, (const uint32_t *)(h->wg_idx + count), count, eager ? 0 : 1, h->wg_fault_dev);
+    h->launches++;
+    CUDA_TRY(h, cudaGetLastError());
+    if (eager) {
+        d2d_reset_kernel<<<h->B, 128, 0, st>>>(h->P, (const uint8_t *)(h->wg_idx + 2 * (size_t)count));
+        h->launches++;
+        CUDA_TRY(h, cudaGetLastError());
+        h->mir_stale = true;      // the eager reset rewrites the device observation only
+    }
+    CUDA_TRY(h, cudaEventRecord(h->wg_ev, st));
+    h->world_set = true;
+    if (h->cfg.var_cam != 0.0) h->rng_set = true;
+    if (h->P.motion_rvo) h->rvo_set = true;
     return D2D_OK;
 }
 

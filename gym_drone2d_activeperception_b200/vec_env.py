@@ -13,7 +13,7 @@ import torch
 
 from . import _native
 from .params import Params
-from .world import count_agents, generate_worlds, load_static_map
+from .world import count_agents, generate_worlds, load_static_map, world_source
 
 _TORCH_DTYPES = {0: (torch.uint8, "|u1"), 1: (torch.int8, "|i1"), 2: (torch.int32, "<i4"), 3: (torch.int64, "<i8"),
                  4: (torch.float32, "<f4"), 5: (torch.float64, "<f8")}
@@ -132,12 +132,19 @@ class Drone2DVecEnv(object):
     worlds    : optional pre-generated worlds (dict of arrays as returned by world.generate_worlds)
     auto_reset: an env that returned done=True is re-initialised (same seed => same world, exactly what the
                 reference's reset() does) at the start of its next step; the terminal observation is returned.
+    world_gen : "host" (default) builds the worlds with world.generate_worlds and uploads them; "device" generates them
+                on the GPU (d2d_generate_worlds), identical except for the documented group-velocity rounding (DESIGN.md
+                section 2).  `reseed` needs neither.  Cannot be combined with `worlds`.
     """
 
     metadata = {"render.modes": []}
 
     def __init__(self, params, num_envs, seeds=None, device="cuda:0", auto_reset=True, trackers=True, oxford=None,
-                 envs_per_block=0, strip_width=10, worlds=None, owl=None, jerk_tie_orders=None):
+                 envs_per_block=0, strip_width=10, worlds=None, owl=None, jerk_tie_orders=None, world_gen="host"):
+        if world_gen not in ("host", "device"):
+            raise ValueError("world_gen must be 'host' or 'device', got %r" % (world_gen,))
+        if world_gen == "device" and worlds is not None:
+            raise ValueError("world_gen='device' generates the worlds itself: do not pass `worlds`")
         if not torch.cuda.is_available():
             raise _native.Drone2DNativeError("CUDA device required: Drone2DVecEnv has no CPU path")
         self.params = params
@@ -163,10 +170,17 @@ class Drone2DVecEnv(object):
             from . import jerk
             self._jerk_tables = jerk.make_tables(params, jerk_tie_orders)
             self._check(self._lib.d2d_set_jerk_tables(self._h, C.byref(self._jerk_tables)), "d2d_set_jerk_tables")
-        self.seeds = np.asarray(seeds if seeds is not None else params.map_id + np.arange(self.num_envs), dtype=np.int64)
-        if worlds is None:
-            worlds = generate_worlds(params, self.seeds, self._smap)
-        self.set_worlds(worlds)
+        # a copy: reseed / clone_envs / load_state rewrite entries, and must not write into the caller's array
+        self.seeds = np.array(seeds if seeds is not None else params.map_id + np.arange(self.num_envs), dtype=np.int64)
+        self._world_source = None
+        if world_gen == "device":
+            self.reseed(np.arange(self.num_envs), self.seeds)
+            torch.cuda.current_stream(self.device).synchronize()
+            self.check_worlds()
+        else:
+            if worlds is None:
+                worlds = generate_worlds(params, self.seeds, self._smap)
+            self.set_worlds(worlds)
         self._views = {}
         self._mirror, self._mirror_ptrs = None, (None, None, None)
         self.local_map_size = 4 * (params.drone_view_depth // params.map_scale) + 1
@@ -207,6 +221,35 @@ class Drone2DVecEnv(object):
             rk = [p(w["rng_key"], np.uint32), p(w["rng_pos"], np.int32), p(w["rng_has_gauss"], np.int32),
                   p(w["rng_gauss"], np.float64)]
             self._check(self._lib.d2d_set_rng(self._h, first_env, count, *[k[1] for k in rk]), "d2d_set_rng")
+
+    def reseed(self, envs, seeds, lazy=False):
+        """Gives envs[i] the world of seeds[i], generated on the GPU (d2d_generate_worlds, one launch, asynchronous):
+        lazy=False resets those envs now, as `reset` does; lazy=True marks them, and each starts its new world at its next
+        step -- the path auto-reset takes after done, so the terminal outputs of an env that just reported done stay
+        readable until then.  Afterwards `seeds[e]` is the seed of the world env e resets into.  Seeds must lie in
+        [0, 2**32), as np.random.RandomState requires.  A seed whose world cannot be built is reported by the next call or
+        by `check_worlds`."""
+        idx = self._env_indices(envs)
+        sd = np.asarray(seeds).reshape(-1)
+        if sd.size and sd.dtype.kind not in "iu":
+            raise ValueError("seeds must be integers, got %s" % sd.dtype)
+        sd = np.ascontiguousarray(sd, dtype=np.int64)
+        if sd.size != idx.size:
+            raise ValueError("reseed: %d seeds for %d envs" % (sd.size, idx.size))
+        if self._world_source is None:
+            src = world_source(self.params, self._smap)
+            self._check(self._lib.d2d_set_world_source(self._h, C.byref(src)), "d2d_set_world_source")
+            self._world_source = src
+        flags = _native.WORLD_LAZY if lazy else _native.WORLD_EAGER
+        self._check(self._lib.d2d_generate_worlds(self._h, idx.ctypes.data_as(C.c_void_p), sd.ctypes.data_as(C.c_void_p),
+                                                  int(idx.size), flags, self._stream()), "d2d_generate_worlds")
+        self.seeds[idx] = sd
+
+    def check_worlds(self):
+        """Raises if an earlier `reseed` met a seed whose world cannot be built (call after synchronising the stream)."""
+        if self._world_source is not None:
+            self._check(self._lib.d2d_generate_worlds(self._h, None, None, 0, _native.WORLD_EAGER, self._stream()),
+                        "d2d_generate_worlds")
 
     def buffer(self, name):
         """Torch tensor aliasing the named arena buffer (see DESIGN.md / d2d_get_buffer)."""

@@ -155,6 +155,34 @@ def generate_world(params, seed, static_map=None):
                 obstacles=np.array(obstacles, dtype=np.float64).reshape(len(obstacles), 3))
 
 
+def world_source(params, static_map=None):
+    """The seed-independent inputs of generate_world as the d2d_world_source struct of d2d_set_world_source: the counts,
+    radii, speed, init position and map size, the static map's group ids, and the random agents' headings evaluated with
+    the same NumPy expression generate_world uses."""
+    from ._native import D2DWorldSource, WORLD_MAX_RANDOM, WORLD_MAX_PILLARS, WORLD_GROUPS
+    import ctypes as C
+    smap = load_static_map(params.static_map if static_map is None else static_map)
+    n_rand = int(params.agent_number)
+    if not 0 <= n_rand <= WORLD_MAX_RANDOM:
+        raise ValueError("device world generation: at most %d random agents (agent_number)" % WORLD_MAX_RANDOM)
+    if not 0 <= int(params.pillar_number) <= WORLD_MAX_PILLARS:
+        raise ValueError("device world generation: at most %d pillars (pillar_number)" % WORLD_MAX_PILLARS)
+    if smap.shape != (50, 50) or smap.min() < 0 or smap.max() >= WORLD_GROUPS or np.any(smap != np.floor(smap)):
+        raise ValueError("device world generation: the static map must be 50x50 integral group ids in [0, %d)" % WORLD_GROUPS)
+    s = D2DWorldSource()
+    s.struct_size = C.sizeof(D2DWorldSource)
+    s.agent_number, s.pillar_number = n_rand, int(params.pillar_number)
+    s.agent_radius, s.agent_max_speed, s.drone_radius = params.agent_radius, params.agent_max_speed, params.drone_radius
+    s.init_x, s.init_y = params.init_position
+    s.map_w, s.map_h = params.map_size
+    for k in range(n_rand):          # generate_world's heading table, element for element
+        h = -params.agent_max_speed * np.array([np.cos(2 * np.pi * k / n_rand), np.sin(2 * np.pi * k / n_rand)])
+        s.headings[k][0], s.headings[k][1] = float(h[0]), float(h[1])
+    groups = np.ascontiguousarray(smap, dtype=np.uint8)
+    C.memmove(C.addressof(s.static_map), groups.ctypes.data, groups.nbytes)
+    return s
+
+
 def _initial_velocities(agent_pref, agent_number):
     """Agent.velocity right after __init__: `(0., 0.)` for the random agents (drone_v2.py:19), the group velocity for the
     map-cell agents (drone_v2.py:62).  Only read under the RVO motion profile (CVM overwrites it with pref_velocity)."""

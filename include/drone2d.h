@@ -325,6 +325,57 @@ int d2d_save_state(d2d_handle *h, const int32_t *envs_host, int32_t count, void 
 int d2d_load_state(d2d_handle *h, const int32_t *envs_host, int32_t count, const void *state_dev,
                    uint64_t fingerprint, void *stream);
 
+/* World generation on the device: the world of a seed, as init_obstacles_random_size + OccupancyGridMap.init_obstacles
+ * build it (drone_v2.py:12-66, utils.py:508-525) and world.generate_world restates it, generated by the GPU instead of the
+ * host.  d2d_world_source holds the seed-independent inputs; the seed decides the rest through the reference's two
+ * streams, Python's `random.Random(seed)` (pillars, agent positions and radii) and `np.random.RandomState(seed)` (the 100
+ * group headings, then the measurement noise).  The result is what d2d_set_world / d2d_set_rng / d2d_set_rvo would store
+ * for the host-generated world of that seed, bit for bit, except for the static-map group velocities: the reference
+ * evaluates agent_max_speed * np.cos / np.sin(direction) with glibc, the device with correctly rounded sin / cos (they
+ * differ by 1 ulp in about 0.1 % of the directions; DESIGN.md section 2). */
+#define D2D_WORLD_MAX_RANDOM 256      /* random disc agents (params.agent_number) */
+#define D2D_WORLD_MAX_PILLARS 64      /* params.pillar_number (at most 16 under the RVO motion profile) */
+#define D2D_WORLD_GROUPS 100          /* group ids of the static map: np.random.rand(100) headings (drone_v2.py:54) */
+#define D2D_WORLD_EAGER 1             /* reset the envs now, as d2d_reset does */
+#define D2D_WORLD_LAZY 2              /* mark the envs (pending_reset): they start the new world at their next step */
+
+typedef struct d2d_world_source {
+    int32_t struct_size;              /* sizeof(d2d_world_source), ABI check */
+    int32_t agent_number;             /* random disc agents, placed by rejection (drone_v2.py:28-47) */
+    int32_t pillar_number;            /* circular obstacles, placed first (drone_v2.py:14-26) */
+    int32_t pad_;
+    double agent_radius;              /* params.agent_radius; -1: random radii uniform(5, 15) */
+    double agent_max_speed;
+    double drone_radius;
+    double init_x, init_y;            /* params.init_position: the drone's reset pose (yaw 270) */
+    double map_w, map_h;              /* params.map_size */
+    /* the random agents' preferred velocities -v * [cos, sin](2 pi k / agent_number) as the host's NumPy evaluates them */
+    double headings[D2D_WORLD_MAX_RANDOM][2];
+    /* the static map (params.static_map), [x][y]: 0 = free, else the group id of the radius-5 agent on that cell, < 100 */
+    uint8_t static_map[50][50];
+} d2d_world_source;
+
+/* Stores the seed-independent inputs (HOST struct, copied).  Once per handle.  Checked against the config: the map must be
+ * the config's, agent_number + the non-zero cells of static_map == num_agents, and under RVO pillar_number <= 16. */
+int d2d_set_world_source(d2d_handle *h, const d2d_world_source *src);
+
+/* Generates the worlds of seeds_host[i] into envs envs_host[i] (HOST arrays, i < count) in ONE launch on `stream`,
+ * asynchronously.  Writes the reset snapshot (agents and their *0 rows, radii, ground truth, the reset pose, the np.random
+ * stream when var_cam != 0, the RVO velocities and obstacles) and then, by `flags`:
+ *   D2D_WORLD_EAGER  resets the envs as d2d_reset does (a second launch) and marks the host mirror stale;
+ *   D2D_WORLD_LAZY   marks them like d2d_request_reset: each starts the new world at its next step.  Under auto_reset this is
+ *                    what happens to an env that just reported done; its terminal outputs stay readable until that step,
+ *                    and a gaze policy called in between already sees the new initial state.
+ * Everything is checked before anything is enqueued (a rejected call changes nothing): envs in [0, num_envs) and distinct,
+ * seeds in [0, 2^32) (np.random.RandomState rejects anything else), exactly one flag.  D2D_ERR_STATE before
+ * d2d_set_world_source and while a pipelined step is in flight.  Statistics are untouched; the first call counts as
+ * d2d_set_world (+ d2d_set_rng / d2d_set_rvo).
+ * A seed whose world cannot be built (the reference's rejection loops would never end: more than 65536 rejected draws in a
+ * row) is recorded by the kernel; the NEXT call reports it with D2D_ERR_STATE (env and seed in d2d_last_error), clears it
+ * and does nothing else.  count = 0 enqueues nothing: after synchronising the stream it reports such a failure at once. */
+int d2d_generate_worlds(d2d_handle *h, const int32_t *envs_host, const int64_t *seeds_host, int32_t count, int32_t flags,
+                        void *stream);
+
 /* Number of kernel launches issued by this handle so far (bench.py's gpu_launches). */
 int64_t d2d_launch_count(const d2d_handle *h);
 
