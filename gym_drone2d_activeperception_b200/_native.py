@@ -3,6 +3,8 @@ a call fails, an exception is raised."""
 import ctypes as C
 import os
 
+import numpy as np
+
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("D2D_LIB") or os.path.join(HERE, "libdrone2d.so")     # D2D_LIB: an A/B build of the same ABI (tools/)
 
@@ -63,6 +65,21 @@ class D2DWorldSource(C.Structure):
     ]
 
 
+class D2DEpisodeRecord(C.Structure):
+    """d2d_episode_record (drone2d.h): one finished episode of the episode log."""
+    _fields_ = [("seed", C.c_int64), ("step", C.c_int64), ("tracked_steps", C.c_int64), ("env", C.c_int32),
+                ("steps", C.c_int32), ("grid_discovered", C.c_int32), ("trackers", C.c_int32),
+                ("state_machine", C.c_uint8), ("collision_flag", C.c_uint8), ("freezing_flag", C.c_uint8),
+                ("dead_lock_flag", C.c_uint8), ("reserved", C.c_int32)]
+
+
+# the same record as a numpy structured dtype (what Drone2DVecEnv.read_episodes returns)
+EPISODE_DTYPE = np.dtype({"names": [f[0] for f in D2DEpisodeRecord._fields_],
+                          "formats": ["<i8", "<i8", "<i8", "<i4", "<i4", "<i4", "<i4", "u1", "u1", "u1", "u1", "<i4"],
+                          "offsets": [getattr(D2DEpisodeRecord, f[0]).offset for f in D2DEpisodeRecord._fields_],
+                          "itemsize": C.sizeof(D2DEpisodeRecord)})
+
+
 class D2DBufferInfo(C.Structure):
     _fields_ = [("dev_ptr", C.c_void_p), ("nbytes", C.c_int64), ("dtype", C.c_int32), ("ndim", C.c_int32),
                 ("shape", C.c_int64 * 4), ("strides", C.c_int64 * 4)]
@@ -71,7 +88,8 @@ class D2DBufferInfo(C.Structure):
 EXPORTS = ["d2d_version", "d2d_last_error", "d2d_create", "d2d_destroy", "d2d_set_world", "d2d_set_rng", "d2d_set_rvo", "d2d_set_jerk_tables", "d2d_reset", "d2d_request_reset", "d2d_step", "d2d_rollout",
            "d2d_step_host", "d2d_bind_host_mirror", "d2d_bind_host_io", "d2d_step_bound", "d2d_step_pipelined", "d2d_plan_oxford", "d2d_step_plan_oxford", "d2d_step_bound_plan_oxford", "d2d_plan_gaze", "d2d_set_drone_pose", "d2d_get_buffer", "d2d_stats",
            "d2d_launch_count", "d2d_clone_envs", "d2d_state_layout", "d2d_save_state", "d2d_load_state",
-           "d2d_set_world_source", "d2d_generate_worlds"]
+           "d2d_set_world_source", "d2d_generate_worlds", "d2d_enable_episode_log", "d2d_read_episode_log",
+           "d2d_set_seed_queue"]
 
 _lib = None
 
@@ -124,6 +142,9 @@ def load():
     L.d2d_load_state.argtypes = [vp, vp, C.c_int32, vp, C.c_uint64, vp]
     L.d2d_set_world_source.argtypes = [vp, C.POINTER(D2DWorldSource)]
     L.d2d_generate_worlds.argtypes = [vp, vp, vp, C.c_int32, C.c_int32, vp]
+    L.d2d_enable_episode_log.argtypes = [vp, C.c_int64]
+    L.d2d_read_episode_log.argtypes = [vp, vp, C.POINTER(C.c_int64), C.POINTER(C.c_int64), vp]
+    L.d2d_set_seed_queue.argtypes = [vp, vp, C.c_int64, vp]
     for name in EXPORTS:
         if name not in ("d2d_version", "d2d_last_error", "d2d_launch_count"):
             getattr(L, name).restype = C.c_int

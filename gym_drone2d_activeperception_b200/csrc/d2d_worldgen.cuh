@@ -322,6 +322,7 @@ __device__ __forceinline__ double wg_random(uint32_t *mt, int &pos, int lane) {
 
 // One warp per generated world: envs[w] gets the world of seeds[w].  lazy: also mark the env pending_reset.  A placement
 // that exceeds D2D_WORLD_MAX_REJECTS stores (1 << 63 | env << 32 | seed) into *fault (mapped host word) and abandons the env.
+// The body is shared with d2d_worldgen_list_kernel through d2d_worldgen_body.inc.
 __global__ void __launch_bounds__(D2D_WG_WARPS * 32) d2d_worldgen_kernel(const DevP P, const WgTables *__restrict__ Tg,
                                                                           const int *__restrict__ envs,
                                                                           const uint32_t *__restrict__ seeds, int count, int lazy,
@@ -330,122 +331,30 @@ __global__ void __launch_bounds__(D2D_WG_WARPS * 32) d2d_worldgen_kernel(const D
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int w = blockIdx.x * D2D_WG_WARPS + wid;
     if (w >= count) return;
-    WgWarp &S = sh[wid];
-    const WgTables &T = *Tg;
-    const d2d_world_source &s = T.src;
-    const int e = envs[w];
-    const uint32_t seed = seeds[w];
-    const size_t base = (size_t)e * P.NP;
-    double *apos = (double *)(P.apos0 + base), *apref = (double *)(P.apref0 + base);
-    double *arad = P.arad + base, *trad = P.trk_radius0 + base;
-    const int W = (int)s.map_w, H = (int)s.map_h;
+#define WG_ABANDON return
+#include "d2d_worldgen_body.inc"
+#undef WG_ABANDON
+}
 
-    if (lane == 0) wg_init_by_array1(S.mt, T.mt_base, seed);
-    __syncwarp();
-    int pos = D2D_MT_N;
-    // pillars (drone_v2.py:14-26): every lane draws and decides the same
-    int npil = 0;
-    for (int rej = 0; npil < s.pillar_number;) {
-        const int x = wg_randint(S.mt, pos, lane, 50, W - 50);
-        const int y = wg_randint(S.mt, pos, lane, 50, H - 50);
-        const int r = wg_randint(S.mt, pos, lane, 15, 20);
-        if (wg_pillar_free(T, x, y, r)) {
-            if (lane == 0) { S.pil[npil][0] = x; S.pil[npil][1] = y; S.pil[npil][2] = r; }
-            npil++; rej = 0;
-        } else if (++rej > D2D_WORLD_MAX_REJECTS) {
-            if (lane == 0) *fault = (1ull << 63) | ((unsigned long long)e << 32) | seed;
-            return;
+// The worlds the seed queue handed out in the step just logged (d2d_episode_log_kernel): list and count are device data, so
+// the launch needs no host round trip and can be captured in a graph.  Grid-stride over warps; always lazy.
+__global__ void __launch_bounds__(D2D_WG_WARPS * 32) d2d_worldgen_list_kernel(const DevP P, const WgTables *__restrict__ Tg,
+                                                                               const int *__restrict__ envs,
+                                                                               const uint32_t *__restrict__ seeds,
+                                                                               const int *__restrict__ count,
+                                                                               volatile unsigned long long *fault) {
+    __shared__ WgWarp sh[D2D_WG_WARPS];
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const int lazy = 1;
+    const int n = *count;
+    for (int w = blockIdx.x * D2D_WG_WARPS + wid; w < n; w += gridDim.x * D2D_WG_WARPS) {
+        __syncwarp();                    // every lane is done with the previous world's shared memory
+        {
+#define WG_ABANDON goto next_world
+#include "d2d_worldgen_body.inc"
+#undef WG_ABANDON
         }
-    }
-    __syncwarp();
-    // random agents (drone_v2.py:28-47): lanes test the accepted agents and the pillars in parallel
-    const double rlo = s.agent_radius == -1.0 ? 5.0 : s.agent_radius - 2.0, rhi = s.agent_radius == -1.0 ? 15.0 : s.agent_radius + 2.0;
-    for (int k = 0, rej = 0; k < s.agent_number;) {
-        const double px = wg_uniform(20.0, (double)(W - 20), wg_random(S.mt, pos, lane));
-        const double py = wg_uniform(20.0, (double)(H - 20), wg_random(S.mt, pos, lane));
-        const double r = wg_uniform(rlo, rhi, wg_random(S.mt, pos, lane));
-        bool hit = lane == 0 && wg_hits_drone(T, px, py);
-        for (int j = lane; j < k; j += 32) hit |= wg_hits_agent(px, py, r, apos[2 * j], apos[2 * j + 1], arad[j]);
-        for (int q = lane; q < npil; q += 32) hit |= wg_hits_pillar(px, py, r, S.pil[q][0], S.pil[q][1], S.pil[q][2]);
-        if (!__any_sync(0xffffffffu, hit)) {
-            if (lane == 0) {
-                apos[2 * k] = px; apos[2 * k + 1] = py;
-                apref[2 * k] = s.headings[k][0]; apref[2 * k + 1] = s.headings[k][1];
-                arad[k] = r; trad[k] = r;
-            }
-            __syncwarp();                // the next candidate's lanes read this agent
-            k++; rej = 0;
-        } else if (++rej > D2D_WORLD_MAX_REJECTS) {
-            if (lane == 0) *fault = (1ull << 63) | ((unsigned long long)e << 32) | seed;
-            return;
-        }
-    }
-    // the NumPy stream: 100 headings -> group velocities, static-map agents (drone_v2.py:49-66), noise stream snapshot
-    if (T.need_np) {
-        __syncwarp();
-        if (lane == 0) wg_init_genrand(S.mt, seed);
-        __syncwarp();
-        wg_twist_warp(S.mt, lane);
-        for (int g = lane; g < D2D_WORLD_GROUPS; g += 32)
-            wg_group_velocity(s.agent_max_speed, wg_temper(S.mt[2 * g]), wg_temper(S.mt[2 * g + 1]), S.vel[g][0], S.vel[g][1]);
-        if (T.noisy) {
-            uint32_t *key = P.rng_key0 + (size_t)e * D2D_MT_N;
-            for (int i = lane; i < D2D_MT_N; i += 32) key[i] = S.mt[i];
-            if (lane == 0) { P.rng_pos0[e] = 200; P.rng_has0[e] = 0; P.rng_gauss0[e] = 0.0; }
-        }
-        __syncwarp();
-        for (int m = lane; m < T.n_map; m += 32) {
-            const int k = s.agent_number + m, g = T.map_group[m], c = T.map_cell[m];
-            apos[2 * k] = (double)(5 + (c / 50) * 10); apos[2 * k + 1] = (double)(5 + (c % 50) * 10);
-            apref[2 * k] = S.vel[g][0]; apref[2 * k + 1] = S.vel[g][1];
-            arad[k] = 5.0; trad[k] = s.agent_radius;
-        }
-    }
-    // ground truth (utils.py:508-525): border + pillar discs, minus the cells whose centre lies in an agent disc
-    for (int i = lane; i < D2D_WG_GRID; i += 32) {
-        unsigned long long row = (i == 0 || i == D2D_WG_GRID - 1) ? ((1ull << D2D_WG_GRID) - 1)
-                                                                              : (1ull | (1ull << 49));
-        for (int q = 0; q < npil; q++) {
-            int i0, i1, j0, j1;
-            wg_pillar_range(T, S.pil[q][0], S.pil[q][2], i0, i1);
-            if (i < i0 || i >= i1) continue;
-            wg_pillar_range(T, S.pil[q][1], S.pil[q][2], j0, j1);
-            for (int j = j0; j < j1; j++)
-                if (wg_pillar_cell(T, i, j, S.pil[q][0], S.pil[q][1], S.pil[q][2])) row |= 1ull << j;
-        }
-        S.occ[i] = row;
-        S.erase[i] = 0ull;
-    }
-    __syncwarp();
-    for (int k = lane; k < T.N; k += 32) {
-        const double ax = apos[2 * k], ay = apos[2 * k + 1], r = arad[k];
-        int i0, i1, j0, j1;
-        wg_cover_range(T, ax, r, i0, i1);
-        wg_cover_range(T, ay, r, j0, j1);
-        for (int i = i0; i < i1; i++) {
-            unsigned long long m = 0ull;
-            for (int j = j0; j < j1; j++)
-                if (wg_cell_covered(T, i, j, ax, ay, r)) m |= 1ull << j;
-            if (m) atomicOr(&S.erase[i], m);
-        }
-    }
-    __syncwarp();
-    for (int i = lane; i < D2D_WG_GRID; i += 32) P.gt_rows[(size_t)e * D2D_GRID + i] = S.occ[i] & ~S.erase[i];
-    if (T.rvo) {
-        double2 *v0 = P.avel0 + base;
-        for (int k = lane; k < T.N; k += 32)
-            v0[k] = k < s.agent_number ? make_double2(0.0, 0.0) : make_double2(apref[2 * k], apref[2 * k + 1]);
-        double *ob = P.rvo_obs + (size_t)e * D2D_RVO_MAX_OBS * 3;
-        for (int q = lane; q < D2D_RVO_MAX_OBS; q += 32) {
-            ob[3 * q] = q < npil ? (double)S.pil[q][0] : 0.0;
-            ob[3 * q + 1] = q < npil ? (double)S.pil[q][1] : 0.0;
-            ob[3 * q + 2] = q < npil ? (double)S.pil[q][2] : 0.0;
-        }
-        if (lane == 0) P.rvo_nobs[e] = npil;
-    }
-    if (lane == 0) {
-        P.rec[e].p0x = s.init_x; P.rec[e].p0y = s.init_y; P.rec[e].p0yaw = 270.0;     // yaw = -90 % 360 (utils.py:718)
-        if (lazy) P.rec[e].pending_reset = 1;
+    next_world:;
     }
 }
 #endif

@@ -16,6 +16,7 @@
 #include "d2d_rvo.cuh"
 #include "d2d_clone.cuh"
 #include "d2d_worldgen.cuh"
+#include "d2d_episode.cuh"
 
 // ------------------------------------------------------------------------------------------ handle
 // Per-env state tag of an arena buffer: env e's row of `row_bytes` bytes starts at offset + e * row_stride, in each of
@@ -73,6 +74,14 @@ struct d2d_handle {
     cudaEvent_t wg_ev = nullptr;          // recorded behind the last kernel that read wg_idx
     volatile unsigned long long *wg_fault = nullptr;   // pinned, mapped: (1 << 63 | env << 32 | seed) of a world given up
     unsigned long long *wg_fault_dev = nullptr;        // device-visible address of wg_fault
+    // episode log and seed queue (d2d_enable_episode_log / d2d_set_seed_queue); ep_mem == nullptr: disabled
+    unsigned char *ep_mem = nullptr;      // records, head, world_seed, list, gen_env, gen_seed, gen_count in one allocation
+    EpLog ep = {};
+    long long *ep_queue = nullptr;        // device copy of the queue
+    int64_t ep_queue_cap = 0;             // seeds it can hold
+    int64_t ep_qlen = 0;                  // seeds of the current queue (0: no queue, no generation launch)
+    int ep_blocks = 1;                    // grid of d2d_episode_log_kernel: one block per 32 envs, at most one per SM
+    long long ep_qhead[2] = {0, 0};       // host staging of head[2], head[3]
     // zero-copy observation mirror (d2d_bind_host_mirror): host addresses as bound; *_stale: the host copy must be
     // refreshed by a full device->host copy at the next d2d_step_host (after bind / eager reset)
     uint8_t *mir_lm = nullptr; float *mir_yaw = nullptr; uint8_t *mir_done = nullptr;
@@ -641,6 +650,8 @@ extern "C" int d2d_destroy(d2d_handle *h) {
     if (h->wg_idx) cudaFree(h->wg_idx);
     if (h->wg_ev) cudaEventDestroy(h->wg_ev);
     if (h->wg_fault) cudaFreeHost((void *)h->wg_fault);
+    if (h->ep_mem) cudaFree(h->ep_mem);
+    if (h->ep_queue) cudaFree(h->ep_queue);
     delete h;
     return D2D_OK;
 }
@@ -661,6 +672,22 @@ extern "C" int d2d_get_buffer(d2d_handle *h, const char *name, d2d_buffer_info *
         out->shape[0] = h->B; out->shape[1] = D2D_GRID; out->shape[2] = D2D_GRID; out->shape[3] = 1;
         out->strides[0] = D2D_CELLS; out->strides[1] = D2D_GRID; out->strides[2] = 1; out->strides[3] = 1;
         return D2D_OK;
+    }
+    {   // the episode log's buffers live outside the arena (allocated by d2d_enable_episode_log)
+        const std::string n(name);
+        if (n == "episode_log" || n == "episode_log_head" || n == "world_seed") {
+            if (!h->ep_mem) { h->err = "d2d_get_buffer(" + n + "): the episode log is not enabled"; return D2D_ERR_STATE; }
+            const bool recs = n == "episode_log", hd = n == "episode_log_head";
+            out->dev_ptr = recs ? (void *)h->ep.rec : hd ? (void *)h->ep.head : (void *)h->ep.world_seed;
+            out->dtype = recs ? D2D_U8 : D2D_I64;
+            out->ndim = recs ? 2 : 1;
+            out->shape[0] = recs ? h->ep.capacity : hd ? 4 : h->B;
+            out->shape[1] = recs ? (int64_t)sizeof(d2d_episode_record) : 1; out->shape[2] = 1; out->shape[3] = 1;
+            out->strides[0] = recs ? (int64_t)sizeof(d2d_episode_record) : 1;
+            out->strides[1] = 1; out->strides[2] = 1; out->strides[3] = 1;
+            out->nbytes = recs ? h->ep.capacity * (int64_t)sizeof(d2d_episode_record) : out->shape[0] * 8;
+            return D2D_OK;
+        }
     }
 #if defined(D2D_WARP_PROF) || defined(D2D_PLAN_PROF)
     if (std::string(name) == "warp_prof") {
@@ -914,7 +941,30 @@ static int launch_jerk_warp(d2d_handle *h, const double *actions, cudaStream_t s
     return D2D_OK;
 }
 
+// The episode log behind a step (and, with a seed queue, the generation of the worlds it handed out).  Nothing while the
+// log is disabled.
+static int log_step(d2d_handle *h, cudaStream_t st) {
+    if (!h->ep_mem) return D2D_OK;
+    d2d_episode_log_kernel<<<h->ep_blocks, D2D_EP_THREADS, 0, st>>>(h->P, h->ep);
+    h->launches++;
+    if (h->ep_qlen > 0) {
+        const int blocks = (h->B + D2D_WG_WARPS - 1) / D2D_WG_WARPS;
+        d2d_worldgen_list_kernel<<<blocks < 4 * 148 ? blocks : 4 * 148, D2D_WG_WARPS * 32, 0, st>>>(
+            h->P, h->wg_tab, h->ep.gen_env, h->ep.gen_seed, h->ep.gen_count, h->wg_fault_dev);
+        h->launches++;
+    }
+    CUDA_TRY(h, cudaGetLastError());
+    return D2D_OK;
+}
+
+static int step_impl(d2d_handle *h, const double *actions_dev, void *stream);
+
 extern "C" int d2d_step(d2d_handle *h, const double *actions_dev, void *stream) {
+    const int rc = step_impl(h, actions_dev, stream);
+    return rc != D2D_OK ? rc : log_step(h, (cudaStream_t)stream);
+}
+
+static int step_impl(d2d_handle *h, const double *actions_dev, void *stream) {
     if (!h || !actions_dev) return D2D_ERR_INVALID;
     D2D_NO_PIPE(h);
     if (!h->world_set) { h->err = "d2d_step before d2d_set_world"; return D2D_ERR_STATE; }
@@ -968,14 +1018,15 @@ extern "C" int d2d_step_plan_oxford(d2d_handle *h, const double *actions_dev, do
     if (h->cfg.var_cam != 0.0 && !h->rng_set) { h->err = "var_cam != 0: d2d_set_rng must provide the np.random stream state"; return D2D_ERR_STATE; }
     if (h->cfg.planner != D2D_PLANNER_PRIMITIVE || h->cfg.envs_per_block > 0 || h->P.motion_rvo) {
         // nothing to overlap (or a path made of other kernels): the two calls this entry point stands for
-        const int rc = d2d_step(h, actions_dev, stream);
-        return rc != D2D_OK ? rc : d2d_plan_oxford(h, next_actions_dev, stream);
+        int rc = step_impl(h, actions_dev, stream);
+        if (rc == D2D_OK) rc = d2d_plan_oxford(h, next_actions_dev, stream);
+        return rc != D2D_OK ? rc : log_step(h, (cudaStream_t)stream);
     }
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     const int rc = launch_prim_warp_entry(h, actions_dev, (cudaStream_t)stream, next_actions_dev);
     if (rc != D2D_OK) return rc;
     CUDA_TRY(h, cudaGetLastError());
-    return D2D_OK;
+    return log_step(h, (cudaStream_t)stream);
 }
 
 #define D2D_RESIDENT_WPB 28          // resident gated kernel: one 28-warp block per SM (28 x 148 = 4144 envs in flight)
@@ -1030,9 +1081,11 @@ extern "C" int d2d_rollout(d2d_handle *h, const double *actions_dev, int32_t num
     // Large batches keep the SMs busier with the 4-warp blocks of the per-step kernel, which the hardware back-fills one by
     // one (131072 envs, N = 96: 0.75 ms per step against 0.81 ms), so they run the K steps as K per-step launches -- same
     // results either way (tests/test_gpu_rollout.py).
-    if (variant == 0 && h->B > 2 * 28 * 148) {
+    // ... and so does a handle with an episode log: every step's done bytes must be seen by the log kernel
+    if ((variant == 0 && h->B > 2 * 28 * 148) || h->ep_mem) {
         for (int t = 0; t < num_steps; t++) {
             rc = launch_fused_warp<4, 7, false>(h, actions_dev + (size_t)t * (size_t)action_stride, st);
+            if (rc == D2D_OK) rc = log_step(h, st);
             if (rc != D2D_OK) return rc;
         }
         CUDA_TRY(h, cudaGetLastError());
@@ -1314,8 +1367,10 @@ extern "C" int d2d_step_pipelined(d2d_handle *h, int32_t prelaunch_next) {
     // synchronously (same results, nothing pre-launched).
     // ... and so do batches whose step lasts much longer than the launch + wake-up latency being hidden (~10 us): beyond
     // ~16k envs the gated instantiation's bookkeeping costs more than the overlap returns (measured at 131072 envs: -6 %).
+    // An enabled episode log must see every step's done bytes: synchronous path as well.
     const bool can_pipe = h->cfg.planner == D2D_PLANNER_NOMOVE && h->cfg.envs_per_block <= 0 && !h->P.motion_rvo &&
-                          h->io_actions_dev != h->stage_actions && (long long)h->B * h->cfg.n_rays <= 16384ll * 50;
+                          h->io_actions_dev != h->stage_actions && (long long)h->B * h->cfg.n_rays <= 16384ll * 50 &&
+                          !h->ep_mem;
     if (!can_pipe || (h->mir_stale && !h->pipe_inflight)) {
         D2D_NO_PIPE(h);
         return step_bound_sync(h);
@@ -1484,19 +1539,23 @@ extern "C" int d2d_set_world_source(d2d_handle *h, const d2d_world_source *src) 
     return D2D_OK;
 }
 
+// A world the generation kernels gave up on: reported (and cleared) by the next d2d_generate_worlds / d2d_read_episode_log.
+static bool take_wg_fault(d2d_handle *h, const char *what) {
+    const unsigned long long fault = h->wg_fault ? *h->wg_fault : 0ull;
+    if (!fault) return false;
+    *h->wg_fault = 0ull;
+    h->err = std::string(what) + ": the world of seed " + std::to_string((unsigned)(fault & 0xffffffffull)) + " (env " +
+             std::to_string((int)((fault >> 32) & 0x7fffffffull)) + ") could not be built: more than " +
+             std::to_string(D2D_WORLD_MAX_REJECTS) + " rejected draws in a row; that env's world is undefined";
+    return true;
+}
+
 extern "C" int d2d_generate_worlds(d2d_handle *h, const int32_t *envs_host, const int64_t *seeds_host, int32_t count,
                                    int32_t flags, void *stream) {
     if (!h) return D2D_ERR_INVALID;
     D2D_NO_PIPE(h);
     if (!h->wg_tab) { h->err = "d2d_generate_worlds before d2d_set_world_source"; return D2D_ERR_STATE; }
-    const unsigned long long fault = *h->wg_fault;
-    if (fault) {
-        *h->wg_fault = 0ull;
-        h->err = "d2d_generate_worlds: the world of seed " + std::to_string((unsigned)(fault & 0xffffffffull)) + " (env " +
-                 std::to_string((int)((fault >> 32) & 0x7fffffffull)) + ") could not be built: more than " +
-                 std::to_string(D2D_WORLD_MAX_REJECTS) + " rejected draws in a row; that env's world is undefined";
-        return D2D_ERR_STATE;
-    }
+    if (take_wg_fault(h, "d2d_generate_worlds")) return D2D_ERR_STATE;
     if (flags != D2D_WORLD_EAGER && flags != D2D_WORLD_LAZY) {
         h->err = "d2d_generate_worlds: flags must be D2D_WORLD_EAGER or D2D_WORLD_LAZY"; return D2D_ERR_INVALID;
     }
@@ -1544,6 +1603,97 @@ extern "C" int d2d_generate_worlds(d2d_handle *h, const int32_t *envs_host, cons
     h->world_set = true;
     if (h->cfg.var_cam != 0.0) h->rng_set = true;
     if (h->P.motion_rvo) h->rvo_set = true;
+    return D2D_OK;
+}
+
+// ------------------------------------------------------------------------------------------ episode log + seed queue
+extern "C" int d2d_enable_episode_log(d2d_handle *h, int64_t capacity) {
+    if (!h) return D2D_ERR_INVALID;
+    if (capacity < 0 || capacity > ((int64_t)1 << 40) / (int64_t)sizeof(d2d_episode_record)) {
+        h->err = "d2d_enable_episode_log: capacity out of range"; return D2D_ERR_INVALID;
+    }
+    D2D_NO_PIPE(h);
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    CUDA_TRY(h, cudaDeviceSynchronize());            // no kernel may still use the old buffers
+    if (h->ep_mem) CUDA_TRY(h, cudaFree(h->ep_mem));
+    h->ep_mem = nullptr; h->ep = EpLog{}; h->ep_qlen = 0;
+    if (capacity == 0) return D2D_OK;
+    const size_t B = (size_t)h->B;
+    const size_t o_head = (size_t)capacity * sizeof(d2d_episode_record);
+    const size_t o_seed = o_head + 64, o_list = o_seed + (B * 8 + 15) / 16 * 16, o_genv = o_list + (B * 4 + 15) / 16 * 16;
+    const size_t o_gsd = o_genv + (B * 4 + 15) / 16 * 16, bytes = o_gsd + (B * 4 + 15) / 16 * 16;
+    unsigned char *m = nullptr;
+    if (cudaMalloc((void **)&m, bytes) != cudaSuccess) {
+        cudaGetLastError();
+        h->err = "d2d_enable_episode_log: cudaMalloc of " + std::to_string(bytes) + " B failed"; return D2D_ERR_NOMEM;
+    }
+    if (cudaMemset(m, 0, bytes) != cudaSuccess) { cudaFree(m); h->err = "d2d_enable_episode_log: cudaMemset failed"; return D2D_ERR_CUDA; }
+    h->ep_mem = m;
+    h->ep.rec = (d2d_episode_record *)m; h->ep.capacity = capacity;
+    h->ep.head = (long long *)(m + o_head); h->ep.gen_count = (int *)(m + o_head + 32);
+    h->ep.ticket = (unsigned int *)(m + o_head + 36);
+    int sms = 0;
+    if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->cfg.device) != cudaSuccess || sms <= 0) sms = 148;
+    h->ep_blocks = (h->B + 31) / 32 < sms ? (h->B + 31) / 32 : sms;
+    h->ep.world_seed = (long long *)(m + o_seed); h->ep.list = (int *)(m + o_list);
+    h->ep.gen_env = (int *)(m + o_genv); h->ep.gen_seed = (uint32_t *)(m + o_gsd);
+    h->ep.queue = h->ep_queue;
+    return D2D_OK;
+}
+
+extern "C" int d2d_read_episode_log(d2d_handle *h, d2d_episode_record *out_host, int64_t *count, int64_t *dropped, void *stream) {
+    if (!h) return D2D_ERR_INVALID;
+    if (!count || !dropped || !out_host) { h->err = "d2d_read_episode_log: null argument"; return D2D_ERR_INVALID; }
+    D2D_NO_PIPE(h);
+    if (!h->ep_mem) { h->err = "d2d_read_episode_log: the episode log is not enabled"; return D2D_ERR_STATE; }
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    cudaStream_t st = (cudaStream_t)stream;
+    CUDA_TRY(h, cudaStreamSynchronize(st));
+    if (take_wg_fault(h, "d2d_read_episode_log")) return D2D_ERR_STATE;
+    long long written = 0;
+    CUDA_TRY(h, cudaMemcpyAsync(&written, h->ep.head, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(h, cudaStreamSynchronize(st));
+    const long long n = written < h->ep.capacity ? written : h->ep.capacity;
+    if (n > 0)
+        CUDA_TRY(h, cudaMemcpyAsync(out_host, h->ep.rec, (size_t)n * sizeof(d2d_episode_record), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(h, cudaMemsetAsync(h->ep.head, 0, 8, st));
+    CUDA_TRY(h, cudaStreamSynchronize(st));
+    *count = n;
+    *dropped = written - n;
+    return D2D_OK;
+}
+
+extern "C" int d2d_set_seed_queue(d2d_handle *h, const int64_t *seeds_host, int64_t count, void *stream) {
+    if (!h) return D2D_ERR_INVALID;
+    D2D_NO_PIPE(h);
+    if (!h->wg_tab) { h->err = "d2d_set_seed_queue before d2d_set_world_source"; return D2D_ERR_STATE; }
+    if (!h->cfg.auto_reset) { h->err = "d2d_set_seed_queue: the handle was created with auto_reset = 0"; return D2D_ERR_STATE; }
+    if (!h->ep_mem) { h->err = "d2d_set_seed_queue: the episode log is not enabled"; return D2D_ERR_STATE; }
+    if (count < 0 || (count > 0 && !seeds_host)) { h->err = "d2d_set_seed_queue: bad count or null array"; return D2D_ERR_INVALID; }
+    for (int64_t i = 0; i < count; i++)
+        if (seeds_host[i] < 0 || seeds_host[i] > 0xffffffffll) {
+            h->err = "d2d_set_seed_queue: seed " + std::to_string((long long)seeds_host[i]) + " outside [0, 2**32)";
+            return D2D_ERR_INVALID;
+        }
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (count > h->ep_queue_cap) {                   // grows only: a captured graph keeps a valid queue address
+        CUDA_TRY(h, cudaDeviceSynchronize());        // no log kernel may still read the old queue
+        long long *q = nullptr;
+        if (cudaMalloc((void **)&q, (size_t)count * 8) != cudaSuccess) {
+            cudaGetLastError();
+            h->err = "d2d_set_seed_queue: cudaMalloc failed"; return D2D_ERR_NOMEM;
+        }
+        if (h->ep_queue) cudaFree(h->ep_queue);
+        h->ep_queue = q; h->ep_queue_cap = count; h->ep.queue = q;
+    } else {
+        CUDA_TRY(h, cudaStreamSynchronize(st));      // the last log kernel on this stream has read the old seeds
+    }
+    if (count > 0) CUDA_TRY(h, cudaMemcpyAsync(h->ep_queue, seeds_host, (size_t)count * 8, cudaMemcpyHostToDevice, st));
+    h->ep_qhead[0] = 0; h->ep_qhead[1] = count;
+    CUDA_TRY(h, cudaMemcpyAsync(h->ep.head + 2, h->ep_qhead, 16, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(h, cudaStreamSynchronize(st));
+    h->ep_qlen = count;
     return D2D_OK;
 }
 

@@ -173,6 +173,7 @@ class Drone2DVecEnv(object):
         # a copy: reseed / clone_envs / load_state rewrite entries, and must not write into the caller's array
         self.seeds = np.array(seeds if seeds is not None else params.map_id + np.arange(self.num_envs), dtype=np.int64)
         self._world_source = None
+        self._log_capacity, self._queue_set = 0, False
         if world_gen == "device":
             self.reseed(np.arange(self.num_envs), self.seeds)
             torch.cuda.current_stream(self.device).synchronize()
@@ -244,6 +245,7 @@ class Drone2DVecEnv(object):
         self._check(self._lib.d2d_generate_worlds(self._h, idx.ctypes.data_as(C.c_void_p), sd.ctypes.data_as(C.c_void_p),
                                                   int(idx.size), flags, self._stream()), "d2d_generate_worlds")
         self.seeds[idx] = sd
+        self._set_world_seeds(idx, sd)
 
     def check_worlds(self):
         """Raises if an earlier `reseed` met a seed whose world cannot be built (call after synchronising the stream)."""
@@ -448,6 +450,9 @@ class Drone2DVecEnv(object):
         self._check(self._lib.d2d_clone_envs(self._h, s.ctypes.data_as(C.c_void_p), d.ctypes.data_as(C.c_void_p), int(s.size),
                                              self._stream()), "d2d_clone_envs")
         self.seeds[d] = self.seeds[s]
+        if self._log_capacity and s.size:
+            ws = self.buffer("world_seed")
+            ws[torch.as_tensor(d.astype(np.int64), device=self.device)] = ws[torch.as_tensor(s.astype(np.int64), device=self.device)]
 
     def save_state(self, envs=None):
         """Packs the state of `envs` (default: all) into a uint8 CUDA tensor [count, bytes_per_env] (d2d_save_state).
@@ -482,7 +487,61 @@ class Drone2DVecEnv(object):
                                              C.c_void_p(state.data_ptr()), C.c_uint64(int(saved["fingerprint"])),
                                              self._stream()), "d2d_load_state")
         if saved.get("seeds") is not None:
-            self.seeds[np.arange(count) if idx is None else idx] = np.asarray(saved["seeds"], dtype=np.int64)
+            envs = np.arange(count) if idx is None else idx
+            self.seeds[envs] = np.asarray(saved["seeds"], dtype=np.int64)
+            self._set_world_seeds(envs, self.seeds[envs])
+
+    # ------------------------------------------------------------------ episode log + seed queue
+    def _set_world_seeds(self, envs, seeds):
+        """While the episode log is enabled, "world_seed" follows the seeds of reseed / clone_envs / load_state (a device
+        write on the current stream, ordered with the library call it mirrors)."""
+        if self._log_capacity and len(envs):
+            self.buffer("world_seed")[torch.as_tensor(np.asarray(envs, dtype=np.int64), device=self.device)] = \
+                torch.as_tensor(np.asarray(seeds, dtype=np.int64), device=self.device)
+
+    def enable_episode_log(self, capacity):
+        """Enables the episode log (d2d_enable_episode_log) with room for `capacity` records between two `read_episodes`
+        calls: from now on every step appends, on the device, one record per env that reported done (the fields of the
+        reference's experiment row).  `B * steps between reads` never drops a record.  "world_seed" is filled from
+        `self.seeds`.  capacity=0 disables the log (and clears a seed queue)."""
+        capacity = int(capacity)
+        self._check(self._lib.d2d_enable_episode_log(self._h, capacity), "d2d_enable_episode_log")
+        for name in ("episode_log", "episode_log_head", "world_seed"):
+            self._views.pop(name, None)
+        self._log_capacity, self._queue_set = capacity, False
+        self._log_out = np.zeros(capacity, dtype=_native.EPISODE_DTYPE)
+        if capacity:
+            self.buffer("world_seed").copy_(torch.as_tensor(self.seeds, dtype=torch.int64))
+
+    def read_episodes(self):
+        """(records, dropped): the records written since the last read as a numpy structured array of dtype
+        `_native.EPISODE_DTYPE` in (step, env) order, and how many the full log could not take (d2d_read_episode_log;
+        synchronises the current stream).  While a seed queue is set, `self.seeds` is refreshed from "world_seed"."""
+        if not self._log_capacity:
+            raise _native.Drone2DNativeError("read_episodes: the episode log is not enabled (enable_episode_log)")
+        n, dropped = C.c_int64(), C.c_int64()
+        self._check(self._lib.d2d_read_episode_log(self._h, self._log_out.ctypes.data_as(C.c_void_p), C.byref(n),
+                                                   C.byref(dropped), self._stream()), "d2d_read_episode_log")
+        if self._queue_set:
+            self.seeds[:] = self.buffer("world_seed").cpu().numpy()
+        return self._log_out[:n.value].copy(), int(dropped.value)
+
+    def set_seed_queue(self, seeds):
+        """Seeds for the envs that finish from now on (d2d_set_seed_queue): in every step each env that reports done takes
+        the next one (ascending env order) and starts that world, generated on the device, at its next step; its record
+        carries the seed of the world it finished.  When the queue runs out, envs replay their last world.  Needs the episode
+        log and auto-reset; the world source is set up here.  An empty sequence clears the queue."""
+        sd = np.asarray(seeds).reshape(-1)
+        if sd.size and sd.dtype.kind not in "iu":
+            raise ValueError("seeds must be integers, got %s" % sd.dtype)
+        sd = np.ascontiguousarray(sd, dtype=np.int64)
+        if self._world_source is None and self._log_capacity and self.cfg.auto_reset:
+            src = world_source(self.params, self._smap)
+            self._check(self._lib.d2d_set_world_source(self._h, C.byref(src)), "d2d_set_world_source")
+            self._world_source = src
+        self._check(self._lib.d2d_set_seed_queue(self._h, sd.ctypes.data_as(C.c_void_p), int(sd.size), self._stream()),
+                    "d2d_set_seed_queue")
+        self._queue_set = sd.size > 0
 
     def plan_oxford(self, out=None):
         """Oxford.plan for every env (yaw_planner.py:81-127): returns float64 CUDA tensor [B] of actions."""

@@ -376,6 +376,55 @@ int d2d_set_world_source(d2d_handle *h, const d2d_world_source *src);
 int d2d_generate_worlds(d2d_handle *h, const int32_t *envs_host, const int64_t *seeds_host, int32_t count, int32_t flags,
                         void *stream);
 
+/* Episode log: one fixed-size record per (step, env) that reported done -- everything the reference's experiment row
+ * (experiment.py:69-101) needs, written on the device by the step that finished the episode, so a driver can step many
+ * times between host synchronisations.  The events are exactly those D2D_STAT_EPISODES counts. */
+typedef struct d2d_episode_record {   /* 48 bytes */
+    int64_t seed;                /* "world_seed"[env] at the step that reported done */
+    int64_t step;                /* index of that step among the steps logged since the log was enabled */
+    int64_t tracked_steps;       /* "tracker_buffer_ts" */
+    int32_t env;
+    int32_t steps;               /* "steps" (flight time = steps * dt) */
+    int32_t grid_discovered;     /* belief cells != 0 */
+    int32_t trackers;            /* "tracker_buffer_count" */
+    uint8_t state_machine, collision_flag, freezing_flag, dead_lock_flag;
+    int32_t reserved;
+} d2d_episode_record;
+
+/* Enables the episode log with room for `capacity` records (0 disables it and frees its buffers; enabling again
+ * reallocates them, so a CUDA graph captured before must be captured again).  Synchronises the device.  The library-owned
+ * DEVICE buffers (d2d_get_buffer; D2D_ERR_STATE while the log is disabled):
+ *   "episode_log"       [capacity][48] u8 records
+ *   "episode_log_head"  int64[4]: records written since the last read, steps logged, seeds handed out by the queue, queue length
+ *   "world_seed"        int64 [num_envs], zero when enabled: the seed of each env's world.  The caller writes it with ordinary
+ *                       device writes; the library writes it only from the seed queue.  Not env state: clone / save / load
+ *                       and the state layout ignore it.
+ * While the log is enabled every step entry point (d2d_step, d2d_step_plan_oxford after its side stream has joined,
+ * d2d_step_host, d2d_step_bound, d2d_step_bound_plan_oxford) enqueues one more kernel behind the step: it appends a record
+ * for every env whose "done" is non-zero, in ascending env order, so the log is in (step, env) order.  The step counter
+ * lives on the device, so replays of a captured graph count correctly.  d2d_rollout runs its K steps as K per-step launches
+ * (each followed by the log kernel) and d2d_step_pipelined takes its synchronous path.  Resets, clone and load write no
+ * records.  A record that finds the log full is not written but counted (the `dropped` of the next read); a capacity of
+ * num_envs x (steps between reads) never drops.  With the log disabled (the default) nothing is launched. */
+int d2d_enable_episode_log(d2d_handle *h, int64_t capacity);
+
+/* Synchronises `stream`, copies the records written since the last read to out_host (HOST, room for `capacity` records),
+ * their number to *count and the number of records the full log could not take to *dropped, then resets the written
+ * count (in stream order).  D2D_ERR_STATE when the log is disabled, or when a world of the seed queue could not be built
+ * (env and seed in d2d_last_error; the failure is cleared, the records stay for the next read). */
+int d2d_read_episode_log(d2d_handle *h, d2d_episode_record *out_host, int64_t *count, int64_t *dropped, void *stream);
+
+/* Seed queue: from the next logged step on, every env that reports done takes the next seed of the queue (ascending env
+ * order within a step, while seeds remain).  Its record carries the OLD "world_seed"; "world_seed"[env] becomes the new seed
+ * and a second kernel behind the log kernel generates that world with D2D_WORLD_LAZY semantics, so the env starts it at its
+ * next step (d2d_generate_worlds).  When the queue runs out, finished envs auto-reset into their last world as before.  A
+ * world that cannot be built is reported by the next d2d_read_episode_log or d2d_generate_worlds.  No host copy per step:
+ * gaze policy, step, log and generation can be captured in a CUDA graph together.
+ * seeds_host: HOST int64 [count], each in [0, 2^32); uploaded, the queue cursor is reset in stream order; count = 0 clears
+ * the queue.  D2D_ERR_STATE without d2d_set_world_source, without cfg.auto_reset or without an enabled log.  A rejected
+ * call changes nothing. */
+int d2d_set_seed_queue(d2d_handle *h, const int64_t *seeds_host, int64_t count, void *stream);
+
 /* Number of kernel launches issued by this handle so far (bench.py's gpu_launches). */
 int64_t d2d_launch_count(const d2d_handle *h);
 
