@@ -17,6 +17,7 @@
 #include "d2d_clone.cuh"
 #include "d2d_worldgen.cuh"
 #include "d2d_episode.cuh"
+#include "d2d_render.cuh"
 
 // ------------------------------------------------------------------------------------------ handle
 // Per-env state tag of an arena buffer: env e's row of `row_bytes` bytes starts at offset + e * row_stride, in each of
@@ -1694,6 +1695,56 @@ extern "C" int d2d_set_seed_queue(d2d_handle *h, const int64_t *seeds_host, int6
     CUDA_TRY(h, cudaMemcpyAsync(h->ep.head + 2, h->ep_qhead, 16, cudaMemcpyHostToDevice, st));
     CUDA_TRY(h, cudaStreamSynchronize(st));
     h->ep_qlen = count;
+    return D2D_OK;
+}
+
+// ------------------------------------------------------------------------------------------ rendering
+extern "C" int d2d_render(d2d_handle *h, const int32_t *envs_host, int32_t first_env, int32_t count, int32_t pixels_per_cell,
+                          int32_t layers, uint8_t *frames_dev, void *stream) {
+    if (!h) return D2D_ERR_INVALID;
+    D2D_NO_PIPE(h);
+    if (!h->world_set) { h->err = "d2d_render before d2d_set_world"; return D2D_ERR_STATE; }
+    if (count < 0) { h->err = "d2d_render: negative count"; return D2D_ERR_INVALID; }
+    if (pixels_per_cell < 1 || pixels_per_cell > D2D_RENDER_MAX_PPC) {
+        h->err = "d2d_render: pixels_per_cell " + std::to_string(pixels_per_cell) + " outside 1.." + std::to_string(D2D_RENDER_MAX_PPC);
+        return D2D_ERR_INVALID;
+    }
+    if (layers & ~D2D_RENDER_ALL) { h->err = "d2d_render: unknown layer bits " + std::to_string(layers & ~D2D_RENDER_ALL); return D2D_ERR_INVALID; }
+    RenderList list;
+    if (envs_host) {
+        if (count > D2D_RENDER_MAX_LIST) {
+            h->err = "d2d_render: a list of " + std::to_string(count) + " envs (at most " + std::to_string(D2D_RENDER_MAX_LIST) +
+                     "; render a larger selection as a contiguous range)";
+            return D2D_ERR_INVALID;
+        }
+        int rc = check_env_indices(h, "d2d_render", envs_host, nullptr, count);
+        if (rc != D2D_OK) return rc;
+        memcpy(list.e, envs_host, (size_t)count * 4);
+    } else if (first_env < 0 || first_env > h->B || count > h->B - first_env) {
+        h->err = "d2d_render: envs [" + std::to_string(first_env) + ", " + std::to_string((long long)first_env + count) +
+                 ") outside [0, " + std::to_string(h->B) + ")";
+        return D2D_ERR_INVALID;
+    }
+    if (count == 0) return D2D_OK;
+    if (!frames_dev) { h->err = "d2d_render: null frame buffer"; return D2D_ERR_INVALID; }
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    cudaPointerAttributes at;
+    if (cudaPointerGetAttributes(&at, frames_dev) != cudaSuccess || at.type != cudaMemoryTypeDevice || at.device != h->cfg.device) {
+        cudaGetLastError();
+        h->err = "d2d_render: the frame buffer is not device memory of device " + std::to_string(h->cfg.device);
+        return D2D_ERR_INVALID;
+    }
+    RenderArgs a;
+    a.frames = frames_dev; a.first_env = first_env; a.count = count; a.use_list = envs_host ? 1 : 0;
+    a.ppc = pixels_per_cell; a.layers = layers; a.W = D2D_GRID * pixels_per_cell;
+    a.band_rows = D2D_RENDER_BAND_PIX / a.W < D2D_GRID * pixels_per_cell ? D2D_RENDER_BAND_PIX / a.W : D2D_GRID * pixels_per_cell;
+    a.nbands = (D2D_GRID * pixels_per_cell + a.band_rows - 1) / a.band_rows;
+    a.s = h->cfg.map_scale / (double)pixels_per_cell;
+    a.span = h->P.ray_da * (double)(h->cfg.n_rays - 1);
+    const long long blocks = (long long)count * a.nbands;
+    d2d_render_kernel<<<(unsigned)blocks, D2D_RENDER_THREADS, 0, (cudaStream_t)stream>>>(h->P, a, list);
+    h->launches++;
+    CUDA_TRY(h, cudaGetLastError());
     return D2D_OK;
 }
 

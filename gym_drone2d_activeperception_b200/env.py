@@ -280,7 +280,12 @@ class Drone2DEnv2(object):
         self._vec.load_state(s, [0])
 
     def render(self, mode="human"):
-        raise NotImplementedError("rendering (pygame) is out of scope of the B200 path; see DESIGN.md §7")
+        """mode="rgb_array": the env's frame as numpy uint8 [500, 500, 3] (10 pixels per cell, every layer), drawn on the
+        device (Drone2DVecEnv.render).  There is no pygame window."""
+        if mode == "rgb_array":
+            return self._vec.render([0], pixels_per_cell=10)[0].cpu().numpy()
+        raise NotImplementedError("render(mode=%r): there is no pygame window on the B200 path; use mode=\"rgb_array\" "
+                                  "(see DESIGN.md §7)" % (mode,))
 
     def close(self):
         self._vec.close()

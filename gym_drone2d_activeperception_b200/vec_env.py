@@ -137,7 +137,7 @@ class Drone2DVecEnv(object):
                 section 2).  `reseed` needs neither.  Cannot be combined with `worlds`.
     """
 
-    metadata = {"render.modes": []}
+    metadata = {"render.modes": ["rgb_array"]}
 
     def __init__(self, params, num_envs, seeds=None, device="cuda:0", auto_reset=True, trackers=True, oxford=None,
                  envs_per_block=0, strip_width=10, worlds=None, owl=None, jerk_tie_orders=None, world_gen="host"):
@@ -574,6 +574,62 @@ class Drone2DVecEnv(object):
         if out is None:
             out = torch.empty(self.num_envs, dtype=torch.float64, device=self.device)
         self._check(self._lib.d2d_plan_gaze(self._h, code, C.c_void_p(out.data_ptr()), self._stream()), "d2d_plan_gaze")
+        return out
+
+    # ------------------------------------------------------------------ rendering
+    @staticmethod
+    def render_layers(layers):
+        """"all", an int mask of _native.RENDER_* bits, or an iterable of names ("ground_truth", "belief", "view", "plan",
+        "trackers", "agents", "drone") -> int mask."""
+        if isinstance(layers, str):
+            if layers.lower() == "all":
+                return _native.RENDER_ALL
+            layers = [layers]
+        if isinstance(layers, (int, np.integer)):
+            return int(layers)
+        mask = 0
+        for name in layers:
+            key = str(name).lower()
+            if key not in _native.RENDER_LAYERS:
+                raise ValueError("unknown render layer %r (one of %s)" % (name, ", ".join(_native.RENDER_LAYERS)))
+            mask |= _native.RENDER_LAYERS[key]
+        return mask
+
+    def render(self, envs=None, pixels_per_cell=2, layers="all", out=None):
+        """RGB frames of `envs` drawn on the device (d2d_render, one kernel): uint8 CUDA tensor [count, H, W, 3] with
+        H = W = 50 * pixels_per_cell, in the reference's screen layout (column = x, row = y, origin top-left).
+        envs: None (all), a step-1 range or an ascending contiguous list (rendered as a range), or any other sequence of
+        at most 1024 env indices (repeats allowed).  layers: "all", an int mask or an iterable of layer names
+        (`render_layers`).  out: a preallocated contiguous uint8 tensor of that shape on this device -- what a captured
+        CUDA graph renders into.  The frames show the arena as it is: an env that just reported done shows its terminal
+        state until its next step."""
+        ppc = int(pixels_per_cell)
+        mask = self.render_layers(layers)
+        first, lst = 0, None
+        if envs is None:
+            count = self.num_envs
+        elif isinstance(envs, range) and envs.step == 1:
+            first, count = envs.start, max(0, envs.stop - envs.start)
+        else:
+            idx = self._env_indices(envs)
+            count = int(idx.size)
+            if count and np.array_equal(idx, np.arange(idx[0], idx[0] + count)):
+                first = int(idx[0])
+            else:
+                if count > _native.RENDER_MAX_LIST:
+                    raise ValueError("render: a list of %d envs (at most %d; a larger selection must be a contiguous range)"
+                                     % (count, _native.RENDER_MAX_LIST))
+                lst = idx
+        H = 50 * ppc
+        shape = (count, H, H, 3)
+        if out is None:
+            out = torch.empty(shape, dtype=torch.uint8, device=self.device)
+        elif (not torch.is_tensor(out) or out.dtype != torch.uint8 or tuple(out.shape) != shape or not out.is_contiguous()
+              or out.device.type != "cuda" or out.device.index != self._dev_index):
+            raise ValueError("render: `out` must be a contiguous uint8 tensor %s on cuda:%d" % (shape, self._dev_index))
+        self._check(self._lib.d2d_render(self._h, None if lst is None else lst.ctypes.data_as(C.c_void_p), int(first),
+                                         int(count), ppc, int(mask), C.c_void_p(out.data_ptr() if count else 0),
+                                         self._stream()), "d2d_render")
         return out
 
     def stats(self, reset=False):

@@ -425,6 +425,27 @@ int d2d_read_episode_log(d2d_handle *h, d2d_episode_record *out_host, int64_t *c
  * call changes nothing. */
 int d2d_set_seed_queue(d2d_handle *h, const int64_t *seeds_host, int64_t count, void *stream);
 
+/* Rendering: replaces Drone2DEnv2.render (drone_v2.py:263-303, utils.py:31-64, 550-558, 786-817) with rgb_array frames drawn
+ * on the device instead of a pygame window.  Frame of one env: uint8 [H][W][3] RGB, C-contiguous, H = W = 50 * ppc
+ * (pixels_per_cell in 1..D2D_RENDER_MAX_PPC; ppc 10 is the reference's 500 x 500 screen), in the screen layout: column =
+ * world x, row = world y, origin top-left; cell (i, j) covers rows j*ppc.. and columns i*ppc...  `layers` (D2D_RENDER_*
+ * bits) are drawn back to front: ground truth / belief cells, the field of view the step's rays sweep, the planner target and
+ * the remaining Primitive waypoints, active tracker rings, agents (red if seen this step, else blue), the drone.  Exact
+ * pixel rules and palette: DESIGN.md section 2, "Rendering".
+ * Envs: envs_host == NULL renders [first_env, first_env + count); otherwise envs_host[0..count) (HOST int32, repeats
+ * allowed, at most D2D_RENDER_MAX_LIST entries), passed by value in the kernel's parameters: either form is ONE kernel
+ * launch with no upload, so it can be captured in a CUDA graph beside the step.  frames_dev: DEVICE [count][H][W][3] of
+ * the handle's device, any byte alignment.  Every argument is checked before anything is enqueued (a rejected call writes
+ * nothing); count = 0 enqueues nothing.  D2D_ERR_STATE before d2d_set_world and while a pipelined step is in flight.
+ * The call reads the arena and writes only the frames.  It shows the arena as it is: an env that just reported done shows
+ * its terminal state until its next step, an env with a lazy reset or reseed pending shows its old world until then. */
+#define D2D_RENDER_MAX_PPC 10
+#define D2D_RENDER_MAX_LIST 1024      /* longest env list; larger selections are a contiguous range */
+enum { D2D_RENDER_GROUND_TRUTH = 1, D2D_RENDER_BELIEF = 2, D2D_RENDER_VIEW = 4, D2D_RENDER_PLAN = 8,
+       D2D_RENDER_TRACKERS = 16, D2D_RENDER_AGENTS = 32, D2D_RENDER_DRONE = 64, D2D_RENDER_ALL = 127 };
+int d2d_render(d2d_handle *h, const int32_t *envs_host, int32_t first_env, int32_t count, int32_t pixels_per_cell,
+               int32_t layers, uint8_t *frames_dev, void *stream);
+
 /* Number of kernel launches issued by this handle so far (bench.py's gpu_launches). */
 int64_t d2d_launch_count(const d2d_handle *h);
 
