@@ -62,6 +62,16 @@ RENDER_LAYERS = {"ground_truth": RENDER_GROUND_TRUTH, "belief": RENDER_BELIEF, "
                  "trackers": RENDER_TRACKERS, "agents": RENDER_AGENTS, "drone": RENDER_DRONE}
 
 
+# d2d_difficulty: position grid and step limits, and the slot-table entry of a step that collision_state does not record
+DIFF_MAX_POS, DIFF_MAX_STEPS, DIFF_NO_SLOT = 1024, 1024, 0xFFFF
+
+
+class D2DDifficultySpec(C.Structure):
+    _fields_ = [("struct_size", C.c_int32), ("nx", C.c_int32), ("ny", C.c_int32),
+                ("x0", C.c_double), ("y0", C.c_double), ("step", C.c_double),
+                ("steps", C.c_int32), ("n_slots", C.c_int32), ("slot", C.c_uint16 * DIFF_MAX_STEPS)]
+
+
 class D2DWorldSource(C.Structure):
     _fields_ = [
         ("struct_size", C.c_int32), ("agent_number", C.c_int32), ("pillar_number", C.c_int32), ("pad_", C.c_int32),
@@ -96,7 +106,7 @@ EXPORTS = ["d2d_version", "d2d_last_error", "d2d_create", "d2d_destroy", "d2d_se
            "d2d_step_host", "d2d_bind_host_mirror", "d2d_bind_host_io", "d2d_step_bound", "d2d_step_pipelined", "d2d_plan_oxford", "d2d_step_plan_oxford", "d2d_step_bound_plan_oxford", "d2d_plan_gaze", "d2d_set_drone_pose", "d2d_get_buffer", "d2d_stats",
            "d2d_launch_count", "d2d_clone_envs", "d2d_state_layout", "d2d_save_state", "d2d_load_state",
            "d2d_set_world_source", "d2d_generate_worlds", "d2d_enable_episode_log", "d2d_read_episode_log",
-           "d2d_set_seed_queue", "d2d_render"]
+           "d2d_set_seed_queue", "d2d_render", "d2d_difficulty"]
 
 _lib = None
 
@@ -153,6 +163,7 @@ def load():
     L.d2d_read_episode_log.argtypes = [vp, vp, C.POINTER(C.c_int64), C.POINTER(C.c_int64), vp]
     L.d2d_set_seed_queue.argtypes = [vp, vp, C.c_int64, vp]
     L.d2d_render.argtypes = [vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, vp, vp]
+    L.d2d_difficulty.argtypes = [vp, C.POINTER(D2DDifficultySpec), C.c_int32, C.c_int32, vp, vp, vp, vp]
     for name in EXPORTS:
         if name not in ("d2d_version", "d2d_last_error", "d2d_launch_count"):
             getattr(L, name).restype = C.c_int

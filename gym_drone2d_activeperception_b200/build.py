@@ -10,7 +10,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libdrone2d.so")
 SOURCES = ["drone2d.cu"]
-DEPS = ["drone2d.cu", "d2d_state.cuh", "d2d_math.cuh", "d2d_step.cuh", "d2d_plan.cuh", "d2d_plan_host.inl", "d2d_plan_math.cuh", "d2d_rvo.cuh", "d2d_rvo_math.cuh", "d2d_clone.cuh", "d2d_worldgen.cuh", "d2d_worldgen_body.inc", "d2d_episode.cuh", "d2d_render.cuh",
+DEPS = ["drone2d.cu", "d2d_state.cuh", "d2d_math.cuh", "d2d_step.cuh", "d2d_plan.cuh", "d2d_plan_host.inl", "d2d_plan_math.cuh", "d2d_rvo.cuh", "d2d_rvo_math.cuh", "d2d_clone.cuh", "d2d_worldgen.cuh", "d2d_worldgen_body.inc", "d2d_episode.cuh", "d2d_render.cuh", "d2d_difficulty.cuh", "d2d_agent_math.cuh",
         "d2d_tan_table.inc", "d2d_sincos_table.inc", os.path.join("..", "..", "include", "drone2d.h")]
 
 NVCC_FLAGS = [

@@ -5,9 +5,12 @@ start position of an 8x8 grid (x, y in range(map_scale + drone_radius, size - ma
 pinned at the position (`env.drone.x = x` before every step), the env is stepped with the NoMove planner and action 0 for
 T / dt steps, and `collision_state[ix, iy, int(t / 0.1)] = 1` whenever `info['collision_flag'] == 2`.  The reference runs the
 64 x 240 steps of one world sequentially on one env object; here all (world, position) pairs are one batch."""
+import copy
+
 import numpy as np
 import torch
 
+from . import _native
 from .params import Params
 from .vec_env import Drone2DVecEnv
 from .world import generate_worlds
@@ -98,10 +101,109 @@ def survivability(params, seeds, T=12, position_step=60, device="cuda:0"):
 def obstacle_density(params, seeds):
     """script/difficulty_calculator/density_calculator.py:13-30: sum of 3.14 * r^2 over the agents / map area (host only)."""
     w = generate_worlds(params, np.asarray(seeds, dtype=np.int64))
+    return _density(params, w["agent_radius"])
+
+
+def _density(params, agent_radius):
     out = []
-    for radii in w["agent_radius"]:
+    for radii in agent_radius:
         area = 0
         for r in radii.tolist():        # the script's own accumulation order and scalar `**` (libm pow)
             area += 3.14 * r ** 2
         out.append(area / (params.map_size[0] * params.map_size[1]))
     return np.array(out)
+
+
+def global_slots(T, dt, steps):
+    """The slot table of `global_survivability` for a difficulty call of `steps` agent steps: (n_slots, table) with
+    n_slots = int(T / dt) and table[k-1] the slot agent step k writes -- the script's int(t / 0.1), doubled slots included
+    -- or DIFF_NO_SLOT for the steps beyond the script's loop."""
+    n_slots = int(T / dt)
+    table = [int(t / 0.1) for t in np.arange(0, T, 0.1)][:n_slots]
+    return n_slots, table[:steps] + [_native.DIFF_NO_SLOT] * (steps - len(table))
+
+
+def survival_from_hits(first_hit, static_hit, T_survivability, n_slots, table):
+    """survivability, its per-seed mean and the global survival time from d2d_difficulty's outputs (first_hit int [S, ...],
+    static_hit bool [S, ...]) and the slot table of `global_slots`, with the scripts' own host arithmetic."""
+    fh = np.asarray(first_hit, dtype=np.int64)
+    S = fh.shape[0]
+    # survivability_calculator.py: loop index i (time ts[i]) sees the state after agent step i + 1
+    ts = np.arange(0, T_survivability, 0.1)
+    L = len(ts)
+    tv = np.concatenate([ts, [float(T_survivability)]])
+    st = tv[np.where((fh >= 1) & (fh <= L), fh - 1, L)] - 0.1
+    st[st < 0] = 0
+    # mean_survival_time: the first slot written -- slots never decrease, so the slot of the first dynamic hit -- unless
+    # the position is static, where collision_flag is never 2
+    tab = np.array(list(table) + [_native.DIFF_NO_SLOT], dtype=np.int64)
+    slot = tab[np.where(fh >= 1, fh - 1, len(table))]
+    first = np.where(np.asarray(static_hit, dtype=bool) | (slot == _native.DIFF_NO_SLOT), n_slots, slot)
+    return {"survivability": st, "mean_survivability": st.reshape(S, -1).mean(1), "global_survival_time": first * 0.1}
+
+
+def difficulty(params, seeds, T_global=24, T_survivability=12, position_step=60, num_envs=65536, world_gen="device",
+               collision_state=False, device="cuda:0"):
+    """`survivability`, `global_survivability` (as `mean_survival_time`) and `obstacle_density` of every seed from ONE
+    kernel per chunk of seeds (d2d_difficulty): the agents are stepped alone from each world's reset state and every grid
+    position is tested after every step, the way both scripts test it.  Under CVM no agent looks at the drone, so one agent
+    trajectory per world answers all positions.  The seeds stream through one scratch handle of min(num_envs, len(seeds))
+    NoMove envs; each chunk is an eager `reseed` (world_gen="device") or `set_worlds` (world_gen="host") and one
+    `difficulty` call into preallocated device outputs, with one synchronisation at the end.  Any planner (the scratch
+    handle is NoMove, as in the scripts); CVM only (RVO: use the functions above).
+    Returns a dict of numpy arrays, S = len(seeds):
+      survivability        float64 [S, nx, ny]  == survivability(params, seeds, T_survivability, position_step)[0]
+      mean_survivability   float64 [S]          == its second output
+      global_survival_time float64 [S, nx, ny]  == mean_survival_time(global_survivability(params, seeds, T_global, ...))
+      density              float64 [S]          == obstacle_density(params, seeds)
+      collision_state      uint8 [S, nx, ny, int(T_global / dt)] == global_survivability(...), with collision_state=True.
+    Device worlds equal host worlds except for the documented group-velocity rounding of static-map agents (DESIGN.md
+    section 2)."""
+    params = copy.copy(params)
+    params.planner = "NoMove"           # as both scripts; the worlds and the agents do not depend on the planner
+    if world_gen not in ("host", "device"):
+        raise ValueError("world_gen must be 'host' or 'device', got %r" % (world_gen,))
+    xs, ys = survivability_positions(params, position_step)
+    nx, ny = len(xs), len(ys)
+    seeds = np.asarray(seeds, dtype=np.int64).reshape(-1)
+    S = len(seeds)
+    ts = np.arange(0, T_survivability, 0.1)
+    steps = max(int(T_global / params.dt), len(ts))
+    n_slots, table = global_slots(T_global, params.dt, steps)
+    B = min(int(num_envs), S)
+    if B == 0 or nx * ny == 0:
+        raise ValueError("difficulty: no seeds or an empty position grid")
+    grid = (xs[0], ys[0], position_step, nx, ny)
+    env = Drone2DVecEnv(params, B, seeds=seeds[:B], device=device, auto_reset=False, trackers=False, oxford=False,
+                        owl=False, world_gen=world_gen)
+    try:
+        dev = env.device
+        first_hit = torch.empty((S, nx, ny), dtype=torch.int16, device=dev)
+        static_hit = torch.empty((S, nx, ny), dtype=torch.uint8, device=dev)
+        cs = torch.empty((S, nx, ny, n_slots), dtype=torch.uint8, device=dev) if collision_state else None
+        radius = torch.empty((S, env.num_agents), dtype=torch.float64, device=dev)
+        for c0 in range(0, S, B):
+            n = min(B, S - c0)
+            if c0 > 0:
+                if world_gen == "device":
+                    env.reseed(np.arange(n), seeds[c0:c0 + n])
+                else:
+                    torch.cuda.current_stream(dev).synchronize()      # the last call has read the snapshot it replaces
+                    env.set_worlds(generate_worlds(params, seeds[c0:c0 + n], env._smap))
+            out = (first_hit[c0:c0 + n], static_hit[c0:c0 + n]) + ((cs[c0:c0 + n],) if collision_state else ())
+            env.difficulty(steps, grid, envs=range(0, n), slots=table, n_slots=n_slots, collision_state=collision_state,
+                           out=out)
+            radius[c0:c0 + n] = env.buffer("agent_radius")[:n]
+        torch.cuda.current_stream(dev).synchronize()
+        env.check_worlds()
+        fh = first_hit.cpu().numpy().astype(np.int64)
+        sh = static_hit.cpu().numpy().astype(bool)
+        rad = radius.cpu().numpy()
+        cs = cs.cpu().numpy() if collision_state else None
+    finally:
+        env.close()
+    res = survival_from_hits(fh, sh, T_survivability, n_slots, table)
+    res["density"] = _density(params, rad)
+    if collision_state:
+        res["collision_state"] = cs
+    return res

@@ -632,6 +632,48 @@ class Drone2DVecEnv(object):
                                          self._stream()), "d2d_render")
         return out
 
+    # ------------------------------------------------------------------ difficulty metrics
+    def difficulty(self, steps, grid, envs=None, slots=None, n_slots=None, collision_state=False, out=None):
+        """Dynamic and static collisions of a drone held at every position of `grid`, over `steps` agent steps from each
+        env's reset snapshot (d2d_difficulty, one kernel; CVM handles only).  It reads the snapshot and writes only its
+        outputs, so the result does not depend on how far the envs have stepped.
+        grid: (x0, y0, step, nx, ny), positions x0 + i * step, y0 + j * step.  envs: None (all) or a step-1 range.
+        Returns {"first_hit": int16 [count, nx, ny] (first agent step k = 1..steps after which an agent disc grown by the
+        drone radius holds the position; 0: none), "static_hit": uint8 [count, nx, ny] (collision_flag would be 1)} and,
+        with collision_state=True, "collision_state": uint8 [count, nx, ny, n_slots], the array of glob_survivability:
+        slot slots[k-1] is set when step k has a dynamic and no static hit.  slots: one slot per step (default: step k ->
+        slot k-1; shorter tables leave the later steps unrecorded); n_slots defaults to the largest slot + 1.
+        out: preallocated contiguous CUDA tensors of those shapes and dtypes, a tuple (first_hit, static_hit[,
+        collision_state]) -- what a captured CUDA graph writes into."""
+        first, count = 0, self.num_envs
+        if envs is not None:
+            if not (isinstance(envs, range) and envs.step == 1):
+                raise ValueError("difficulty: envs must be None or a step-1 range")
+            first, count = envs.start, max(0, envs.stop - envs.start)
+        spec, n_slots = difficulty_spec(steps, grid, collision_state, slots, n_slots)
+        nx, ny = spec.nx, spec.ny
+        shapes = [((count, nx, ny), torch.int16), ((count, nx, ny), torch.uint8)]
+        if collision_state:
+            shapes.append(((count, nx, ny, n_slots), torch.uint8))
+        if out is None:
+            out = tuple(torch.empty(s, dtype=d, device=self.device) for s, d in shapes)
+        else:
+            out = tuple(out)
+            if len(out) != len(shapes) or any(
+                    not torch.is_tensor(t) or t.dtype != d or tuple(t.shape) != s or not t.is_contiguous() or
+                    t.device.type != "cuda" or t.device.index != self._dev_index for t, (s, d) in zip(out, shapes)):
+                raise ValueError("difficulty: `out` must be contiguous tensors %s on cuda:%d"
+                                 % (", ".join("%s %s" % (d, s) for s, d in shapes), self._dev_index))
+
+        def ptr(t):
+            return C.c_void_p(t.data_ptr() if count else 0)
+        self._check(self._lib.d2d_difficulty(self._h, C.byref(spec), int(first), int(count), ptr(out[0]), ptr(out[1]),
+                                             ptr(out[2]) if collision_state else None, self._stream()), "d2d_difficulty")
+        res = {"first_hit": out[0], "static_hit": out[1]}
+        if collision_state:
+            res["collision_state"] = out[2]
+        return res
+
     def stats(self, reset=False):
         """Episode statistics accumulated on device (int64 [16], names in _native.STAT_NAMES)."""
         out = np.zeros(_native.NUM_STATS, dtype=np.int64)
@@ -653,6 +695,33 @@ class Drone2DVecEnv(object):
             self.close()
         except Exception:
             pass
+
+
+def difficulty_spec(steps, grid, collision_state=False, slots=None, n_slots=None):
+    """The d2d_difficulty_spec of `Drone2DVecEnv.difficulty` and its number of collision_state slots (0 without
+    collision_state)."""
+    x0, y0, step, nx, ny = grid
+    spec = _native.D2DDifficultySpec()
+    spec.struct_size = C.sizeof(_native.D2DDifficultySpec)
+    spec.nx, spec.ny = int(nx), int(ny)
+    spec.x0, spec.y0, spec.step = float(x0), float(y0), float(step)
+    spec.steps = int(steps)
+    if not 1 <= spec.steps <= _native.DIFF_MAX_STEPS:
+        raise ValueError("difficulty: steps %d outside 1..%d" % (spec.steps, _native.DIFF_MAX_STEPS))
+    if not collision_state:
+        return spec, 0
+    table = list(range(spec.steps)) if slots is None else [int(s) for s in slots]
+    if len(table) > spec.steps:
+        raise ValueError("difficulty: %d slots for %d steps" % (len(table), spec.steps))
+    if any(s < 0 or s >= _native.DIFF_NO_SLOT for s in table):
+        raise ValueError("difficulty: slot indices must lie in [0, %d)" % _native.DIFF_NO_SLOT)
+    n = int(n_slots) if n_slots is not None else (max(table) + 1 if table else 0)
+    if n < 1:
+        raise ValueError("difficulty: collision_state needs at least one slot")
+    table += [_native.DIFF_NO_SLOT] * (spec.steps - len(table))
+    spec.n_slots = n
+    spec.slot[:spec.steps] = table
+    return spec, n
 
 
 def trajectory_waypoints(cfg, coeff, nseg, cursor):

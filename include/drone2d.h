@@ -446,6 +446,39 @@ enum { D2D_RENDER_GROUND_TRUTH = 1, D2D_RENDER_BELIEF = 2, D2D_RENDER_VIEW = 4, 
 int d2d_render(d2d_handle *h, const int32_t *envs_host, int32_t first_env, int32_t count, int32_t pixels_per_cell,
                int32_t layers, uint8_t *frames_dev, void *stream);
 
+/* Difficulty: the survivability metric family of the reference (script/difficulty_calculator/survivability_calculator.py,
+ * glob_survivability_calculator.py) evaluated on the device from each env's RESET SNAPSHOT (agent_pos0 / agent_pref0,
+ * agent_radius, ground truth).  The kernel steps the agents alone, K = spec->steps times, with the step kernels' CVM
+ * Agent.step, and after agent step k = 1..K tests every position p of the grid x = x0 + i * step, y = y0 + j * step
+ * (i < nx, j < ny; position index i * ny + j):
+ *   dynamic hit  any agent a: norm(agent_a - p) < r_a + drone_radius     (Drone2D.is_collide's agent test)
+ *   static hit   one of the five probes of Drone2D.is_collide at p meets an occupied or off-map cell (collision_flag 1)
+ * Outputs, DEVICE memory of the handle's device, for envs [first_env, first_env + count):
+ *   first_hit       int16 [count][nx*ny]  first step k with a dynamic hit (0: none within `steps`); statics ignored
+ *   static_hit      uint8 [count][nx*ny]  1 if the drone at p collides with a static cell
+ *   collision_state uint8 [count][nx*ny][n_slots] or NULL: byte [p][slot[k-1]] is OR-ed with (dynamic hit after step k and
+ *                   no static hit) -- glob_survivability's array, collision_flag == 2 -- for every k with slot[k-1] !=
+ *                   D2D_DIFF_NO_SLOT; every other byte is 0.  NULL requires n_slots == 0 and vice versa.
+ * Only CVM handles: under RVO the agents' motion needs d2d_rvo_kernel, and the call returns D2D_ERR_STATE (use the step
+ * kernels, as metrics.global_survivability does).  The planner does not matter.  The spec travels by value in the kernel
+ * parameters: a call is ONE launch with no upload and can be captured in a CUDA graph.  Every argument is checked before
+ * anything is enqueued (a rejected call changes nothing); count = 0 enqueues nothing.  The call reads the reset snapshot and
+ * writes only the outputs: env state, statistics, the episode log and the host mirror are untouched, and the result does not
+ * depend on how far the envs have stepped.  D2D_ERR_STATE before d2d_set_world and while a pipelined step is in flight. */
+#define D2D_DIFF_MAX_POS   1024
+#define D2D_DIFF_MAX_STEPS 1024
+#define D2D_DIFF_NO_SLOT   0xFFFF      /* slot[] entry: step k is not recorded in collision_state */
+typedef struct d2d_difficulty_spec {
+    int32_t struct_size;                  /* sizeof(d2d_difficulty_spec) */
+    int32_t nx, ny;                       /* position grid, nx * ny in 1..D2D_DIFF_MAX_POS */
+    double  x0, y0, step;                 /* finite; step > 0 */
+    int32_t steps;                        /* K agent steps from the reset snapshot, 1..D2D_DIFF_MAX_STEPS */
+    int32_t n_slots;                      /* collision_state slots per position, 0..D2D_DIFF_MAX_STEPS; 0 = not written */
+    uint16_t slot[D2D_DIFF_MAX_STEPS];    /* slot of step k (k = 1..steps): < n_slots or D2D_DIFF_NO_SLOT, non-decreasing */
+} d2d_difficulty_spec;
+int d2d_difficulty(d2d_handle *h, const d2d_difficulty_spec *spec, int32_t first_env, int32_t count, int16_t *first_hit,
+                   uint8_t *static_hit, uint8_t *collision_state, void *stream);
+
 /* Number of kernel launches issued by this handle so far (bench.py's gpu_launches). */
 int64_t d2d_launch_count(const d2d_handle *h);
 
