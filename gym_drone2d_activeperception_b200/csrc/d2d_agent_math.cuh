@@ -4,7 +4,8 @@
 //
 // d2d_cvm_agent_step restates the CVM branch of d2d_phase_agents (d2d_step.cuh) operation for operation; the step kernel
 // keeps its own copy so that its code is unchanged, and tests/test_difficulty_host.py holds the two together through the
-// oracle, which the step kernels are held to.
+// oracle, which the step kernels are held to.  The small-crowd form of the rollout kernel (d2d_agents_lane) steps its
+// agents with this helper; tests/test_gpu_rollout.py holds it to the step kernels bit for bit.
 #pragma once
 #include "d2d_math.cuh"
 

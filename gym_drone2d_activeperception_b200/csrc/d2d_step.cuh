@@ -21,6 +21,7 @@
 #pragma once
 #include "d2d_state.cuh"
 #include "d2d_math.cuh"
+#include "d2d_agent_math.cuh"
 
 // big, once-per-env-step helpers: inlined by default; -DD2D_COLD_NOINLINE=1 keeps one shared copy of each
 #if defined(D2D_COLD_NOINLINE) && D2D_COLD_NOINLINE
@@ -112,6 +113,8 @@ __device__ __forceinline__ BlockCtx d2d_carve(unsigned char *base, int E, int NP
 // ------------------------------------------------------------------------------------------ P0: scalars + bulk loads
 // After the record has been copied into the head of `s`: lazy reset (Drone2DEnv2.__init__, drone_v2.py:88-117: drone at the
 // init pose, zero velocity, WAIT_FOR_GOAL; Planner.__init__ traj_planner.py:22) and this step's scratch.  One thread.
+// CELL = false: ix / iy are left to the caller (the small-crowd rollout keeps them for as long as the pose is unchanged).
+template <bool CELL = true>
 __device__ __forceinline__ void d2d_env_begin(const DevP &P, EnvS &s, bool was_done) {
     const bool rs = s.pending_reset != 0 || (P.auto_reset && was_done);
     s.ox_was_fresh = s.ox_fresh; s.owl_was_fresh = s.owl_fresh;
@@ -122,7 +125,7 @@ __device__ __forceinline__ void d2d_env_begin(const DevP &P, EnvS &s, bool was_d
         s.nseg = 0; s.cursor = 0;
         if (P.planner == D2D_PLANNER_JERK) { s.tgx = 0.0; s.tgy = 0.0; }   // Jerk_Primitive.__init__: target = np.zeros(4) (:406)
     }
-    s.ix = d2d_cell(s.px, P.scale, P.inv_scale); s.iy = d2d_cell(s.py, P.scale, P.inv_scale);
+    if (CELL) { s.ix = d2d_cell(s.px, P.scale, P.inv_scale); s.iy = d2d_cell(s.py, P.scale, P.inv_scale); }
     s.valid = 1; s.reset = rs; s.jerk_has = 0;
     s.ncull = 0; s.coll_agent = 0; s.arch_cnt = 0; s.arch_ts = 0; s.act_cnt = 0; s.act_ts = 0; s.newly = 0; s.done_now = 0;
 }
@@ -364,7 +367,8 @@ __device__ __forceinline__ double d2d_ray_angle(const DevP &P, double yaw, int r
 // Hits on the first 32 entries of the culled list are returned as a bit mask over the LIST SLOTS (the caller ORs the
 // masks of its rays and publishes them once: no shared-memory atomics inside the march, where a disc seen by ~20 rays
 // at the same sample index would serialise them); hits on the unfiltered tail go to `hitw` directly.
-template <bool SAFE = false>
+// SMALL: the culled list never exceeds 32 entries (at most 32 agents), so there is no tail and `hitw` is not used.
+template <bool SAFE = false, bool SMALL = false>
 __device__ __forceinline__ uint32_t d2d_cast_ray(const DevP &P, const EnvS &s, double a, double slope, const RayOut &o,
                                                  const uint64_t *gt, const double *sx, const double *sy, const double *sr2,
                                                  const uint16_t *cull, uint32_t *hitw) {
@@ -395,7 +399,7 @@ __device__ __forceinline__ uint32_t d2d_cast_ray(const DevP &P, const EnvS &s, d
     {
         const double dd2 = xs * xs + ys * ys;
         const float inv_dd2 = 1.0f / (float)dd2;
-        const int ncm = nc < 32 ? nc : 32;
+        const int ncm = (SMALL || nc < 32) ? nc : 32;
 #pragma unroll 1
         for (int q = 0; q < ncm; q++) {
             const int k = cull[q];
@@ -410,7 +414,7 @@ __device__ __forceinline__ uint32_t d2d_cast_ray(const DevP &P, const EnvS &s, d
                 mhi = max(mhi, (int)floorf(t + hw));
             }
         }
-        if (nc > 32) { mlo = 0; mhi = 0x7fff; }                  // unfiltered tail of a very long culled list
+        if (!SMALL && nc > 32) { mlo = 0; mhi = 0x7fff; }        // unfiltered tail of a very long culled list
     }
     const unsigned mspan = mhi >= mlo ? (unsigned)(mhi - mlo) : 0u;   // no candidate: mlo = 0x7fff, (m - mlo) wraps to huge
     // The march runs in MIRRORED coordinates: u = x when the ray moves up the axis, -x when it moves down (negation is
@@ -455,11 +459,13 @@ __device__ __forceinline__ uint32_t d2d_cast_ray(const DevP &P, const EnvS &s, d
                     const double ex = sx[k] - x, ey = sy[k] - y;
                     if (ex * ex + ey * ey <= sr2[k]) { hm |= 1u << q; any = true; }
                 }
+                if (!SMALL) {
 #pragma unroll 1
-                for (int q = 32; q < nc; q++) {
-                    const int k = cull[q];
-                    const double ex = sx[k] - x, ey = sy[k] - y;
-                    if (ex * ex + ey * ey <= sr2[k]) { atomicOr(&hitw[k >> 5], 1u << (k & 31)); any = true; }
+                    for (int q = 32; q < nc; q++) {
+                        const int k = cull[q];
+                        const double ex = sx[k] - x, ey = sy[k] - y;
+                        if (ex * ex + ey * ey <= sr2[k]) { atomicOr(&hitw[k >> 5], 1u << (k & 31)); any = true; }
+                    }
                 }
                 if (any) break;
             }
@@ -546,13 +552,15 @@ __device__ __forceinline__ uint32_t d2d_cast_ray(const DevP &P, const EnvS &s, d
                     any = true;
                 }
             }
+            if (!SMALL) {
 #pragma unroll 1
-            for (int q = 32; q < nc; q++) {
-                const int k = cull[q];
-                const double ex = sx[k] - x, ey = sy[k] - y;
-                if (ex * ex + ey * ey <= sr2[k]) {
-                    atomicOr(&hitw[k >> 5], 1u << (k & 31));
-                    any = true;
+                for (int q = 32; q < nc; q++) {
+                    const int k = cull[q];
+                    const double ex = sx[k] - x, ey = sy[k] - y;
+                    if (ex * ex + ey * ey <= sr2[k]) {
+                        atomicOr(&hitw[k >> 5], 1u << (k & 31));
+                        any = true;
+                    }
                 }
             }
             if (any) break;
@@ -627,8 +635,11 @@ __device__ __forceinline__ int d2d_border_intact(const uint64_t *gt, int lane) {
 // straight-line code (two dependency chains for the scheduler; best when all warps run in phase, i.e. one wave).
 // Otherwise a single copy of the ray body (half the code: best when many waves de-phase the warps and the
 // instruction cache becomes the limiter).
-template <bool ILP2>
-__device__ __forceinline__ void d2d_phase_rays_warp(const DevP &P, const BlockCtx &c, const RayOut &o, int lane) {
+// SMALL (at most 32 agents, single-copy march only): the env's hit mask over AGENTS is returned in every lane instead of
+// being published into the hit words.
+template <bool ILP2, bool SMALL = false>
+__device__ __forceinline__ uint32_t d2d_phase_rays_warp(const DevP &P, const BlockCtx &c, const RayOut &o, int lane) {
+    static_assert(!(ILP2 && SMALL), "the small-crowd form casts one ray per lane per pass");
     const EnvS &s = c.S[0];
     const int R = P.n_rays;
     uint32_t hm = 0u;
@@ -647,16 +658,18 @@ __device__ __forceinline__ void d2d_phase_rays_warp(const DevP &P, const BlockCt
         for (int ray = lane; ray < R; ray += 32) {
             const double a = d2d_ray_angle(P, s.yaw, ray);
             const double tn = d2d_tan(a);
-            if (safe) hm |= d2d_cast_ray<true>(P, s, a, tn, o, c.gt, c.sx, c.sy, c.sr2, c.cull, c.hitw);
-            else hm |= d2d_cast_ray<false>(P, s, a, tn, o, c.gt, c.sx, c.sy, c.sr2, c.cull, c.hitw);
+            if (safe) hm |= d2d_cast_ray<true, SMALL>(P, s, a, tn, o, c.gt, c.sx, c.sy, c.sr2, c.cull, c.hitw);
+            else hm |= d2d_cast_ray<false, SMALL>(P, s, a, tn, o, c.gt, c.sx, c.sy, c.sr2, c.cull, c.hitw);
         }
     }
     // OR over the warp, then lane q publishes slot q (all rays of the env are cast by this warp)
     hm = __reduce_or_sync(0xffffffffu, hm);
+    if (SMALL) return __reduce_or_sync(0xffffffffu, ((hm >> lane) & 1u) ? 1u << c.cull[lane] : 0u);
     if ((hm >> lane) & 1u) {
         const int k = c.cull[lane];
         atomicOr(&c.hitw[k >> 5], 1u << (k & 31));
     }
+    return 0u;
 }
 
 // ------------------------------------------------------------------------------------------ noisy measurements
@@ -1358,6 +1371,95 @@ __global__ void __launch_bounds__(WPB * 32, MINB) d2d_step_fused_warp_kernel(con
     D2D_PROF(3);
 }
 
+// ------------------------------------------------------------------------------------------ small-crowd rollout phases
+// One env per warp and at most 32 agents: lane k owns agent k (global index g), no division, no loop.
+
+// P1: Agent.step under CVM (d2d_rollout serves CVM handles only) from the state the lane holds in registers (live, or the
+// snapshot of an env being reset), which is updated in place.  The culled list is built by ballot; returns whether an
+// agent collides with the drone (Drone2D.is_collide utils.py:773-776).
+__device__ __forceinline__ bool d2d_agents_lane(const DevP &P, const BlockCtx &c, EnvS &s, size_t g, int lane, double2 &pos,
+                                                double2 &pref, double r) {
+    bool in = false, hit = false;
+    if (lane < P.N) {
+        d2d_cvm_agent_step(pos.x, pos.y, pref.x, pref.y, r, P.dt, P.scale, P.map_w, P.map_h);
+        P.apos[g] = pos;
+        P.apref[g] = pref;
+        c.sx[lane] = pos.x; c.sy[lane] = pos.y; c.sr2[lane] = r * r;
+        const double ddx = pos.x - s.px, ddy = pos.y - s.py;
+        const double reach = r + P.cull_reach;
+        in = ddx * ddx + ddy * ddy <= reach * reach;
+        hit = d2d_norm2_lt(ddx, ddy, r + P.drone_r);
+    }
+    const uint32_t b = __ballot_sync(0xffffffffu, in);
+    if (in) c.cull[__popc(b & ((1u << lane) - 1u))] = (uint16_t)lane;
+    if (lane == 0) s.ncull = __popc(b);
+    return __any_sync(0xffffffffu, hit);
+}
+
+// P3: hit flag and Kalman tracker of agent `lane`; hmask is the env's hit mask over agents
+__device__ __forceinline__ void d2d_trackers_lane(const DevP &P, const BlockCtx &c, EnvS &s, size_t g, int lane, uint32_t hmask,
+                                                  uint8_t pf_act) {
+    if (lane >= P.N) return;
+    const bool hit = (hmask >> lane) & 1u;
+    P.hit[g] = hit ? 1 : 0;
+    if (P.trackers) {
+        const bool was_active = !s.reset && pf_act != 0;
+        if (hit && !was_active) atomicAdd(&s.newly, 1);   // utils.py:606-607
+        if (was_active || hit || s.reset) {
+            const bool noisy = P.var_cam != 0.0;
+            d2d_tracker_update(P, s, g, hit, noisy ? c.mx[lane] : c.sx[lane], noisy ? c.my[lane] : c.sy[lane], was_active);
+        }
+    }
+}
+
+// P4 under NoMove, one thread: what d2d_leader_finish + d2d_leader_flags do, given the invariants of the drone's pose `inv`
+// (bit 0: the static probes hit, bit 1: within reach of NoMove's fixed target (-1, -1)).  NoMove.plan always succeeds, so the
+// brake never runs and fail is 0 when the flags are computed: the drone cannot dead-lock.  Only a trajectory written into
+// the record from outside (nseg > 0) can move the drone; step_pos then pops its waypoints through the general code and the
+// invariants are recomputed for the new pose (the static probes of this step were taken before the move, as in is_collide).
+__device__ __forceinline__ void d2d_leader_nomove(const DevP &P, EnvS &s, const uint64_t *gt, int e, double action, bool coll,
+                                                  int &inv) {
+    const int shit = inv & 1;
+    bool goal = (inv & 2) != 0;
+    s.tgx = -1.0; s.tgy = -1.0;                                      // NoMove.plan traj_planner.py:70-73
+    if (s.nseg * P.n_way - s.cursor > 0) {
+        d2d_leader_finish(P, s, gt, e, 0.0, true, false);
+        s.ix = d2d_cell(s.px, P.scale, P.inv_scale); s.iy = d2d_cell(s.py, P.scale, P.inv_scale);
+        goal = d2d_norm2_le(s.px - s.tgx, s.py - s.tgy, 10.0);
+        int sh = 0;
+        for (int q = 0; q < 5; q++) sh |= d2d_static_probe(P, gt, s.px, s.py, q);
+        inv = sh | (goal ? 2 : 0);
+    } else {
+        s.sm = SM_EXECUTING; s.fail = 0;
+    }
+    s.yaw = d2d_pymod(s.yaw + (action * P.max_yaw_speed) * P.dt, 360.0);   // step_yaw utils.py:741-743
+    // is_collide utils.py:764-778: the static probes first, then the agents
+    const int col = shit ? 1 : (coll ? 2 : 0);
+    int frz = 0;
+    if (col == 0) {   // drone_v2.py:222-225
+        if (goal) s.sm = SM_GOAL_REACHED;
+        frz = ((double)s.steps >= P.max_steps) ? 1 : 0;
+    }
+    const int done = (col != 0 || frz || (s.sm == SM_GOAL_REACHED && s.tcur >= P.n_targets)) ? 1 : 0;
+    s.bufc += s.arch_cnt; s.bufts += s.arch_ts; s.tracked += s.newly;
+    if (done) { s.bufc += s.act_cnt; s.bufts += s.act_ts; }
+    s.done_now = done;
+    P.collision[e] = (uint8_t)col; P.dead_lock[e] = 0; P.freezing[e] = (uint8_t)frz; P.done[e] = (uint8_t)done;
+    P.yaw_obs[e] = (float)s.yaw;
+    if (P.yaw_mirror) P.yaw_mirror[e] = (float)s.yaw;
+    if (P.done_mirror) P.done_mirror[e] = (uint8_t)done;
+    if (done) {
+        atomicAdd(&P.stats[D2D_STAT_EPISODES], 1ull);
+        if (s.sm == SM_GOAL_REACHED) atomicAdd(&P.stats[D2D_STAT_SUCCESS], 1ull);
+        if (col == 1) atomicAdd(&P.stats[D2D_STAT_STATIC_COLLISION], 1ull);
+        if (col == 2) atomicAdd(&P.stats[D2D_STAT_DYNAMIC_COLLISION], 1ull);
+        if (frz) atomicAdd(&P.stats[D2D_STAT_FREEZING], 1ull);
+        atomicAdd(&P.stats[D2D_STAT_FLIGHT_STEPS], (unsigned long long)s.steps);
+        atomicAdd(&P.stats[D2D_STAT_AGENTS_TRACKED], (unsigned long long)s.bufc);
+        atomicAdd(&P.stats[D2D_STAT_TRACKED_STEPS], (unsigned long long)s.bufts);
+    }
+}
+
 // =============================================================================================================
 // Multi-step ("rollout") variant of the fused warp kernel: consecutive Drone2DEnv2.step calls of an env in ONE launch.
 // Step k+1 of an env depends on step k of the SAME env only, so a warp that owns an env can walk it through many steps
@@ -1381,13 +1483,30 @@ __global__ void __launch_bounds__(WPB * 32, MINB) d2d_step_fused_warp_kernel(con
 //   cache and a third of the warp-state samples become `no_instruction` stalls (profiles/r2_ncu_rollout_cfg2_nosync.txt:
 //   20.1 us per step without the barrier, 16.9 us with 28-warp blocks and one barrier per step).  The gate re-aligns the
 //   warps by itself, so the GATED form needs no barrier.
+//
+// SMALL (d2d_rollout when N <= 32; GATED = false only): the small-crowd form.  A latency-bound warp's step is a chain of
+//   mostly lane-serial code, so the form strips what N <= 32 and NoMove make constant:
+//   - every warp slice is carved for exactly 32 agents and one hit word, so each shared-memory array sits at a fixed offset
+//     from the slice base (an immediate) instead of being derived from the runtime N;
+//   - lane k owns agent k in the agent and tracker phases; the culled list (at most 32 entries) is built by ballot, the
+//     drone-vs-agent test is a warp vote, the march has no tail beyond 32 entries, and the env's hit mask comes out of the
+//     ray phase as a warp reduction (stored into the hit word only for the noisy-measurement walk);
+//   - under NoMove the drone's pose changes only when the env is reset (or when waypoints were written into the record from
+//     outside), so the drone cell, the five static probes and the goal test against NoMove's fixed target are computed
+//     once per pose and kept in registers: at kernel entry (after the bulk copy of the ground truth has landed), after
+//     every in-kernel reset and after a popped waypoint.  They are never stored in the env record: clone / save / load,
+//     d2d_set_drone_pose and in-place reseeding rewrite the record between launches, and every launch recomputes them
+//     from whatever the record holds.
+//   Results are bit-identical to the general form (tests/test_gpu_rollout.py, tests/test_gpu_rollout_small.py: N = 10, 32, 33).
 // =============================================================================================================
 #define D2D_GATE_STAMP_SLOT(B) ((size_t)(B))     // staging slot behind the B action slots: (session step << 1) | more
+#define D2D_SMALL_N 32                           // agents the small-crowd rollout form carves every warp slice for
 
-template <int WPB, int MINB, bool SYNC, bool GATED>
+template <int WPB, int MINB, bool SYNC, bool GATED, bool SMALL = false>
 __global__ void __launch_bounds__(WPB * 32, MINB) d2d_rollout_warp_kernel(const DevP P, const double *__restrict__ actions,
                                                                           int K, long long action_stride, int sync_every,
                                                                           unsigned int t_first) {
+    static_assert(!(SMALL && GATED), "the small-crowd form serves d2d_rollout only");
     extern __shared__ __align__(128) unsigned char smem[];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int e = blockIdx.x * WPB + wid;
@@ -1444,12 +1563,16 @@ __global__ void __launch_bounds__(WPB * 32, MINB) d2d_rollout_warp_kernel(const 
         if (SYNC) for (int t = 1; t < K; t++) if (t % sync_every == 0) __syncthreads();
         return;
     }
-    unsigned char *slice = smem + (size_t)wid * d2d_warp_slice_bytes(P.NP, P.HW, GATED ? D2D_FUSED_WARP_EXTRA : 0);
-    const BlockCtx c = d2d_carve(slice, 1, P.NP, P.HW);
-    uint32_t *chg = (uint32_t *)(slice + d2d_step_smem_bytes(1, P.NP, P.HW));   // GATED: this step's changed cells
+    // slice layout: SMALL carves every slice for D2D_SMALL_N agents and one hit word (compile-time offsets)
+    unsigned char *slice = smem + (size_t)wid * d2d_warp_slice_bytes(SMALL ? D2D_SMALL_N : P.NP, SMALL ? 1 : P.HW,
+                                                                     GATED ? D2D_FUSED_WARP_EXTRA : 0);
+    const BlockCtx c = d2d_carve(slice, 1, SMALL ? D2D_SMALL_N : P.NP, SMALL ? 1 : P.HW);
+    // GATED: this step's changed cells
+    uint32_t *chg = (uint32_t *)(slice + d2d_step_smem_bytes(1, SMALL ? D2D_SMALL_N : P.NP, SMALL ? 1 : P.HW));
     int *nchg = (int *)(chg + D2D_CHG_CAP);
     // GATED: block-level publication area behind the warp slices: arrival counter, this step's yaw / done of the block's envs
-    unsigned char *blk = smem + (size_t)WPB * d2d_warp_slice_bytes(P.NP, P.HW, GATED ? D2D_FUSED_WARP_EXTRA : 0);
+    unsigned char *blk = smem + (size_t)WPB * d2d_warp_slice_bytes(SMALL ? D2D_SMALL_N : P.NP, SMALL ? 1 : P.HW,
+                                                                   GATED ? D2D_FUSED_WARP_EXTRA : 0);
     int *blk_cnt = (int *)blk;
     unsigned int *blk_yaw = (unsigned int *)(blk + 16);             // float bits; handed over with shared-memory atomics (below)
     unsigned int *blk_done = (unsigned int *)(blk + 16 + WPB * 4);
@@ -1474,11 +1597,14 @@ __global__ void __launch_bounds__(WPB * 32, MINB) d2d_rollout_warp_kernel(const 
     }
     d2d_load_env_warp(P, s, e, lane);
     if (lane == 0) c.misc[1] = s.reset;
+    if (!SMALL) {
 #pragma unroll 1
-    for (int w = lane; w < P.HW; w += 32) c.hitw[w] = 0u;
+        for (int w = lane; w < P.HW; w += 32) c.hitw[w] = 0u;
+    }
     __syncwarp();
     int border_ok = 0;
     const bool mirror = GATED && P.lm_mirror != nullptr;
+    int inv = 0;   // SMALL, lane 0: the drone-pose invariants of the current pose (bit 0: static probes, bit 1: goal test)
 #pragma unroll 1
     for (int t = 0;;) {
         // here: the record is begun (d2d_env_begin), c.misc[1] = s.reset, the hit words are clear, pf_* hold the live agent
@@ -1486,10 +1612,27 @@ __global__ void __launch_bounds__(WPB * 32, MINB) d2d_rollout_warp_kernel(const 
         D2D_PROF(0);
         d2d_reset_prefetch(P, s, e, lane, pf_pos, pf_pref);
         d2d_reset_arrays(P, c, e, 1, lane, 32, t == 0 ? c.mbar : nullptr);
-        d2d_phase_agents<true, true>(P, c, e, 1, lane, 32, pf_pos, pf_pref, pf_r, &pf_pos, &pf_pref);
+        bool coll = false;
+        if (SMALL) coll = d2d_agents_lane(P, c, s, ga, lane, pf_pos, pf_pref, pf_r);
+        else d2d_phase_agents<true, true>(P, c, e, 1, lane, 32, pf_pos, pf_pref, pf_r, &pf_pos, &pf_pref);
         if (t == 0 && pf_act && !s.reset) d2d_prefetch_tracker(P, ga);
         if (lane == 0) d2d_leader_begin(P, s);
         __syncwarp();
+        if (SMALL) {
+            if (t == 0) {
+                d2d_mbar_wait(c.mbar, 0);
+                border_ok = d2d_border_intact(c.gt, lane);           // the ground truth never changes
+            }
+            if (t == 0 || s.reset) {                                 // warp-uniform: a pose from the record or the reset pose
+                const double px = s.px, py = s.py;
+                const int sh = __any_sync(0xffffffffu, lane < 5 ? d2d_static_probe(P, c.gt, px, py, lane) : 0);
+                if (lane == 0) {
+                    inv = sh | (d2d_norm2_le(px - -1.0, py - -1.0, 10.0) ? 2 : 0);   // NoMove's target is (-1, -1)
+                    s.ix = d2d_cell(px, P.scale, P.inv_scale); s.iy = d2d_cell(py, P.scale, P.inv_scale);
+                }
+                __syncwarp();
+            }
+        }
         // same window as the observation tensor holds: patched in place by the rays; an env that starts a new episode there
         // has its slice cleared first (d2d_obs_clear_warp) -- GATED: on the device only, the host mirror gets the finished slice
         // behind the gate
@@ -1502,21 +1645,25 @@ __global__ void __launch_bounds__(WPB * 32, MINB) d2d_rollout_warp_kernel(const 
         ro.bel_s = c.belief; ro.e = e; ro.patch = patch ? 1 : 0;
         ro.wi = s.ix - 16; ro.wj = s.iy - 16;
         ro.chg = (mirror && patch && !refill) ? chg : nullptr; ro.nchg = nchg; ro.defer_mirror = GATED ? 1 : 0;
-        if (t == 0) {
+        if (!SMALL && t == 0) {
             d2d_mbar_wait(c.mbar, 0);
             border_ok = d2d_border_intact(c.gt, lane);               // the ground truth never changes
         }
         ro.border_ok = border_ok;
         D2D_PROF(1);
-        d2d_phase_rays_warp<false>(P, c, ro, lane);
+        const uint32_t hmask = d2d_phase_rays_warp<false, SMALL>(P, c, ro, lane);
         __syncwarp();
         D2D_PROF(2);
         if (P.var_cam != 0.0) {
-            if (lane == 0) d2d_measure_env(P, c, e);
+            if (lane == 0) {
+                if (SMALL) c.hitw[0] = hmask;
+                d2d_measure_env(P, c, e);
+            }
             __syncwarp();
         }
-        d2d_phase_trackers<true>(P, c, e, 1, lane, 32, pf_act);
-        const int shit = __any_sync(0xffffffffu, lane < 5 ? d2d_static_probe(P, c.gt, s.px, s.py, lane) : 0);
+        if (SMALL) d2d_trackers_lane(P, c, s, ga, lane, hmask, pf_act);
+        else d2d_phase_trackers<true>(P, c, e, 1, lane, 32, pf_act);
+        const int shit = SMALL ? 0 : __any_sync(0xffffffffu, lane < 5 ? d2d_static_probe(P, c.gt, s.px, s.py, lane) : 0);
         __syncwarp();
         int more = (t + 1 < K) ? 1 : 0;
         bool rewrite = false;
@@ -1582,9 +1729,12 @@ __global__ void __launch_bounds__(WPB * 32, MINB) d2d_rollout_warp_kernel(const 
             __syncwarp();
         } else {
             if (lane == 0) {
-                s.tgx = -1.0; s.tgy = -1.0;                          // NoMove.plan traj_planner.py:70-73
-                d2d_leader_finish(P, s, c.gt, e, action, true);
-                d2d_leader_flags(P, s, c.gt, e, shit);
+                if (SMALL) d2d_leader_nomove(P, s, c.gt, e, action, coll, inv);
+                else {
+                    s.tgx = -1.0; s.tgy = -1.0;                      // NoMove.plan traj_planner.py:70-73
+                    d2d_leader_finish(P, s, c.gt, e, action, true);
+                    d2d_leader_flags(P, s, c.gt, e, shit);
+                }
                 if (patch && P.lm_mirror) {
                     int *cnt = (int *)(c.belief + D2D_MIRCNT_OFF);
                     const int nb = *cnt;
@@ -1645,12 +1795,14 @@ __global__ void __launch_bounds__(WPB * 32, MINB) d2d_rollout_warp_kernel(const 
         // ---- next step of the same env: what d2d_load_env_warp does at kernel entry, from the live record
         if (!GATED) action = actions[(size_t)t * (size_t)action_stride + e];
         if (P.trackers && lane < P.N) pf_act = P.trk_active[ga];     // written by this very lane in the tracker phase
+        if (!SMALL) {
 #pragma unroll 1
-        for (int w = lane; w < P.HW; w += 32) c.hitw[w] = 0u;
+            for (int w = lane; w < P.HW; w += 32) c.hitw[w] = 0u;
+        }
         __syncwarp();
         if (lane == 0) {
             const bool was_done = s.done_now != 0;
-            d2d_env_begin(P, s, was_done);
+            d2d_env_begin<!SMALL>(P, s, was_done);
             c.misc[1] = s.reset;
             if (GATED) *nchg = 0;
         }

@@ -1033,15 +1033,16 @@ extern "C" int d2d_step_plan_oxford(d2d_handle *h, const double *actions_dev, do
 
 #define D2D_RESIDENT_WPB 28          // resident gated kernel: one 28-warp block per SM (28 x 148 = 4144 envs in flight)
 
-template <int WPB, int MINB, bool SYNC, bool GATED>
+template <int WPB, int MINB, bool SYNC, bool GATED, bool SMALL = false>
 static int launch_rollout(d2d_handle *h, const double *actions, int K, long long stride, cudaStream_t st, unsigned int t_first = 0,
                           int extra_blocks = 0) {
-    const size_t smem = (size_t)WPB * d2d_warp_slice_bytes(h->NP, h->HW, GATED ? D2D_FUSED_WARP_EXTRA : 0) + (GATED ? 256 : 0);
+    const size_t smem = (size_t)WPB * d2d_warp_slice_bytes(SMALL ? D2D_SMALL_N : h->NP, SMALL ? 1 : h->HW,
+                                                           GATED ? D2D_FUSED_WARP_EXTRA : 0) + (GATED ? 256 : 0);
     if (smem > 227 * 1024) { h->err = "rollout kernel: shared memory per block exceeds 227 KB"; return D2D_ERR_INVALID; }
-    const int rc = ensure_smem_attr(h, (const void *)d2d_rollout_warp_kernel<WPB, MINB, SYNC, GATED>, "rollout warp");
+    const int rc = ensure_smem_attr(h, (const void *)d2d_rollout_warp_kernel<WPB, MINB, SYNC, GATED, SMALL>, "rollout warp");
     if (rc != D2D_OK) return rc;
     static const int sync_every = getenv("D2D_ROLLOUT_SYNC") ? atoi(getenv("D2D_ROLLOUT_SYNC")) : 1;
-    d2d_rollout_warp_kernel<WPB, MINB, SYNC, GATED><<<(h->B + WPB - 1) / WPB + extra_blocks, WPB * 32, smem, st>>>(
+    d2d_rollout_warp_kernel<WPB, MINB, SYNC, GATED, SMALL><<<(h->B + WPB - 1) / WPB + extra_blocks, WPB * 32, smem, st>>>(
         h->P, actions, K, stride, sync_every > 0 ? sync_every : 1, t_first);
     return D2D_OK;
 }
@@ -1098,7 +1099,10 @@ extern "C" int d2d_rollout(d2d_handle *h, const double *actions_dev, int32_t num
         case 2: rc = launch_rollout<4, 7, true, false>(h, actions_dev, num_steps, action_stride, st); break;
         case 3: rc = launch_rollout<7, 4, true, false>(h, actions_dev, num_steps, action_stride, st); break;
         case 4: rc = launch_rollout<14, 2, true, false>(h, actions_dev, num_steps, action_stride, st); break;
-        default: rc = launch_rollout<28, 1, true, false>(h, actions_dev, num_steps, action_stride, st); break;
+        // the small-crowd form (N <= 32, see d2d_rollout_warp_kernel); larger crowds take the general one
+        default: rc = h->N <= D2D_SMALL_N ? launch_rollout<28, 1, true, false, true>(h, actions_dev, num_steps, action_stride, st)
+                                          : launch_rollout<28, 1, true, false>(h, actions_dev, num_steps, action_stride, st);
+                 break;
     }
     if (rc != D2D_OK) return rc;
     h->launches++;
