@@ -6,7 +6,7 @@ Public API (mirrors the reference's names):
     generate_world(s) -- host-side world generation from seeds (drone_v2.py:12-117)
 """
 from .params import Params, grid_type, state_machine  # noqa: F401
-from .world import generate_world, generate_worlds, count_agents, load_static_map  # noqa: F401
+from .world import generate_world, generate_worlds, count_agents, load_static_map, world_key, split_world_key  # noqa: F401
 
 
 def __getattr__(name):

@@ -53,6 +53,7 @@ class D2DJerkTables(C.Structure):
 
 WORLD_MAX_RANDOM, WORLD_MAX_PILLARS, WORLD_GROUPS = 256, 64, 100
 WORLD_EAGER, WORLD_LAZY = 1, 2
+WORLD_MAX_SOURCES = 4096                # world sources of one handle (d2d_set_world_sources); key = source * 2**32 + seed
 
 # d2d_render: frame layers (drone2d.h D2D_RENDER_*), drawn back to front in this order
 RENDER_MAX_PPC, RENDER_MAX_LIST = 10, 1024
@@ -106,7 +107,8 @@ EXPORTS = ["d2d_version", "d2d_last_error", "d2d_create", "d2d_destroy", "d2d_se
            "d2d_step_host", "d2d_bind_host_mirror", "d2d_bind_host_io", "d2d_step_bound", "d2d_step_pipelined", "d2d_plan_oxford", "d2d_step_plan_oxford", "d2d_step_bound_plan_oxford", "d2d_plan_gaze", "d2d_set_drone_pose", "d2d_get_buffer", "d2d_stats",
            "d2d_launch_count", "d2d_clone_envs", "d2d_state_layout", "d2d_save_state", "d2d_load_state",
            "d2d_set_world_source", "d2d_generate_worlds", "d2d_enable_episode_log", "d2d_read_episode_log",
-           "d2d_set_seed_queue", "d2d_render", "d2d_difficulty"]
+           "d2d_set_seed_queue", "d2d_render", "d2d_difficulty", "d2d_set_world_sources", "d2d_generate_worlds_keyed",
+           "d2d_set_world_queue"]
 
 _lib = None
 
@@ -162,6 +164,9 @@ def load():
     L.d2d_enable_episode_log.argtypes = [vp, C.c_int64]
     L.d2d_read_episode_log.argtypes = [vp, vp, C.POINTER(C.c_int64), C.POINTER(C.c_int64), vp]
     L.d2d_set_seed_queue.argtypes = [vp, vp, C.c_int64, vp]
+    L.d2d_set_world_sources.argtypes = [vp, vp, C.c_int32]
+    L.d2d_generate_worlds_keyed.argtypes = [vp, vp, vp, C.c_int32, C.c_int32, vp]
+    L.d2d_set_world_queue.argtypes = [vp, vp, C.c_int64, vp]
     L.d2d_render.argtypes = [vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, vp, vp]
     L.d2d_difficulty.argtypes = [vp, C.POINTER(D2DDifficultySpec), C.c_int32, C.c_int32, vp, vp, vp, vp]
     for name in EXPORTS:

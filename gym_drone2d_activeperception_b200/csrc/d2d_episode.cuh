@@ -13,13 +13,13 @@ struct EpLog {
     d2d_episode_record *rec;     // [capacity]
     long long capacity;
     long long *head;             // [4]
-    long long *world_seed;       // [B]
+    long long *world_seed;       // [B] world key of each env
     int *list;                   // [B] scratch: the envs that reported done this step, ascending (each block its own entries)
     int *gen_env;                // [B] worlds the queue handed out this step (read by d2d_worldgen_list_kernel) ...
-    uint32_t *gen_seed;          // [B] ... their seeds
+    long long *gen_key;          // [B] ... their world keys
     int *gen_count;              // ... and their number
     unsigned int *ticket;        // blocks of d2d_episode_log_kernel done with this step (0 between launches)
-    const long long *queue;      // [head[3]] seeds of the queue
+    const long long *queue;      // [head[3]] world keys of the queue
 };
 
 // bit k of the result: byte k of the 16 bytes is non-zero
@@ -108,7 +108,7 @@ __global__ void __launch_bounds__(D2D_EP_THREADS) d2d_episode_log_kernel(const D
             if (j < taken) {
                 const long long s = L.queue[q0 + j];
                 L.world_seed[e] = s;
-                L.gen_env[j] = e; L.gen_seed[j] = (uint32_t)s;
+                L.gen_env[j] = e; L.gen_key[j] = s;
             }
         }
     }

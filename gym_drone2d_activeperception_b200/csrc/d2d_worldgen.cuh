@@ -22,7 +22,8 @@
 #define D2D_WG_GRID 50                   // cells per side (D2D_GRID; this header does not need d2d_state.cuh)
 #define D2D_WG_MAX_OBS 16                // RVO obstacle rows per env (D2D_RVO_MAX_OBS)
 
-// Seed-independent tables derived once from d2d_world_source and the config (wg_build_tables), in device memory.
+// Seed-independent tables derived from one d2d_world_source and the config (wg_build_tables); the device holds one per
+// source of the handle's table (d2d_set_world_sources), indexed by the key's high word.
 struct WgTables {
     d2d_world_source src;
     uint32_t mt_base[D2D_MT_N];          // init_genrand(19650218): the start of every init_by_array
@@ -320,13 +321,29 @@ __device__ __forceinline__ double wg_random(uint32_t *mt, int &pos, int lane) {
     return wg_random53(a, wg_next(mt, pos, lane));
 }
 
-// One warp per generated world: envs[w] gets the world of seeds[w].  lazy: also mark the env pending_reset.  A placement
-// that exceeds D2D_WORLD_MAX_REJECTS stores (1 << 63 | env << 32 | seed) into *fault (mapped host word) and abandons the env.
-// The body is shared with d2d_worldgen_list_kernel through d2d_worldgen_body.inc.
-__global__ void __launch_bounds__(D2D_WG_WARPS * 32) d2d_worldgen_kernel(const DevP P, const WgTables *__restrict__ Tg,
+// A world given up: the first warp to claim the (device) claim word stores the env into fault[1] and then (1 << 63 | key)
+// into fault[0] (mapped host words), so the host never pairs one world's key with another's env.  The host clears the words
+// and the claim when it reports the failure.
+__device__ __noinline__ void wg_report_fault(volatile unsigned long long *fault, unsigned int *claim, int env, long long key) {
+    if (atomicCAS(claim, 0u, 1u) != 0u) return;
+    fault[1] = (unsigned long long)env;
+    __threadfence_system();
+    fault[0] = (1ull << 63) | (unsigned long long)key;
+}
+
+// Blocks per SM the generation kernels are compiled for (__launch_bounds__): 8 for d2d_worldgen_kernel and 7 for
+// d2d_worldgen_list_kernel cap them at 64 and 72 registers, the figures of the single-table kernels, so reading the table
+// through the key costs no occupancy (the 22.7 KB of shared memory per block would allow 9).
+#define D2D_WG_MIN_BLOCKS 8
+#define D2D_WG_LIST_MIN_BLOCKS 7
+
+// One warp per generated world: envs[w] gets the world of keys[w] (source << 32 | seed), built from the tables Tg[source].
+// lazy: also mark the env pending_reset.  A placement that exceeds D2D_WORLD_MAX_REJECTS is reported (wg_report_fault) and
+// the env abandoned.  The body is shared with d2d_worldgen_list_kernel through d2d_worldgen_body.inc.
+__global__ void __launch_bounds__(D2D_WG_WARPS * 32, D2D_WG_MIN_BLOCKS) d2d_worldgen_kernel(const DevP P, const WgTables *__restrict__ Tg,
                                                                           const int *__restrict__ envs,
-                                                                          const uint32_t *__restrict__ seeds, int count, int lazy,
-                                                                          volatile unsigned long long *fault) {
+                                                                          const long long *__restrict__ keys, int count, int lazy,
+                                                                          volatile unsigned long long *fault, unsigned int *claim) {
     __shared__ WgWarp sh[D2D_WG_WARPS];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int w = blockIdx.x * D2D_WG_WARPS + wid;
@@ -338,11 +355,12 @@ __global__ void __launch_bounds__(D2D_WG_WARPS * 32) d2d_worldgen_kernel(const D
 
 // The worlds the seed queue handed out in the step just logged (d2d_episode_log_kernel): list and count are device data, so
 // the launch needs no host round trip and can be captured in a graph.  Grid-stride over warps; always lazy.
-__global__ void __launch_bounds__(D2D_WG_WARPS * 32) d2d_worldgen_list_kernel(const DevP P, const WgTables *__restrict__ Tg,
+__global__ void __launch_bounds__(D2D_WG_WARPS * 32, D2D_WG_LIST_MIN_BLOCKS) d2d_worldgen_list_kernel(const DevP P, const WgTables *__restrict__ Tg,
                                                                                const int *__restrict__ envs,
-                                                                               const uint32_t *__restrict__ seeds,
+                                                                               const long long *__restrict__ keys,
                                                                                const int *__restrict__ count,
-                                                                               volatile unsigned long long *fault) {
+                                                                               volatile unsigned long long *fault,
+                                                                               unsigned int *claim) {
     __shared__ WgWarp sh[D2D_WG_WARPS];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int lazy = 1;

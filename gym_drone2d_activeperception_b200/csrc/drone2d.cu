@@ -68,20 +68,23 @@ struct d2d_handle {
     std::vector<int32_t> clone_stage;     // host staging of those arrays
     cudaEvent_t clone_ev = nullptr;       // recorded behind the last kernel that read clone_idx
     double *ox_export = nullptr;          // lazily allocated [B][2500] view of last_time_observed
-    // world generation (d2d_set_world_source / d2d_generate_worlds)
-    WgTables *wg_tab = nullptr;           // device copy of the seed-independent tables
-    int32_t *wg_idx = nullptr;            // device: [count] envs, [count] seeds (u32), [num_envs] eager reset mask
+    // world generation (d2d_set_world_sources / d2d_generate_worlds_keyed)
+    WgTables *wg_tab = nullptr;           // device table of the seed-independent tables, one per world source
+    int32_t wg_count = 0;                 // sources in the table (the valid range of a key's high word)
+    int32_t wg_cap = 0;                   // sources wg_tab can hold (grows only)
+    int32_t *wg_idx = nullptr;            // device: [count] envs, (8-byte aligned) [count] keys (i64), [num_envs] reset mask
     size_t wg_idx_bytes = 0;
     std::vector<int32_t> wg_stage;        // host staging of those arrays
     cudaEvent_t wg_ev = nullptr;          // recorded behind the last kernel that read wg_idx
-    volatile unsigned long long *wg_fault = nullptr;   // pinned, mapped: (1 << 63 | env << 32 | seed) of a world given up
+    volatile unsigned long long *wg_fault = nullptr;   // pinned, mapped [2]: (1 << 63 | key), env of a world given up
     unsigned long long *wg_fault_dev = nullptr;        // device-visible address of wg_fault
-    // episode log and seed queue (d2d_enable_episode_log / d2d_set_seed_queue); ep_mem == nullptr: disabled
-    unsigned char *ep_mem = nullptr;      // records, head, world_seed, list, gen_env, gen_seed, gen_count in one allocation
+    unsigned int *wg_claim = nullptr;     // device: non-zero once a kernel has claimed wg_fault (first failure wins)
+    // episode log and seed queue (d2d_enable_episode_log / d2d_set_world_queue); ep_mem == nullptr: disabled
+    unsigned char *ep_mem = nullptr;      // records, head, world_seed, list, gen_env, gen_key, gen_count in one allocation
     EpLog ep = {};
     long long *ep_queue = nullptr;        // device copy of the queue
-    int64_t ep_queue_cap = 0;             // seeds it can hold
-    int64_t ep_qlen = 0;                  // seeds of the current queue (0: no queue, no generation launch)
+    int64_t ep_queue_cap = 0;             // keys it can hold
+    int64_t ep_qlen = 0;                  // keys of the current queue (0: no queue, no generation launch)
     int ep_blocks = 1;                    // grid of d2d_episode_log_kernel: one block per 32 envs, at most one per SM
     long long ep_qhead[2] = {0, 0};       // host staging of head[2], head[3]
     // zero-copy observation mirror (d2d_bind_host_mirror): host addresses as bound; *_stale: the host copy must be
@@ -652,6 +655,7 @@ extern "C" int d2d_destroy(d2d_handle *h) {
     if (h->wg_idx) cudaFree(h->wg_idx);
     if (h->wg_ev) cudaEventDestroy(h->wg_ev);
     if (h->wg_fault) cudaFreeHost((void *)h->wg_fault);
+    if (h->wg_claim) cudaFree(h->wg_claim);
     if (h->ep_mem) cudaFree(h->ep_mem);
     if (h->ep_queue) cudaFree(h->ep_queue);
     delete h;
@@ -952,7 +956,7 @@ static int log_step(d2d_handle *h, cudaStream_t st) {
     if (h->ep_qlen > 0) {
         const int blocks = (h->B + D2D_WG_WARPS - 1) / D2D_WG_WARPS;
         d2d_worldgen_list_kernel<<<blocks < 4 * 148 ? blocks : 4 * 148, D2D_WG_WARPS * 32, 0, st>>>(
-            h->P, h->wg_tab, h->ep.gen_env, h->ep.gen_seed, h->ep.gen_count, h->wg_fault_dev);
+            h->P, h->wg_tab, h->ep.gen_env, h->ep.gen_key, h->ep.gen_count, h->wg_fault_dev, h->wg_claim);
         h->launches++;
     }
     CUDA_TRY(h, cudaGetLastError());
@@ -1520,66 +1524,121 @@ extern "C" int d2d_load_state(d2d_handle *h, const int32_t *envs_host, int32_t c
 }
 
 // ------------------------------------------------------------------------------------------ world generation
-extern "C" int d2d_set_world_source(d2d_handle *h, const d2d_world_source *src) {
+extern "C" int d2d_set_world_sources(d2d_handle *h, const d2d_world_source *srcs, int32_t count) {
     if (!h) return D2D_ERR_INVALID;
-    if (!src) { h->err = "d2d_set_world_source: null source"; return D2D_ERR_INVALID; }
+    if (!srcs || count < 1 || count > D2D_WORLD_MAX_SOURCES) {
+        h->err = "d2d_set_world_sources: " + std::to_string(count) + " sources (1.." + std::to_string(D2D_WORLD_MAX_SOURCES) +
+                 ", non-null array)";
+        return D2D_ERR_INVALID;
+    }
     D2D_NO_PIPE(h);
-    std::vector<unsigned char> tmp(sizeof(WgTables));
+    std::vector<unsigned char> tmp((size_t)count * sizeof(WgTables));
     WgTables *T = (WgTables *)tmp.data();
-    const char *bad = wg_build_tables(T, src, h->cfg.targets, h->cfg.n_targets, h->cfg.map_scale, h->N, h->P.motion_rvo,
-                                      h->cfg.var_cam != 0.0 ? 1 : 0);
-    if (bad) { h->err = std::string("d2d_set_world_source: ") + bad; return D2D_ERR_INVALID; }
-    if (src->map_w != h->cfg.map_w || src->map_h != h->cfg.map_h || src->drone_radius != h->cfg.drone_radius ||
-        src->agent_radius != h->cfg.agent_radius) {
-        h->err = "d2d_set_world_source: map size, drone_radius or agent_radius differ from the config"; return D2D_ERR_INVALID;
+    for (int32_t i = 0; i < count; i++) {           // all checked before anything changes
+        const d2d_world_source *src = srcs + i;
+        const char *bad = wg_build_tables(T + i, src, h->cfg.targets, h->cfg.n_targets, h->cfg.map_scale, h->N,
+                                          h->P.motion_rvo, h->cfg.var_cam != 0.0 ? 1 : 0);
+        if (!bad && (src->map_w != h->cfg.map_w || src->map_h != h->cfg.map_h || src->drone_radius != h->cfg.drone_radius ||
+                     src->agent_radius != h->cfg.agent_radius))
+            bad = "map size, drone_radius or agent_radius differ from the config";
+        if (bad) { h->err = "d2d_set_world_sources: source " + std::to_string(i) + ": " + bad; return D2D_ERR_INVALID; }
     }
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    if (!h->wg_tab) CUDA_TRY(h, cudaMalloc((void **)&h->wg_tab, sizeof(WgTables)));
     if (!h->wg_fault) {
-        CUDA_TRY(h, cudaHostAlloc((void **)&h->wg_fault, sizeof(unsigned long long), cudaHostAllocMapped));
-        *h->wg_fault = 0ull;
+        CUDA_TRY(h, cudaHostAlloc((void **)&h->wg_fault, 2 * sizeof(unsigned long long), cudaHostAllocMapped));
+        h->wg_fault[0] = 0ull; h->wg_fault[1] = 0ull;
         CUDA_TRY(h, cudaHostGetDevicePointer((void **)&h->wg_fault_dev, (void *)h->wg_fault, 0));
     }
-    if (h->wg_ev) CUDA_TRY(h, cudaEventSynchronize(h->wg_ev));     // no generation kernel may still read the old tables
-    CUDA_TRY(h, cudaMemcpy(h->wg_tab, T, sizeof(WgTables), cudaMemcpyHostToDevice));
+    if (!h->wg_claim) {
+        CUDA_TRY(h, cudaMalloc((void **)&h->wg_claim, sizeof(unsigned int)));
+        CUDA_TRY(h, cudaMemset(h->wg_claim, 0, sizeof(unsigned int)));
+    }
+    if (count > h->wg_cap) {                        // grows only: a captured graph keeps a valid table address until then
+        CUDA_TRY(h, cudaDeviceSynchronize());        // no generation kernel may still read the old table
+        WgTables *t = nullptr;
+        if (cudaMalloc((void **)&t, (size_t)count * sizeof(WgTables)) != cudaSuccess) {
+            cudaGetLastError();
+            h->err = "d2d_set_world_sources: cudaMalloc failed"; return D2D_ERR_NOMEM;
+        }
+        if (h->wg_tab) cudaFree(h->wg_tab);
+        h->wg_tab = t; h->wg_cap = count;
+    } else {
+        CUDA_TRY(h, cudaDeviceSynchronize());        // no generation kernel (nor one behind a queue step) may still read it
+    }
+    CUDA_TRY(h, cudaMemcpy(h->wg_tab, T, (size_t)count * sizeof(WgTables), cudaMemcpyHostToDevice));
+    h->wg_count = count;
     return D2D_OK;
 }
 
-// A world the generation kernels gave up on: reported (and cleared) by the next d2d_generate_worlds / d2d_read_episode_log.
-static bool take_wg_fault(d2d_handle *h, const char *what) {
-    const unsigned long long fault = h->wg_fault ? *h->wg_fault : 0ull;
+extern "C" int d2d_set_world_source(d2d_handle *h, const d2d_world_source *src) { return d2d_set_world_sources(h, src, 1); }
+
+// A world the generation kernels gave up on: reported (and cleared, with the claim in stream order) by the next
+// d2d_generate_worlds / d2d_read_episode_log.
+static bool take_wg_fault(d2d_handle *h, const char *what, cudaStream_t st) {
+    const unsigned long long fault = h->wg_fault ? h->wg_fault[0] : 0ull;
     if (!fault) return false;
-    *h->wg_fault = 0ull;
-    h->err = std::string(what) + ": the world of seed " + std::to_string((unsigned)(fault & 0xffffffffull)) + " (env " +
-             std::to_string((int)((fault >> 32) & 0x7fffffffull)) + ") could not be built: more than " +
-             std::to_string(D2D_WORLD_MAX_REJECTS) + " rejected draws in a row; that env's world is undefined";
+    const unsigned long long env = h->wg_fault[1];
+    h->wg_fault[0] = 0ull; h->wg_fault[1] = 0ull;
+    cudaMemsetAsync(h->wg_claim, 0, sizeof(unsigned int), st);
+    h->err = std::string(what) + ": the world of seed " + std::to_string((unsigned)(fault & 0xffffffffull)) + " from source " +
+             std::to_string((unsigned)((fault >> 32) & 0x7fffffffull)) + " (env " + std::to_string(env) +
+             ") could not be built: more than " + std::to_string(D2D_WORLD_MAX_REJECTS) +
+             " rejected draws in a row; that env's world is undefined";
     return true;
 }
 
+// Seeds (source 0, [0, 2^32)) or world keys whose source is in the table; false (error set) on the first bad one.
+static bool check_world_keys(d2d_handle *h, const char *what, const int64_t *keys, int64_t count, bool seeds_only) {
+    for (int64_t i = 0; i < count; i++) {
+        const long long k = (long long)keys[i];
+        if (seeds_only && (k < 0 || k > 0xffffffffll)) {
+            h->err = std::string(what) + ": seed " + std::to_string(k) + " outside [0, 2**32)";
+            return false;
+        }
+        if (k < 0 || (k >> 32) >= h->wg_count) {
+            h->err = std::string(what) + ": key " + std::to_string(k) + (k < 0 ? " is negative" : ": source " +
+                     std::to_string(k >> 32) + " outside the table of " + std::to_string(h->wg_count) + " world sources");
+            return false;
+        }
+    }
+    return true;
+}
+
+static int generate_worlds(d2d_handle *h, const int32_t *envs_host, const int64_t *keys_host, int32_t count, int32_t flags,
+                           void *stream, bool seeds_only);
+
 extern "C" int d2d_generate_worlds(d2d_handle *h, const int32_t *envs_host, const int64_t *seeds_host, int32_t count,
                                    int32_t flags, void *stream) {
+    return generate_worlds(h, envs_host, seeds_host, count, flags, stream, true);
+}
+
+extern "C" int d2d_generate_worlds_keyed(d2d_handle *h, const int32_t *envs_host, const int64_t *keys_host, int32_t count,
+                                         int32_t flags, void *stream) {
+    return generate_worlds(h, envs_host, keys_host, count, flags, stream, false);
+}
+
+// seeds_only: d2d_generate_worlds (every key a seed of source 0, checked as such)
+static int generate_worlds(d2d_handle *h, const int32_t *envs_host, const int64_t *keys_host, int32_t count, int32_t flags,
+                           void *stream, bool seeds_only) {
     if (!h) return D2D_ERR_INVALID;
     D2D_NO_PIPE(h);
-    if (!h->wg_tab) { h->err = "d2d_generate_worlds before d2d_set_world_source"; return D2D_ERR_STATE; }
-    if (take_wg_fault(h, "d2d_generate_worlds")) return D2D_ERR_STATE;
+    if (!h->wg_tab) { h->err = "d2d_generate_worlds before d2d_set_world_sources"; return D2D_ERR_STATE; }
+    if (take_wg_fault(h, "d2d_generate_worlds", (cudaStream_t)stream)) return D2D_ERR_STATE;
     if (flags != D2D_WORLD_EAGER && flags != D2D_WORLD_LAZY) {
         h->err = "d2d_generate_worlds: flags must be D2D_WORLD_EAGER or D2D_WORLD_LAZY"; return D2D_ERR_INVALID;
     }
-    if (count < 0 || (count > 0 && (!envs_host || !seeds_host))) { h->err = "d2d_generate_worlds: bad count or null array"; return D2D_ERR_INVALID; }
+    if (count < 0 || (count > 0 && (!envs_host || !keys_host))) { h->err = "d2d_generate_worlds: bad count or null array"; return D2D_ERR_INVALID; }
     int rc = check_env_indices(h, "d2d_generate_worlds", nullptr, envs_host, count);
     if (rc != D2D_OK) return rc;
-    for (int32_t i = 0; i < count; i++)
-        if (seeds_host[i] < 0 || seeds_host[i] > 0xffffffffll) {
-            h->err = "d2d_generate_worlds: seed " + std::to_string((long long)seeds_host[i]) + " outside [0, 2**32)";
-            return D2D_ERR_INVALID;
-        }
+    if (!check_world_keys(h, "d2d_generate_worlds", keys_host, count, seeds_only)) return D2D_ERR_INVALID;
     if (count == 0) return D2D_OK;
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     cudaStream_t st = (cudaStream_t)stream;
     const bool eager = flags == D2D_WORLD_EAGER;
-    // envs, seeds and (eager) the reset mask in one staged copy; the event keeps the next call from overwriting the device
-    // buffer while a kernel still reads it (as launch_clone does)
-    const size_t words = 2 * (size_t)count + (eager ? ((size_t)h->B + 3) / 4 : 0);
+    // envs, keys (8-byte aligned) and (eager) the reset mask in one staged copy; the event keeps the next call from
+    // overwriting the device buffer while a kernel still reads it (as launch_clone does)
+    const size_t ko = (size_t)count + (count & 1), mo = ko + 2 * (size_t)count;
+    const size_t words = mo + (eager ? ((size_t)h->B + 3) / 4 : 0);
     if (!h->wg_ev) CUDA_TRY(h, cudaEventCreateWithFlags(&h->wg_ev, cudaEventDisableTiming));
     if (words * 4 > h->wg_idx_bytes) {
         CUDA_TRY(h, cudaEventSynchronize(h->wg_ev));
@@ -1590,17 +1649,18 @@ extern "C" int d2d_generate_worlds(d2d_handle *h, const int32_t *envs_host, cons
     }
     h->wg_stage.assign(words, 0);
     memcpy(h->wg_stage.data(), envs_host, (size_t)count * 4);
-    for (int32_t i = 0; i < count; i++) h->wg_stage[(size_t)count + i] = (int32_t)(uint32_t)seeds_host[i];
-    uint8_t *mask = (uint8_t *)(h->wg_stage.data() + 2 * (size_t)count);
+    memcpy(h->wg_stage.data() + ko, keys_host, (size_t)count * 8);
+    uint8_t *mask = (uint8_t *)(h->wg_stage.data() + mo);
     if (eager) for (int32_t i = 0; i < count; i++) mask[envs_host[i]] = 1;
     CUDA_TRY(h, cudaStreamWaitEvent(st, h->wg_ev, 0));
     CUDA_TRY(h, cudaMemcpyAsync(h->wg_idx, h->wg_stage.data(), words * 4, cudaMemcpyHostToDevice, st));
     d2d_worldgen_kernel<<<(count + D2D_WG_WARPS - 1) / D2D_WG_WARPS, D2D_WG_WARPS * 32, 0, st>>>(
-        h->P, h->wg_tab, h->wg_idx, (const uint32_t *)(h->wg_idx + count), count, eager ? 0 : 1, h->wg_fault_dev);
+        h->P, h->wg_tab, h->wg_idx, (const long long *)(h->wg_idx + ko), count, eager ? 0 : 1, h->wg_fault_dev,
+        h->wg_claim);
     h->launches++;
     CUDA_TRY(h, cudaGetLastError());
     if (eager) {
-        d2d_reset_kernel<<<h->B, 128, 0, st>>>(h->P, (const uint8_t *)(h->wg_idx + 2 * (size_t)count));
+        d2d_reset_kernel<<<h->B, 128, 0, st>>>(h->P, (const uint8_t *)(h->wg_idx + mo));
         h->launches++;
         CUDA_TRY(h, cudaGetLastError());
         h->mir_stale = true;      // the eager reset rewrites the device observation only
@@ -1627,7 +1687,7 @@ extern "C" int d2d_enable_episode_log(d2d_handle *h, int64_t capacity) {
     const size_t B = (size_t)h->B;
     const size_t o_head = (size_t)capacity * sizeof(d2d_episode_record);
     const size_t o_seed = o_head + 64, o_list = o_seed + (B * 8 + 15) / 16 * 16, o_genv = o_list + (B * 4 + 15) / 16 * 16;
-    const size_t o_gsd = o_genv + (B * 4 + 15) / 16 * 16, bytes = o_gsd + (B * 4 + 15) / 16 * 16;
+    const size_t o_gkey = o_genv + (B * 4 + 15) / 16 * 16, bytes = o_gkey + (B * 8 + 15) / 16 * 16;
     unsigned char *m = nullptr;
     if (cudaMalloc((void **)&m, bytes) != cudaSuccess) {
         cudaGetLastError();
@@ -1642,7 +1702,7 @@ extern "C" int d2d_enable_episode_log(d2d_handle *h, int64_t capacity) {
     if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->cfg.device) != cudaSuccess || sms <= 0) sms = 148;
     h->ep_blocks = (h->B + 31) / 32 < sms ? (h->B + 31) / 32 : sms;
     h->ep.world_seed = (long long *)(m + o_seed); h->ep.list = (int *)(m + o_list);
-    h->ep.gen_env = (int *)(m + o_genv); h->ep.gen_seed = (uint32_t *)(m + o_gsd);
+    h->ep.gen_env = (int *)(m + o_genv); h->ep.gen_key = (long long *)(m + o_gkey);
     h->ep.queue = h->ep_queue;
     return D2D_OK;
 }
@@ -1655,7 +1715,7 @@ extern "C" int d2d_read_episode_log(d2d_handle *h, d2d_episode_record *out_host,
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     cudaStream_t st = (cudaStream_t)stream;
     CUDA_TRY(h, cudaStreamSynchronize(st));
-    if (take_wg_fault(h, "d2d_read_episode_log")) return D2D_ERR_STATE;
+    if (take_wg_fault(h, "d2d_read_episode_log", st)) return D2D_ERR_STATE;
     long long written = 0;
     CUDA_TRY(h, cudaMemcpyAsync(&written, h->ep.head, 8, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(h, cudaStreamSynchronize(st));
@@ -1669,18 +1729,27 @@ extern "C" int d2d_read_episode_log(d2d_handle *h, d2d_episode_record *out_host,
     return D2D_OK;
 }
 
+static int set_world_queue(d2d_handle *h, const char *what, const int64_t *keys_host, int64_t count, void *stream,
+                           bool seeds_only);
+
 extern "C" int d2d_set_seed_queue(d2d_handle *h, const int64_t *seeds_host, int64_t count, void *stream) {
+    return set_world_queue(h, "d2d_set_seed_queue", seeds_host, count, stream, true);
+}
+
+extern "C" int d2d_set_world_queue(d2d_handle *h, const int64_t *keys_host, int64_t count, void *stream) {
+    return set_world_queue(h, "d2d_set_world_queue", keys_host, count, stream, false);
+}
+
+// seeds_only: d2d_set_seed_queue (every key a seed of source 0, checked as such)
+static int set_world_queue(d2d_handle *h, const char *what, const int64_t *keys_host, int64_t count, void *stream,
+                           bool seeds_only) {
     if (!h) return D2D_ERR_INVALID;
     D2D_NO_PIPE(h);
-    if (!h->wg_tab) { h->err = "d2d_set_seed_queue before d2d_set_world_source"; return D2D_ERR_STATE; }
-    if (!h->cfg.auto_reset) { h->err = "d2d_set_seed_queue: the handle was created with auto_reset = 0"; return D2D_ERR_STATE; }
-    if (!h->ep_mem) { h->err = "d2d_set_seed_queue: the episode log is not enabled"; return D2D_ERR_STATE; }
-    if (count < 0 || (count > 0 && !seeds_host)) { h->err = "d2d_set_seed_queue: bad count or null array"; return D2D_ERR_INVALID; }
-    for (int64_t i = 0; i < count; i++)
-        if (seeds_host[i] < 0 || seeds_host[i] > 0xffffffffll) {
-            h->err = "d2d_set_seed_queue: seed " + std::to_string((long long)seeds_host[i]) + " outside [0, 2**32)";
-            return D2D_ERR_INVALID;
-        }
+    if (!h->wg_tab) { h->err = std::string(what) + " before d2d_set_world_sources"; return D2D_ERR_STATE; }
+    if (!h->cfg.auto_reset) { h->err = std::string(what) + ": the handle was created with auto_reset = 0"; return D2D_ERR_STATE; }
+    if (!h->ep_mem) { h->err = std::string(what) + ": the episode log is not enabled"; return D2D_ERR_STATE; }
+    if (count < 0 || (count > 0 && !keys_host)) { h->err = std::string(what) + ": bad count or null array"; return D2D_ERR_INVALID; }
+    if (!check_world_keys(h, what, keys_host, count, seeds_only)) return D2D_ERR_INVALID;
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     cudaStream_t st = (cudaStream_t)stream;
     if (count > h->ep_queue_cap) {                   // grows only: a captured graph keeps a valid queue address
@@ -1688,14 +1757,14 @@ extern "C" int d2d_set_seed_queue(d2d_handle *h, const int64_t *seeds_host, int6
         long long *q = nullptr;
         if (cudaMalloc((void **)&q, (size_t)count * 8) != cudaSuccess) {
             cudaGetLastError();
-            h->err = "d2d_set_seed_queue: cudaMalloc failed"; return D2D_ERR_NOMEM;
+            h->err = std::string(what) + ": cudaMalloc failed"; return D2D_ERR_NOMEM;
         }
         if (h->ep_queue) cudaFree(h->ep_queue);
         h->ep_queue = q; h->ep_queue_cap = count; h->ep.queue = q;
     } else {
-        CUDA_TRY(h, cudaStreamSynchronize(st));      // the last log kernel on this stream has read the old seeds
+        CUDA_TRY(h, cudaStreamSynchronize(st));      // the last log kernel on this stream has read the old keys
     }
-    if (count > 0) CUDA_TRY(h, cudaMemcpyAsync(h->ep_queue, seeds_host, (size_t)count * 8, cudaMemcpyHostToDevice, st));
+    if (count > 0) CUDA_TRY(h, cudaMemcpyAsync(h->ep_queue, keys_host, (size_t)count * 8, cudaMemcpyHostToDevice, st));
     h->ep_qhead[0] = 0; h->ep_qhead[1] = count;
     CUDA_TRY(h, cudaMemcpyAsync(h->ep.head + 2, h->ep_qhead, 16, cudaMemcpyHostToDevice, st));
     CUDA_TRY(h, cudaStreamSynchronize(st));

@@ -158,14 +158,56 @@ def difficulty(params, seeds, T_global=24, T_survivability=12, position_step=60,
       density              float64 [S]          == obstacle_density(params, seeds)
       collision_state      uint8 [S, nx, ny, int(T_global / dt)] == global_survivability(...), with collision_state=True.
     Device worlds equal host worlds except for the documented group-velocity rounding of static-map agents (DESIGN.md
-    section 2)."""
-    params = copy.copy(params)
-    params.planner = "NoMove"           # as both scripts; the worlds and the agents do not depend on the planner
+    section 2).
+    `params` may be a list of K configs (world_gen="device" only): every key then has a leading config axis, [K, S, ...],
+    equal to the per-config calls stacked.  The configs are split into batch groups (experiment.batch_groups of their
+    NoMove scratch configs); each group streams its (config, seed) pairs through one scratch handle with keyed `reseed`
+    chunks.  The configs must share the position grid and dt (the output shapes)."""
     if world_gen not in ("host", "device"):
         raise ValueError("world_gen must be 'host' or 'device', got %r" % (world_gen,))
+    kw = dict(T_global=T_global, T_survivability=T_survivability, position_step=position_step, num_envs=num_envs,
+              collision_state=collision_state, device=device)
+    if not isinstance(params, (list, tuple)):
+        return _difficulty([_scratch(params)], np.asarray(seeds, dtype=np.int64).reshape(-1), world_gen=world_gen, **kw)
+    if world_gen != "device":
+        raise ValueError("difficulty over a list of configs generates the worlds on the device (world_gen='device')")
+    from .experiment import batch_groups
+    from .world import world_key
+    configs = [_scratch(p) for p in params]
+    seeds = np.asarray(seeds, dtype=np.int64).reshape(-1)
+    K, S = len(configs), len(seeds)
+    if K == 0 or S == 0:
+        raise ValueError("difficulty: no configs or no seeds")
+    res = None
+    for group in batch_groups(configs):
+        keys = world_key(np.repeat(np.arange(len(group)), S), np.tile(seeds, len(group)))
+        r = _difficulty([configs[k] for k in group], keys, world_gen="device", **kw)
+        if res is None:
+            res = {n: np.empty((K, S) + v.shape[1:], v.dtype) for n, v in r.items()}
+        for n, v in r.items():
+            if v.shape[1:] != res[n].shape[2:]:
+                raise ValueError("difficulty: configs %s give %s of shape %s, others %s (position grid or dt differ)"
+                                 % (group, n, v.shape[1:], res[n].shape[2:]))
+            res[n][group] = v.reshape((len(group), S) + v.shape[1:])
+    return res
+
+
+def _scratch(p):
+    """The scratch config of the difficulty handle: NoMove, as both scripts; the worlds and the agents do not depend on
+    the planner.  The handle runs no gaze policy, so one gaze value keeps the gaze out of the batch grouping."""
+    p = copy.copy(p)
+    p.planner = "NoMove"
+    p.gaze_method = "LookAhead"
+    return p
+
+
+def _difficulty(configs, seeds, T_global, T_survivability, position_step, num_envs, world_gen, collision_state, device):
+    """difficulty over `seeds` on one scratch handle: world seeds of configs[0] (one config), or world keys over
+    `configs` (one batch group, world_gen="device")."""
+    params = configs[0]
+    keyed = len(configs) > 1            # else the keys of source 0 are the seeds
     xs, ys = survivability_positions(params, position_step)
     nx, ny = len(xs), len(ys)
-    seeds = np.asarray(seeds, dtype=np.int64).reshape(-1)
     S = len(seeds)
     ts = np.arange(0, T_survivability, 0.1)
     steps = max(int(T_global / params.dt), len(ts))
@@ -174,8 +216,14 @@ def difficulty(params, seeds, T_global=24, T_survivability=12, position_step=60,
     if B == 0 or nx * ny == 0:
         raise ValueError("difficulty: no seeds or an empty position grid")
     grid = (xs[0], ys[0], position_step, nx, ny)
-    env = Drone2DVecEnv(params, B, seeds=seeds[:B], device=device, auto_reset=False, trackers=False, oxford=False,
-                        owl=False, world_gen=world_gen)
+    if keyed:
+        from .world import split_world_key
+        src, sd = split_world_key(seeds)
+        env = Drone2DVecEnv(params, B, seeds=sd[:B], device=device, auto_reset=False, trackers=False, oxford=False,
+                            owl=False, world_gen="device", world_sources=configs, sources=src[:B])
+    else:
+        env = Drone2DVecEnv(params, B, seeds=seeds[:B], device=device, auto_reset=False, trackers=False, oxford=False,
+                            owl=False, world_gen=world_gen)
     try:
         dev = env.device
         first_hit = torch.empty((S, nx, ny), dtype=torch.int16, device=dev)
@@ -185,7 +233,9 @@ def difficulty(params, seeds, T_global=24, T_survivability=12, position_step=60,
         for c0 in range(0, S, B):
             n = min(B, S - c0)
             if c0 > 0:
-                if world_gen == "device":
+                if keyed:
+                    env.reseed(np.arange(n), sd[c0:c0 + n], sources=src[c0:c0 + n])
+                elif world_gen == "device":
                     env.reseed(np.arange(n), seeds[c0:c0 + n])
                 else:
                     torch.cuda.current_stream(dev).synchronize()      # the last call has read the snapshot it replaces

@@ -13,7 +13,7 @@ import torch
 
 from . import _native
 from .params import Params
-from .world import count_agents, generate_worlds, load_static_map, world_source
+from .world import count_agents, generate_worlds, load_static_map, world_key, world_source
 
 _TORCH_DTYPES = {0: (torch.uint8, "|u1"), 1: (torch.int8, "|i1"), 2: (torch.int32, "<i4"), 3: (torch.int64, "<i8"),
                  4: (torch.float32, "<f4"), 5: (torch.float64, "<f8")}
@@ -123,6 +123,15 @@ def make_config(params, num_envs, num_agents, device_index, auto_reset=True, tra
     return cfg
 
 
+def config_difference(a, b):
+    """The name of the first d2d_config field in which `a` and `b` differ (compared byte for byte), or None."""
+    for f in _native.D2DConfig._fields_:
+        d = getattr(_native.D2DConfig, f[0])
+        if C.string_at(C.addressof(a) + d.offset, d.size) != C.string_at(C.addressof(b) + d.offset, d.size):
+            return f[0]
+    return None
+
+
 class Drone2DVecEnv(object):
     """Batched `Drone2DEnv2`.
 
@@ -135,16 +144,24 @@ class Drone2DVecEnv(object):
     world_gen : "host" (default) builds the worlds with world.generate_worlds and uploads them; "device" generates them
                 on the GPU (d2d_generate_worlds), identical except for the documented group-velocity rounding (DESIGN.md
                 section 2).  `reseed` needs neither.  Cannot be combined with `worlds`.
+    world_sources, sources : world_gen="device" only: the handle's table of world sources (`set_world_sources`, a list of
+                Params that share this handle's config) and the source of each env's initial world (default 0), so the
+                initial worlds can come from many configurations; `seeds` then holds world keys (world.world_key).
     """
 
     metadata = {"render.modes": ["rgb_array"]}
 
     def __init__(self, params, num_envs, seeds=None, device="cuda:0", auto_reset=True, trackers=True, oxford=None,
-                 envs_per_block=0, strip_width=10, worlds=None, owl=None, jerk_tie_orders=None, world_gen="host"):
+                 envs_per_block=0, strip_width=10, worlds=None, owl=None, jerk_tie_orders=None, world_gen="host",
+                 world_sources=None, sources=None):
         if world_gen not in ("host", "device"):
             raise ValueError("world_gen must be 'host' or 'device', got %r" % (world_gen,))
         if world_gen == "device" and worlds is not None:
             raise ValueError("world_gen='device' generates the worlds itself: do not pass `worlds`")
+        if world_gen != "device" and (world_sources is not None or sources is not None):
+            raise ValueError("world_sources / sources need world_gen='device'")
+        if sources is not None and world_sources is None:
+            raise ValueError("sources index a table of world sources: pass world_sources too")
         if not torch.cuda.is_available():
             raise _native.Drone2DNativeError("CUDA device required: Drone2DVecEnv has no CPU path")
         self.params = params
@@ -158,9 +175,9 @@ class Drone2DVecEnv(object):
             oxford = getattr(params, "gaze_method", "") == "Oxford"
         if owl is None:
             owl = getattr(params, "gaze_method", "") == "Owl"
-        self.cfg = make_config(params, self.num_envs, self.num_agents, self._dev_index, auto_reset=auto_reset,
-                               trackers=trackers, oxford=oxford, envs_per_block=envs_per_block,
-                               strip_width=strip_width, owl=owl)
+        self._cfg_kw = dict(auto_reset=auto_reset, trackers=trackers, oxford=oxford, envs_per_block=envs_per_block,
+                            strip_width=strip_width, owl=owl)
+        self.cfg = make_config(params, self.num_envs, self.num_agents, self._dev_index, **self._cfg_kw)
         self._h = C.c_void_p()
         rc = self._lib.d2d_create(C.byref(self.cfg), C.byref(self._h))
         if rc != 0:
@@ -172,10 +189,12 @@ class Drone2DVecEnv(object):
             self._check(self._lib.d2d_set_jerk_tables(self._h, C.byref(self._jerk_tables)), "d2d_set_jerk_tables")
         # a copy: reseed / clone_envs / load_state rewrite entries, and must not write into the caller's array
         self.seeds = np.array(seeds if seeds is not None else params.map_id + np.arange(self.num_envs), dtype=np.int64)
-        self._world_source = None
+        self._world_sources = None
         self._log_capacity, self._queue_set = 0, False
         if world_gen == "device":
-            self.reseed(np.arange(self.num_envs), self.seeds)
+            if world_sources is not None:
+                self.set_world_sources(world_sources)
+            self.reseed(np.arange(self.num_envs), self.seeds, sources=sources)
             torch.cuda.current_stream(self.device).synchronize()
             self.check_worlds()
         else:
@@ -223,33 +242,72 @@ class Drone2DVecEnv(object):
                   p(w["rng_gauss"], np.float64)]
             self._check(self._lib.d2d_set_rng(self._h, first_env, count, *[k[1] for k in rk]), "d2d_set_rng")
 
-    def reseed(self, envs, seeds, lazy=False):
+    def set_world_sources(self, configs):
+        """The handle's table of world sources (d2d_set_world_sources): `configs[k]` (a Params) is source k of the world
+        keys `reseed(..., sources=)` and `set_seed_queue(..., sources=)` take.  Every config must give this handle's
+        d2d_config field for field (make_config: agent_radius, num_agents, drone and planner parameters, targets, view
+        range, ...); they may differ in what only shapes the world -- the static map, agent_number within the same agent
+        count, pillar_number, agent_max_speed, init_pos.  ValueError names the first field that differs.  Replaces the
+        table; until the first call the handle's own params are source 0."""
+        configs = list(configs)
+        if not 1 <= len(configs) <= _native.WORLD_MAX_SOURCES:
+            raise ValueError("set_world_sources: %d configs (1..%d)" % (len(configs), _native.WORLD_MAX_SOURCES))
+        srcs = (_native.D2DWorldSource * len(configs))()
+        for k, p in enumerate(configs):
+            smap = load_static_map(p.static_map)
+            field = config_difference(self.cfg, make_config(p, self.num_envs, count_agents(p, smap), self._dev_index,
+                                                            **self._cfg_kw))
+            if field is not None:
+                raise ValueError("set_world_sources: config %d differs from the handle's config in %r" % (k, field))
+            srcs[k] = world_source(p, smap)
+        self._upload_sources(configs, srcs)
+
+    def _upload_sources(self, configs, srcs):
+        self._check(self._lib.d2d_set_world_sources(self._h, srcs, len(configs)), "d2d_set_world_sources")
+        self._world_sources = list(configs)
+
+    def _default_sources(self):
+        """The handle's own params as source 0, as the handle was created (no config comparison)."""
+        if self._world_sources is None:
+            self._upload_sources([self.params], (_native.D2DWorldSource * 1)(world_source(self.params, self._smap)))
+
+    def _keys(self, what, seeds, sources, n):
+        """`seeds` (sources=None: seeds or keys as given) or world_key(sources, seeds) as a contiguous int64 array of n."""
+        sd = np.asarray(seeds).reshape(-1)
+        if sd.size and sd.dtype.kind not in "iu":
+            raise ValueError("seeds must be integers, got %s" % sd.dtype)
+        if sources is not None:
+            src = np.asarray(sources).reshape(-1)
+            if src.size != sd.size:
+                raise ValueError("%s: %d sources for %d seeds" % (what, src.size, sd.size))
+            sd = world_key(src, sd)
+        sd = np.ascontiguousarray(sd, dtype=np.int64)
+        if n is not None and sd.size != n:
+            raise ValueError("%s: %d seeds for %d envs" % (what, sd.size, n))
+        return sd
+
+    def reseed(self, envs, seeds, lazy=False, sources=None):
         """Gives envs[i] the world of seeds[i], generated on the GPU (d2d_generate_worlds, one launch, asynchronous):
         lazy=False resets those envs now, as `reset` does; lazy=True marks them, and each starts its new world at its next
         step -- the path auto-reset takes after done, so the terminal outputs of an env that just reported done stay
         readable until then.  Afterwards `seeds[e]` is the seed of the world env e resets into.  Seeds must lie in
-        [0, 2**32), as np.random.RandomState requires.  A seed whose world cannot be built is reported by the next call or
-        by `check_worlds`."""
+        [0, 2**32), as np.random.RandomState requires.  With `sources` (indices into the table of `set_world_sources`) env
+        envs[i] gets the world of seed seeds[i] built from source sources[i] (d2d_generate_worlds_keyed), and `seeds[e]`
+        holds its world key.  A seed whose world cannot be built is reported by the next call or by `check_worlds`."""
         idx = self._env_indices(envs)
-        sd = np.asarray(seeds).reshape(-1)
-        if sd.size and sd.dtype.kind not in "iu":
-            raise ValueError("seeds must be integers, got %s" % sd.dtype)
-        sd = np.ascontiguousarray(sd, dtype=np.int64)
-        if sd.size != idx.size:
-            raise ValueError("reseed: %d seeds for %d envs" % (sd.size, idx.size))
-        if self._world_source is None:
-            src = world_source(self.params, self._smap)
-            self._check(self._lib.d2d_set_world_source(self._h, C.byref(src)), "d2d_set_world_source")
-            self._world_source = src
+        sd = self._keys("reseed", seeds, sources, idx.size)
+        self._default_sources()
         flags = _native.WORLD_LAZY if lazy else _native.WORLD_EAGER
-        self._check(self._lib.d2d_generate_worlds(self._h, idx.ctypes.data_as(C.c_void_p), sd.ctypes.data_as(C.c_void_p),
-                                                  int(idx.size), flags, self._stream()), "d2d_generate_worlds")
+        fn, name = ((self._lib.d2d_generate_worlds, "d2d_generate_worlds") if sources is None else
+                    (self._lib.d2d_generate_worlds_keyed, "d2d_generate_worlds_keyed"))
+        self._check(fn(self._h, idx.ctypes.data_as(C.c_void_p), sd.ctypes.data_as(C.c_void_p), int(idx.size), flags,
+                       self._stream()), name)
         self.seeds[idx] = sd
         self._set_world_seeds(idx, sd)
 
     def check_worlds(self):
         """Raises if an earlier `reseed` met a seed whose world cannot be built (call after synchronising the stream)."""
-        if self._world_source is not None:
+        if self._world_sources is not None:
             self._check(self._lib.d2d_generate_worlds(self._h, None, None, 0, _native.WORLD_EAGER, self._stream()),
                         "d2d_generate_worlds")
 
@@ -526,21 +584,19 @@ class Drone2DVecEnv(object):
             self.seeds[:] = self.buffer("world_seed").cpu().numpy()
         return self._log_out[:n.value].copy(), int(dropped.value)
 
-    def set_seed_queue(self, seeds):
+    def set_seed_queue(self, seeds, sources=None):
         """Seeds for the envs that finish from now on (d2d_set_seed_queue): in every step each env that reports done takes
         the next one (ascending env order) and starts that world, generated on the device, at its next step; its record
         carries the seed of the world it finished.  When the queue runs out, envs replay their last world.  Needs the episode
-        log and auto-reset; the world source is set up here.  An empty sequence clears the queue."""
-        sd = np.asarray(seeds).reshape(-1)
-        if sd.size and sd.dtype.kind not in "iu":
-            raise ValueError("seeds must be integers, got %s" % sd.dtype)
-        sd = np.ascontiguousarray(sd, dtype=np.int64)
-        if self._world_source is None and self._log_capacity and self.cfg.auto_reset:
-            src = world_source(self.params, self._smap)
-            self._check(self._lib.d2d_set_world_source(self._h, C.byref(src)), "d2d_set_world_source")
-            self._world_source = src
-        self._check(self._lib.d2d_set_seed_queue(self._h, sd.ctypes.data_as(C.c_void_p), int(sd.size), self._stream()),
-                    "d2d_set_seed_queue")
+        log and auto-reset; the world source is set up here.  With `sources` the queue holds the world keys
+        world_key(sources, seeds) (d2d_set_world_queue), and the records and `seeds` carry keys.  An empty sequence clears
+        the queue."""
+        sd = self._keys("set_seed_queue", seeds, sources, None)
+        if self._log_capacity and self.cfg.auto_reset:
+            self._default_sources()
+        fn, name = ((self._lib.d2d_set_seed_queue, "d2d_set_seed_queue") if sources is None else
+                    (self._lib.d2d_set_world_queue, "d2d_set_world_queue"))
+        self._check(fn(self._h, sd.ctypes.data_as(C.c_void_p), int(sd.size), self._stream()), name)
         self._queue_set = sd.size > 0
 
     def plan_oxford(self, out=None):

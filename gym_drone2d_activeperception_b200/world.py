@@ -183,6 +183,32 @@ def world_source(params, static_map=None):
     return s
 
 
+def world_key(sources, seeds):
+    """World keys `source * 2**32 + seed` (int64 array, broadcast) for d2d_generate_worlds_keyed and the keyed seed queue:
+    `source` indexes the handle's table of world sources (`Drone2DVecEnv.set_world_sources`), [0, WORLD_MAX_SOURCES), and
+    `seed` is the reference's map_id, [0, 2**32).  With source 0 the key is the seed."""
+    from ._native import WORLD_MAX_SOURCES
+    src, sd = np.asarray(sources), np.asarray(seeds)
+    for name, a, hi in (("sources", src, WORLD_MAX_SOURCES), ("seeds", sd, 2 ** 32)):
+        if a.size and a.dtype.kind not in "iu":
+            raise ValueError("world_key: %s must be integers, got %s" % (name, a.dtype))
+        if a.size and (a.min() < 0 or a.max() >= hi):
+            raise ValueError("world_key: %s outside [0, %d)" % (name, hi))
+    return (src.astype(np.int64) << np.int64(32)) | sd.astype(np.int64)
+
+
+def split_world_key(keys):
+    """(sources, seeds) of world keys, both int64 arrays; the inverse of world_key."""
+    from ._native import WORLD_MAX_SOURCES
+    k = np.asarray(keys)
+    if k.size and k.dtype.kind not in "iu":
+        raise ValueError("split_world_key: keys must be integers, got %s" % k.dtype)
+    k = k.astype(np.int64)
+    if k.size and (k.min() < 0 or k.max() >= np.int64(WORLD_MAX_SOURCES) << np.int64(32)):
+        raise ValueError("split_world_key: keys outside [0, %d * 2**32)" % WORLD_MAX_SOURCES)
+    return k >> np.int64(32), k & np.int64(0xFFFFFFFF)
+
+
 def _initial_velocities(agent_pref, agent_number):
     """Agent.velocity right after __init__: `(0., 0.)` for the random agents (drone_v2.py:19), the group velocity for the
     map-cell agents (drone_v2.py:62).  Only read under the RVO motion profile (CVM overwrites it with pref_velocity)."""

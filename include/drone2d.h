@@ -355,8 +355,22 @@ typedef struct d2d_world_source {
     uint8_t static_map[50][50];
 } d2d_world_source;
 
-/* Stores the seed-independent inputs (HOST struct, copied).  Once per handle.  Checked against the config: the map must be
- * the config's, agent_number + the non-zero cells of static_map == num_agents, and under RVO pillar_number <= 16. */
+/* World keys: a world is named by key = source * 2^32 + seed, `source` an index into the handle's table of world sources
+ * (d2d_set_world_sources) and `seed` in [0, 2^32).  With source 0 the key is the seed, so a handle with one source sees
+ * seeds everywhere a key is stored ("world_seed", d2d_episode_record.seed). */
+#define D2D_WORLD_MAX_SOURCES 4096
+
+/* Stores the table of world sources srcs[0, count) (HOST structs, copied), 1 <= count <= D2D_WORLD_MAX_SOURCES; a later
+ * call replaces the table.  Every source is checked against the config: the map size, drone_radius and agent_radius must
+ * be the config's, agent_number + the non-zero cells of static_map == num_agents, and under RVO pillar_number <= 16.  All
+ * or nothing: a rejected call changes nothing and names the index of the first bad source.  The device table grows only:
+ * a call with more sources than any earlier one reallocates it and synchronises the device first, so a CUDA graph captured
+ * before (its generation kernels hold the table's address) must be captured again; a call that fits also synchronises the
+ * device (no d2d_generate_worlds kernel and no seed-queue generation behind a logged step may still read the table) and
+ * overwrites the table in place.  Keys queued before (d2d_set_world_queue) are not re-checked. */
+int d2d_set_world_sources(d2d_handle *h, const d2d_world_source *srcs, int32_t count);
+
+/* d2d_set_world_sources(h, src, 1). */
 int d2d_set_world_source(d2d_handle *h, const d2d_world_source *src);
 
 /* Generates the worlds of seeds_host[i] into envs envs_host[i] (HOST arrays, i < count) in ONE launch on `stream`,
@@ -371,16 +385,22 @@ int d2d_set_world_source(d2d_handle *h, const d2d_world_source *src);
  * d2d_set_world_source and while a pipelined step is in flight.  Statistics are untouched; the first call counts as
  * d2d_set_world (+ d2d_set_rng / d2d_set_rvo).
  * A seed whose world cannot be built (the reference's rejection loops would never end: more than 65536 rejected draws in a
- * row) is recorded by the kernel; the NEXT call reports it with D2D_ERR_STATE (env and seed in d2d_last_error), clears it
- * and does nothing else.  count = 0 enqueues nothing: after synchronising the stream it reports such a failure at once. */
+ * row) is recorded by the kernel; the NEXT call reports it with D2D_ERR_STATE (env, seed and source in d2d_last_error),
+ * clears it and does nothing else.  count = 0 enqueues nothing: after synchronising the stream it reports such a failure at once. */
 int d2d_generate_worlds(d2d_handle *h, const int32_t *envs_host, const int64_t *seeds_host, int32_t count, int32_t flags,
                         void *stream);
+
+/* d2d_generate_worlds with world keys: envs_host[i] gets the world of seed keys_host[i] & 0xffffffff built from source
+ * keys_host[i] >> 32.  A negative key, or one whose source is not in the table, is rejected before anything is enqueued.
+ * A world that cannot be built is reported as above, with its env, seed and source. */
+int d2d_generate_worlds_keyed(d2d_handle *h, const int32_t *envs_host, const int64_t *keys_host, int32_t count, int32_t flags,
+                              void *stream);
 
 /* Episode log: one fixed-size record per (step, env) that reported done -- everything the reference's experiment row
  * (experiment.py:69-101) needs, written on the device by the step that finished the episode, so a driver can step many
  * times between host synchronisations.  The events are exactly those D2D_STAT_EPISODES counts. */
 typedef struct d2d_episode_record {   /* 48 bytes */
-    int64_t seed;                /* "world_seed"[env] at the step that reported done */
+    int64_t seed;                /* "world_seed"[env] at the step that reported done: the world key (the seed for source 0) */
     int64_t step;                /* index of that step among the steps logged since the log was enabled */
     int64_t tracked_steps;       /* "tracker_buffer_ts" */
     int32_t env;
@@ -396,9 +416,9 @@ typedef struct d2d_episode_record {   /* 48 bytes */
  * DEVICE buffers (d2d_get_buffer; D2D_ERR_STATE while the log is disabled):
  *   "episode_log"       [capacity][48] u8 records
  *   "episode_log_head"  int64[4]: records written since the last read, steps logged, seeds handed out by the queue, queue length
- *   "world_seed"        int64 [num_envs], zero when enabled: the seed of each env's world.  The caller writes it with ordinary
- *                       device writes; the library writes it only from the seed queue.  Not env state: clone / save / load
- *                       and the state layout ignore it.
+ *   "world_seed"        int64 [num_envs], zero when enabled: the key of each env's world (its seed for source 0).  The
+ *                       caller writes it with ordinary device writes; the library writes it only from the seed queue.
+ *                       Not env state: clone / save / load and the state layout ignore it.
  * While the log is enabled every step entry point (d2d_step, d2d_step_plan_oxford after its side stream has joined,
  * d2d_step_host, d2d_step_bound, d2d_step_bound_plan_oxford) enqueues one more kernel behind the step: it appends a record
  * for every env whose "done" is non-zero, in ascending env order, so the log is in (step, env) order.  The step counter
@@ -411,7 +431,7 @@ int d2d_enable_episode_log(d2d_handle *h, int64_t capacity);
 /* Synchronises `stream`, copies the records written since the last read to out_host (HOST, room for `capacity` records),
  * their number to *count and the number of records the full log could not take to *dropped, then resets the written
  * count (in stream order).  D2D_ERR_STATE when the log is disabled, or when a world of the seed queue could not be built
- * (env and seed in d2d_last_error; the failure is cleared, the records stay for the next read). */
+ * (env, seed and source in d2d_last_error; the failure is cleared, the records stay for the next read). */
 int d2d_read_episode_log(d2d_handle *h, d2d_episode_record *out_host, int64_t *count, int64_t *dropped, void *stream);
 
 /* Seed queue: from the next logged step on, every env that reports done takes the next seed of the queue (ascending env
@@ -424,6 +444,10 @@ int d2d_read_episode_log(d2d_handle *h, d2d_episode_record *out_host, int64_t *c
  * the queue.  D2D_ERR_STATE without d2d_set_world_source, without cfg.auto_reset or without an enabled log.  A rejected
  * call changes nothing. */
 int d2d_set_seed_queue(d2d_handle *h, const int64_t *seeds_host, int64_t count, void *stream);
+
+/* The seed queue with world keys (d2d_generate_worlds_keyed): keys_host HOST int64 [count], each naming a source of the
+ * current table; "world_seed" and the records carry the keys.  The same contract as d2d_set_seed_queue otherwise. */
+int d2d_set_world_queue(d2d_handle *h, const int64_t *keys_host, int64_t count, void *stream);
 
 /* Rendering: replaces Drone2DEnv2.render (drone_v2.py:263-303, utils.py:31-64, 550-558, 786-817) with rgb_array frames drawn
  * on the device instead of a pygame window.  Frame of one env: uint8 [H][W][3] RGB, C-contiguous, H = W = 50 * ppc
