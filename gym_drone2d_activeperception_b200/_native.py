@@ -108,7 +108,7 @@ EXPORTS = ["d2d_version", "d2d_last_error", "d2d_create", "d2d_destroy", "d2d_se
            "d2d_launch_count", "d2d_clone_envs", "d2d_state_layout", "d2d_save_state", "d2d_load_state",
            "d2d_set_world_source", "d2d_generate_worlds", "d2d_enable_episode_log", "d2d_read_episode_log",
            "d2d_set_seed_queue", "d2d_render", "d2d_difficulty", "d2d_set_world_sources", "d2d_generate_worlds_keyed",
-           "d2d_set_world_queue"]
+           "d2d_set_world_queue", "d2d_grid_hits"]
 
 _lib = None
 
@@ -169,6 +169,7 @@ def load():
     L.d2d_set_world_queue.argtypes = [vp, vp, C.c_int64, vp]
     L.d2d_render.argtypes = [vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, vp, vp]
     L.d2d_difficulty.argtypes = [vp, C.POINTER(D2DDifficultySpec), C.c_int32, C.c_int32, vp, vp, vp, vp]
+    L.d2d_grid_hits.argtypes = [vp, C.POINTER(D2DDifficultySpec), C.c_int32, C.c_int32, C.c_int32, vp, vp, vp, vp]
     for name in EXPORTS:
         if name not in ("d2d_version", "d2d_last_error", "d2d_launch_count"):
             getattr(L, name).restype = C.c_int

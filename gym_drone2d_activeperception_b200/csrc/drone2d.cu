@@ -1823,13 +1823,70 @@ extern "C" int d2d_render(d2d_handle *h, const int32_t *envs_host, int32_t first
 }
 
 // ------------------------------------------------------------------------------------------ difficulty metrics
-static int check_dev_out(d2d_handle *h, const char *what, const void *p) {
+static int check_dev_out(d2d_handle *h, const char *fn, const char *what, const void *p) {
     cudaPointerAttributes at;
     if (cudaPointerGetAttributes(&at, p) != cudaSuccess || at.type != cudaMemoryTypeDevice || at.device != h->cfg.device) {
         cudaGetLastError();
-        h->err = std::string("d2d_difficulty: ") + what + " is not device memory of device " + std::to_string(h->cfg.device);
+        h->err = std::string(fn) + ": " + what + " is not device memory of device " + std::to_string(h->cfg.device);
         return D2D_ERR_INVALID;
     }
+    return D2D_OK;
+}
+
+// The checks d2d_difficulty and d2d_grid_hits share: the spec, the env range and, for count > 0, the outputs (non-null
+// device memory of the handle's device).  Error texts start with `fn`.  On D2D_OK the caller fills `o`.
+static int check_difficulty_call(d2d_handle *h, const char *fn, const d2d_difficulty_spec *spec, int32_t first_env,
+                                 int32_t count, int16_t *first_hit, uint8_t *static_hit, uint8_t *collision_state,
+                                 DiffOut *o) {
+    const std::string f = std::string(fn) + ": ";
+    if (!spec) { h->err = f + "null spec"; return D2D_ERR_INVALID; }
+    const d2d_difficulty_spec &S = *spec;
+    if (S.struct_size != (int32_t)sizeof(d2d_difficulty_spec)) { h->err = f + "d2d_difficulty_spec size mismatch (ABI)"; return D2D_ERR_INVALID; }
+    if (S.nx < 1 || S.ny < 1 || (int64_t)S.nx * S.ny > D2D_DIFF_MAX_POS) {
+        h->err = f + "a " + std::to_string(S.nx) + " x " + std::to_string(S.ny) + " grid (1 to " +
+                 std::to_string(D2D_DIFF_MAX_POS) + " positions)";
+        return D2D_ERR_INVALID;
+    }
+    if (!std::isfinite(S.x0) || !std::isfinite(S.y0) || !std::isfinite(S.step) || !(S.step > 0.0)) {
+        h->err = f + "x0, y0 and step must be finite and step > 0"; return D2D_ERR_INVALID;
+    }
+    if (S.steps < 1 || S.steps > D2D_DIFF_MAX_STEPS) {
+        h->err = f + "steps " + std::to_string(S.steps) + " outside 1.." + std::to_string(D2D_DIFF_MAX_STEPS);
+        return D2D_ERR_INVALID;
+    }
+    if (S.n_slots < 0 || S.n_slots > D2D_DIFF_MAX_STEPS) {
+        h->err = f + "n_slots " + std::to_string(S.n_slots) + " outside 0.." + std::to_string(D2D_DIFF_MAX_STEPS);
+        return D2D_ERR_INVALID;
+    }
+    if ((collision_state == nullptr) != (S.n_slots == 0)) {
+        h->err = f + "collision_state must be given exactly when n_slots > 0"; return D2D_ERR_INVALID;
+    }
+    if (S.n_slots > 0)
+        for (int k = 0; k < S.steps; k++) {
+            const int s = S.slot[k];
+            if ((s >= S.n_slots && s != D2D_DIFF_NO_SLOT) || (k > 0 && s < S.slot[k - 1])) {
+                h->err = f + "slot[" + std::to_string(k) + "] = " + std::to_string(s) +
+                         ": the slot table must be non-decreasing with entries < n_slots or D2D_DIFF_NO_SLOT";
+                return D2D_ERR_INVALID;
+            }
+        }
+    if (count < 0 || first_env < 0 || first_env > h->B || count > h->B - first_env) {
+        h->err = f + "envs [" + std::to_string(first_env) + ", " + std::to_string((long long)first_env + count) +
+                 ") outside [0, " + std::to_string(h->B) + ")";
+        return D2D_ERR_INVALID;
+    }
+    if (count > 0) {
+        if (!first_hit || !static_hit) { h->err = f + "null output"; return D2D_ERR_INVALID; }
+        CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+        int rc;
+        if ((rc = check_dev_out(h, fn, "first_hit", first_hit)) != D2D_OK) return rc;
+        if ((rc = check_dev_out(h, fn, "static_hit", static_hit)) != D2D_OK) return rc;
+        if (collision_state && (rc = check_dev_out(h, fn, "collision_state", collision_state)) != D2D_OK) return rc;
+    }
+    o->first_hit = first_hit; o->static_hit = static_hit; o->cs = collision_state;
+    o->first_env = first_env; o->count = count;
+    o->nchunks = (S.nx * S.ny + 63) / 64;
+    o->nwords = (S.n_slots + 31) / 32;
     return D2D_OK;
 }
 
@@ -1843,58 +1900,37 @@ extern "C" int d2d_difficulty(d2d_handle *h, const d2d_difficulty_spec *spec, in
                  "envs (metrics.global_survivability / metrics.survivability)";
         return D2D_ERR_STATE;
     }
-    if (!spec) { h->err = "d2d_difficulty: null spec"; return D2D_ERR_INVALID; }
-    const d2d_difficulty_spec &S = *spec;
-    if (S.struct_size != (int32_t)sizeof(d2d_difficulty_spec)) { h->err = "d2d_difficulty: d2d_difficulty_spec size mismatch (ABI)"; return D2D_ERR_INVALID; }
-    if (S.nx < 1 || S.ny < 1 || (int64_t)S.nx * S.ny > D2D_DIFF_MAX_POS) {
-        h->err = "d2d_difficulty: a " + std::to_string(S.nx) + " x " + std::to_string(S.ny) + " grid (1 to " +
-                 std::to_string(D2D_DIFF_MAX_POS) + " positions)";
-        return D2D_ERR_INVALID;
-    }
-    if (!std::isfinite(S.x0) || !std::isfinite(S.y0) || !std::isfinite(S.step) || !(S.step > 0.0)) {
-        h->err = "d2d_difficulty: x0, y0 and step must be finite and step > 0"; return D2D_ERR_INVALID;
-    }
-    if (S.steps < 1 || S.steps > D2D_DIFF_MAX_STEPS) {
-        h->err = "d2d_difficulty: steps " + std::to_string(S.steps) + " outside 1.." + std::to_string(D2D_DIFF_MAX_STEPS);
-        return D2D_ERR_INVALID;
-    }
-    if (S.n_slots < 0 || S.n_slots > D2D_DIFF_MAX_STEPS) {
-        h->err = "d2d_difficulty: n_slots " + std::to_string(S.n_slots) + " outside 0.." + std::to_string(D2D_DIFF_MAX_STEPS);
-        return D2D_ERR_INVALID;
-    }
-    if ((collision_state == nullptr) != (S.n_slots == 0)) {
-        h->err = "d2d_difficulty: collision_state must be given exactly when n_slots > 0"; return D2D_ERR_INVALID;
-    }
-    if (S.n_slots > 0)
-        for (int k = 0; k < S.steps; k++) {
-            const int s = S.slot[k];
-            if ((s >= S.n_slots && s != D2D_DIFF_NO_SLOT) || (k > 0 && s < S.slot[k - 1])) {
-                h->err = "d2d_difficulty: slot[" + std::to_string(k) + "] = " + std::to_string(s) +
-                         ": the slot table must be non-decreasing with entries < n_slots or D2D_DIFF_NO_SLOT";
-                return D2D_ERR_INVALID;
-            }
-        }
-    if (count < 0 || first_env < 0 || first_env > h->B || count > h->B - first_env) {
-        h->err = "d2d_difficulty: envs [" + std::to_string(first_env) + ", " + std::to_string((long long)first_env + count) +
-                 ") outside [0, " + std::to_string(h->B) + ")";
-        return D2D_ERR_INVALID;
-    }
-    if (count == 0) return D2D_OK;
-    if (!first_hit || !static_hit) { h->err = "d2d_difficulty: null output"; return D2D_ERR_INVALID; }
-    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    int rc;
-    if ((rc = check_dev_out(h, "first_hit", first_hit)) != D2D_OK) return rc;
-    if ((rc = check_dev_out(h, "static_hit", static_hit)) != D2D_OK) return rc;
-    if (collision_state && (rc = check_dev_out(h, "collision_state", collision_state)) != D2D_OK) return rc;
     DiffOut o;
-    o.first_hit = first_hit; o.static_hit = static_hit; o.cs = collision_state;
-    o.first_env = first_env; o.count = count;
-    o.nchunks = (S.nx * S.ny + 63) / 64;
-    o.nwords = (S.n_slots + 31) / 32;
+    const int rc = check_difficulty_call(h, "d2d_difficulty", spec, first_env, count, first_hit, static_hit,
+                                         collision_state, &o);
+    if (rc != D2D_OK || count == 0) return rc;
+    const d2d_difficulty_spec &S = *spec;
     const long long tasks = (long long)count * o.nchunks;
     const size_t smem = (size_t)D2D_DIFF_WARPS * 64 * o.nwords * 4;
     d2d_difficulty_kernel<<<(unsigned)((tasks + D2D_DIFF_WARPS - 1) / D2D_DIFF_WARPS), D2D_DIFF_WARPS * 32, smem,
                             (cudaStream_t)stream>>>(h->P, o, S);
+    h->launches++;
+    CUDA_TRY(h, cudaGetLastError());
+    return D2D_OK;
+}
+
+extern "C" int d2d_grid_hits(d2d_handle *h, const d2d_difficulty_spec *spec, int32_t t, int32_t first_env, int32_t count,
+                             int16_t *first_hit, uint8_t *static_hit, uint8_t *collision_state, void *stream) {
+    if (!h) return D2D_ERR_INVALID;
+    D2D_NO_PIPE(h);
+    if (!h->world_set) { h->err = "d2d_grid_hits before d2d_set_world"; return D2D_ERR_STATE; }
+    DiffOut o;
+    const int rc = check_difficulty_call(h, "d2d_grid_hits", spec, first_env, count, first_hit, static_hit,
+                                         collision_state, &o);
+    if (rc != D2D_OK) return rc;
+    if (t < 1 || t > spec->steps) {
+        h->err = "d2d_grid_hits: step " + std::to_string(t) + " outside 1.." + std::to_string(spec->steps);
+        return D2D_ERR_INVALID;
+    }
+    if (count == 0) return D2D_OK;
+    const long long tasks = (long long)count * o.nchunks;
+    d2d_grid_hits_kernel<<<(unsigned)((tasks + D2D_DIFF_WARPS - 1) / D2D_DIFF_WARPS), D2D_DIFF_WARPS * 32, 0,
+                           (cudaStream_t)stream>>>(h->P, o, *spec, t);
     h->launches++;
     CUDA_TRY(h, cudaGetLastError());
     return D2D_OK;

@@ -144,13 +144,16 @@ def survival_from_hits(first_hit, static_hit, T_survivability, n_slots, table):
 
 def difficulty(params, seeds, T_global=24, T_survivability=12, position_step=60, num_envs=65536, world_gen="device",
                collision_state=False, device="cuda:0"):
-    """`survivability`, `global_survivability` (as `mean_survival_time`) and `obstacle_density` of every seed from ONE
-    kernel per chunk of seeds (d2d_difficulty): the agents are stepped alone from each world's reset state and every grid
-    position is tested after every step, the way both scripts test it.  Under CVM no agent looks at the drone, so one agent
-    trajectory per world answers all positions.  The seeds stream through one scratch handle of min(num_envs, len(seeds))
-    NoMove envs; each chunk is an eager `reseed` (world_gen="device") or `set_worlds` (world_gen="host") and one
-    `difficulty` call into preallocated device outputs, with one synchronisation at the end.  Any planner (the scratch
-    handle is NoMove, as in the scripts); CVM only (RVO: use the functions above).
+    """`survivability`, `global_survivability` (as `mean_survival_time`) and `obstacle_density` of every seed, with every
+    grid position tested after every agent step, the way both scripts test it.  No agent looks at the drone (under CVM
+    nor RVO), so one agent trajectory per world answers all positions.  The seeds stream through one scratch handle of
+    min(num_envs, len(seeds)) NoMove envs; each chunk is an eager `reseed` (world_gen="device") or `set_worlds`
+    (world_gen="host"), then, by the motion profile of the config:
+      CVM  one `difficulty` call (d2d_difficulty: the agents are stepped alone from each world's reset state);
+      RVO  `steps` iterations of `step` + `grid_hits(t, ...)` (the step kernels move the agents, d2d_grid_hits tests the
+           grid), eager for the first chunk and replayed from a CUDA graph captured once per chunk size afterwards;
+    into preallocated device outputs, with one synchronisation at the end.  Any planner (the scratch handle is NoMove, as
+    in the scripts).
     Returns a dict of numpy arrays, S = len(seeds):
       survivability        float64 [S, nx, ny]  == survivability(params, seeds, T_survivability, position_step)[0]
       mean_survivability   float64 [S]          == its second output
@@ -161,8 +164,9 @@ def difficulty(params, seeds, T_global=24, T_survivability=12, position_step=60,
     section 2).
     `params` may be a list of K configs (world_gen="device" only): every key then has a leading config axis, [K, S, ...],
     equal to the per-config calls stacked.  The configs are split into batch groups (experiment.batch_groups of their
-    NoMove scratch configs); each group streams its (config, seed) pairs through one scratch handle with keyed `reseed`
-    chunks.  The configs must share the position grid and dt (the output shapes)."""
+    NoMove scratch configs; CVM and RVO configs never share one); each group streams its (config, seed) pairs through one
+    scratch handle with keyed `reseed` chunks, on its motion profile's path.  The configs must share the position grid and
+    dt (the output shapes)."""
     if world_gen not in ("host", "device"):
         raise ValueError("world_gen must be 'host' or 'device', got %r" % (world_gen,))
     kw = dict(T_global=T_global, T_survivability=T_survivability, position_step=position_step, num_envs=num_envs,
@@ -230,6 +234,7 @@ def _difficulty(configs, seeds, T_global, T_survivability, position_step, num_en
         static_hit = torch.empty((S, nx, ny), dtype=torch.uint8, device=dev)
         cs = torch.empty((S, nx, ny, n_slots), dtype=torch.uint8, device=dev) if collision_state else None
         radius = torch.empty((S, env.num_agents), dtype=torch.float64, device=dev)
+        rvo = _GridHitsRun(env, steps, grid, table, n_slots, collision_state) if params.motion_profile == "RVO" else None
         for c0 in range(0, S, B):
             n = min(B, S - c0)
             if c0 > 0:
@@ -241,8 +246,11 @@ def _difficulty(configs, seeds, T_global, T_survivability, position_step, num_en
                     torch.cuda.current_stream(dev).synchronize()      # the last call has read the snapshot it replaces
                     env.set_worlds(generate_worlds(params, seeds[c0:c0 + n], env._smap))
             out = (first_hit[c0:c0 + n], static_hit[c0:c0 + n]) + ((cs[c0:c0 + n],) if collision_state else ())
-            env.difficulty(steps, grid, envs=range(0, n), slots=table, n_slots=n_slots, collision_state=collision_state,
-                           out=out)
+            if rvo is not None:
+                rvo.run(n, out, eager=c0 == 0)
+            else:
+                env.difficulty(steps, grid, envs=range(0, n), slots=table, n_slots=n_slots, collision_state=collision_state,
+                               out=out)
             radius[c0:c0 + n] = env.buffer("agent_radius")[:n]
         torch.cuda.current_stream(dev).synchronize()
         env.check_worlds()
@@ -257,3 +265,35 @@ def _difficulty(configs, seeds, T_global, T_survivability, position_step, num_en
     if collision_state:
         res["collision_state"] = cs
     return res
+
+
+class _GridHitsRun:
+    """The RVO path of `_difficulty`: `steps` iterations of `env.step(zeros)` + `env.grid_hits(t, ...)` over the first n
+    envs of the scratch handle, from the state the chunk's reseed left.  The first chunk runs eagerly (which also warms up
+    every launch); later chunks replay a CUDA graph captured once per chunk size into chunk buffers, and copy out."""
+
+    def __init__(self, env, steps, grid, table, n_slots, collision_state):
+        self.env, self.steps, self.grid = env, steps, grid
+        self.kw = dict(slots=table, n_slots=n_slots, collision_state=collision_state)
+        self.zero = torch.zeros(env.num_envs, dtype=torch.float64, device=env.device)
+        self.graphs, self.buf = {}, None
+
+    def _loop(self, n, out):
+        for t in range(1, self.steps + 1):
+            self.env.step(self.zero)
+            self.env.grid_hits(t, self.grid, envs=range(0, n), out=out, **self.kw)
+
+    def run(self, n, out, eager):
+        if eager:
+            self._loop(n, out)
+            return
+        if self.buf is None:
+            self.buf = tuple(torch.empty((self.env.num_envs,) + o.shape[1:], dtype=o.dtype, device=o.device) for o in out)
+        if n not in self.graphs:
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g):
+                self._loop(n, tuple(b[:n] for b in self.buf))
+            self.graphs[n] = g
+        self.graphs[n].replay()
+        for o, b in zip(out, self.buf):
+            o.copy_(b[:n])

@@ -691,8 +691,9 @@ class Drone2DVecEnv(object):
     # ------------------------------------------------------------------ difficulty metrics
     def difficulty(self, steps, grid, envs=None, slots=None, n_slots=None, collision_state=False, out=None):
         """Dynamic and static collisions of a drone held at every position of `grid`, over `steps` agent steps from each
-        env's reset snapshot (d2d_difficulty, one kernel; CVM handles only).  It reads the snapshot and writes only its
-        outputs, so the result does not depend on how far the envs have stepped.
+        env's reset snapshot (d2d_difficulty, one kernel; CVM handles only -- under RVO step the envs and call
+        `grid_hits`).  It reads the snapshot and writes only its outputs, so the result does not depend on how far the
+        envs have stepped.
         grid: (x0, y0, step, nx, ny), positions x0 + i * step, y0 + j * step.  envs: None (all) or a step-1 range.
         Returns {"first_hit": int16 [count, nx, ny] (first agent step k = 1..steps after which an agent disc grown by the
         drone radius holds the position; 0: none), "static_hit": uint8 [count, nx, ny] (collision_flag would be 1)} and,
@@ -701,10 +702,43 @@ class Drone2DVecEnv(object):
         slot k-1; shorter tables leave the later steps unrecorded); n_slots defaults to the largest slot + 1.
         out: preallocated contiguous CUDA tensors of those shapes and dtypes, a tuple (first_hit, static_hit[,
         collision_state]) -- what a captured CUDA graph writes into."""
+        spec, first, count, out, ptrs = self._difficulty_args("difficulty", steps, grid, envs, slots, n_slots,
+                                                              collision_state, out)
+        self._check(self._lib.d2d_difficulty(self._h, C.byref(spec), int(first), int(count), *ptrs, self._stream()),
+                    "d2d_difficulty")
+        return self._difficulty_result(out)
+
+    def grid_hits(self, t, grid, envs=None, slots=None, n_slots=None, collision_state=False, out=None):
+        """`difficulty`'s outputs built one step at a time from the LIVE agents (d2d_grid_hits, one kernel per call), for
+        CVM and RVO handles and any planner: step the envs, call grid_hits(t, ...) after step t = 1, 2, ..., steps, and
+        `out` then holds what `difficulty` returns for agents moved by those steps.  Call t = 1 initialises first_hit and
+        collision_state; later calls fold their hits in.  So every call of a run passes the same `out` (and the same grid,
+        envs and slot table), and nothing resets or reseeds the envs in between.  Same arguments and outputs as
+        `difficulty`, except that collision_state needs `slots` or `n_slots` (default table: step k -> slot k - 1 for
+        k <= n_slots); steps beyond the slot table are not recorded.  Returns the dict of `out`.  It reads the agents and
+        the ground truth and writes only its outputs.  A loop of `step` and `grid_hits` calls can be captured in a CUDA
+        graph."""
+        t = int(t)
+        if t < 1:
+            raise ValueError("grid_hits: step t = %d, must be >= 1" % t)
+        if collision_state and slots is None:
+            if n_slots is None:
+                raise ValueError("grid_hits: collision_state needs `slots` or `n_slots` (the same on every call of a run)")
+            slots = range(int(n_slots))
+        steps = max(t, len(slots)) if slots is not None else t
+        spec, first, count, out, ptrs = self._difficulty_args("grid_hits", steps, grid, envs, slots, n_slots,
+                                                              collision_state, out)
+        self._check(self._lib.d2d_grid_hits(self._h, C.byref(spec), t, int(first), int(count), *ptrs, self._stream()),
+                    "d2d_grid_hits")
+        return self._difficulty_result(out)
+
+    def _difficulty_args(self, what, steps, grid, envs, slots, n_slots, collision_state, out):
+        """The spec, env range, output tensors (allocated or checked) and output pointers of `difficulty` and
+        `grid_hits`."""
         first, count = 0, self.num_envs
         if envs is not None:
             if not (isinstance(envs, range) and envs.step == 1):
-                raise ValueError("difficulty: envs must be None or a step-1 range")
+                raise ValueError("%s: envs must be None or a step-1 range" % what)
             first, count = envs.start, max(0, envs.stop - envs.start)
         spec, n_slots = difficulty_spec(steps, grid, collision_state, slots, n_slots)
         nx, ny = spec.nx, spec.ny
@@ -718,15 +752,18 @@ class Drone2DVecEnv(object):
             if len(out) != len(shapes) or any(
                     not torch.is_tensor(t) or t.dtype != d or tuple(t.shape) != s or not t.is_contiguous() or
                     t.device.type != "cuda" or t.device.index != self._dev_index for t, (s, d) in zip(out, shapes)):
-                raise ValueError("difficulty: `out` must be contiguous tensors %s on cuda:%d"
-                                 % (", ".join("%s %s" % (d, s) for s, d in shapes), self._dev_index))
+                raise ValueError("%s: `out` must be contiguous tensors %s on cuda:%d"
+                                 % (what, ", ".join("%s %s" % (d, s) for s, d in shapes), self._dev_index))
 
         def ptr(t):
             return C.c_void_p(t.data_ptr() if count else 0)
-        self._check(self._lib.d2d_difficulty(self._h, C.byref(spec), int(first), int(count), ptr(out[0]), ptr(out[1]),
-                                             ptr(out[2]) if collision_state else None, self._stream()), "d2d_difficulty")
+        ptrs = (ptr(out[0]), ptr(out[1]), ptr(out[2]) if collision_state else None)
+        return spec, first, count, out, ptrs
+
+    @staticmethod
+    def _difficulty_result(out):
         res = {"first_hit": out[0], "static_hit": out[1]}
-        if collision_state:
+        if len(out) > 2:
             res["collision_state"] = out[2]
         return res
 

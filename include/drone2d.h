@@ -483,9 +483,9 @@ int d2d_render(d2d_handle *h, const int32_t *envs_host, int32_t first_env, int32
  *   collision_state uint8 [count][nx*ny][n_slots] or NULL: byte [p][slot[k-1]] is OR-ed with (dynamic hit after step k and
  *                   no static hit) -- glob_survivability's array, collision_flag == 2 -- for every k with slot[k-1] !=
  *                   D2D_DIFF_NO_SLOT; every other byte is 0.  NULL requires n_slots == 0 and vice versa.
- * Only CVM handles: under RVO the agents' motion needs d2d_rvo_kernel, and the call returns D2D_ERR_STATE (use the step
- * kernels, as metrics.global_survivability does).  The planner does not matter.  The spec travels by value in the kernel
- * parameters: a call is ONE launch with no upload and can be captured in a CUDA graph.  Every argument is checked before
+ * Only CVM handles: under RVO the agents' motion needs d2d_rvo_kernel, and the call returns D2D_ERR_STATE (step the envs
+ * and test the grid after every step with d2d_grid_hits below).  The planner does not matter.  The spec travels by value
+ * in the kernel parameters: a call is ONE launch with no upload and can be captured in a CUDA graph.  Every argument is checked before
  * anything is enqueued (a rejected call changes nothing); count = 0 enqueues nothing.  The call reads the reset snapshot and
  * writes only the outputs: env state, statistics, the episode log and the host mirror are untouched, and the result does not
  * depend on how far the envs have stepped.  D2D_ERR_STATE before d2d_set_world and while a pipelined step is in flight. */
@@ -502,6 +502,25 @@ typedef struct d2d_difficulty_spec {
 } d2d_difficulty_spec;
 int d2d_difficulty(d2d_handle *h, const d2d_difficulty_spec *spec, int32_t first_env, int32_t count, int16_t *first_hit,
                    uint8_t *static_hit, uint8_t *collision_state, void *stream);
+
+/* Grid hits: the outputs of d2d_difficulty built one step at a time from the LIVE agents (agent_pos, agent_radius) instead
+ * of the reset snapshot, for every motion profile (CVM and RVO) and any planner.  The caller steps the envs with the step
+ * kernels and calls d2d_grid_hits with t = 1, 2, ..., spec->steps after step t; the outputs then equal d2d_difficulty's
+ * for agents moved by those steps (under CVM from a reset, exactly d2d_difficulty's).  Call t folds the positions hit now
+ * into the outputs:
+ *   t == 1          first_hit is set to 1 where hit and 0 elsewhere, and the range's collision_state rows are zero-filled;
+ *   t > 1           first_hit is set to t where it is still 0 and the position is hit;
+ *   every call      static_hit is written (the same value each time: the ground truth does not move), and for a step with
+ *                   slot[t-1] != D2D_DIFF_NO_SLOT byte [p][slot[t-1]] of collision_state is set to 1 at every hit position
+ *                   that is not static.
+ * Same spec, outputs, range and checks as d2d_difficulty, plus 1 <= t <= spec->steps.  A run's calls must go to one stream
+ * (or be otherwise ordered), use the same spec, range and outputs, and see no reset, reseed or world change between t = 1
+ * and spec->steps.  Every argument is checked before anything is enqueued (a rejected call changes nothing); count = 0
+ * enqueues nothing.  ONE launch with no upload, so a loop of steps and calls can be captured in a CUDA graph.  The call
+ * reads the agents and the ground truth and writes only the outputs: env state, statistics, the episode log and the host
+ * mirror are untouched.  D2D_ERR_STATE before d2d_set_world and while a pipelined step is in flight. */
+int d2d_grid_hits(d2d_handle *h, const d2d_difficulty_spec *spec, int32_t t, int32_t first_env, int32_t count,
+                  int16_t *first_hit, uint8_t *static_hit, uint8_t *collision_state, void *stream);
 
 /* Number of kernel launches issued by this handle so far (bench.py's gpu_launches). */
 int64_t d2d_launch_count(const d2d_handle *h);
